@@ -58,6 +58,16 @@ int hsv_device_supported(void);
 /* Rows per (b, chunk) of a blk16 buffer for sequence length L. */
 int64_t hsv_blk16_rows(int64_t L);
 
+/* Test hook, read-only: which kernel variant the most recent host-side launch decision of a family chose.
+ * Process-global (like the bring-up switches); it never changes what is launched.  Copies min(n, count) ints to
+ * out and returns count (negative on a bad argument).
+ *   family 0, tcgen05 conv (count 14): kind (0 one-tile, 1 persistent, 2 fused activation, 3 operand-writing
+ *             epilogue), msub, warps per CTA, vec_epi (float4 epilogue), nphase, n_tile, stages, G (weight blocks
+ *             per ring stage), resident, nabuf (persistent only, else 0), grid x, y, z, launches so far
+ *   family 1, Activation1d (count 4): run length R (0 when the tensor-core kernel ran), act1d_mma ran, out_mode,
+ *             launches so far */
+int hsv_last_launch_config(int family, int *out, int n);
+
 /* ---- Activation1d(SnakeBeta): alias_free_torch/act.py:23-27 =
  * UpSample1d (resample.py:25-32) o SnakeBeta (activations.py:107-119, log-scale
  * alpha/beta) o DownSample1d (resample.py:46-48 -> filter.py:86-94), with the

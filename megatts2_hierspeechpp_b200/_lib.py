@@ -20,6 +20,7 @@ SIGNATURES = {
     "hsv_last_error": (c_char_p, []),
     "hsv_device_supported": (c_int, []),
     "hsv_blk16_rows": (c_int64, [c_int64]),
+    "hsv_last_launch_config": (c_int, [c_int, c_void_p, c_int]),
     "hsv_act1d_snakebeta": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_float,
                                     c_void_p]),
     "hsv_weight_norm_fold": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),

@@ -180,6 +180,15 @@ int g_act_run = 0;      // bring-up aid: force the run length (17 or 25); 0 = au
 #endif
 int g_act_mma = 0;      // fp16-operand output: 0 = auto, 1 = CUDA-core kernel (act1d.cu), 2 = tensor-core kernel (act1d_mma.cu)
 
+// hsv_last_launch_config, family 1: run length R (0 for the tensor-core kernel), act1d_mma ran, out_mode, launch count
+void note_launch(int R, int mma, int out_mode) {
+  int *last = hsv::g_last_launch[1];
+  last[0] = R;
+  last[1] = mma;
+  last[2] = out_mode;
+  ++last[3];
+}
+
 template <int R, int OUT_MODE>
 int launch(const float *x, void *out, const float *alpha, const float *beta, int B, int C, int64_t L, float sc,
            cudaStream_t st) {
@@ -207,6 +216,7 @@ int launch(const float *x, void *out, const float *alpha, const float *beta, int
   const int nt_i = (int)ntiles;
   const int64_t Lp = hsv::blk16_rows(L);
   const int cw = OUT_MODE == 1 ? hsv::blk_cw(C) : 0;
+  note_launch(R, 0, OUT_MODE);
   cudaError_t e = cudaLaunchKernelEx(&cfg, act1d_kernel<R, OUT_MODE>, x, out, alpha, beta, C, L, nrows, nt_i, Lp, sc, cw);
   if (e != cudaSuccess) {
     cudaGetLastError();
@@ -271,7 +281,10 @@ extern "C" int hsv_act1d_snakebeta(const float *x, void *out, const float *alpha
   // kernel keeps the tiny sequences (its tiles are 8 x 272 instead of 8 x 512)
   if (g_act_mma == 2 || (g_act_mma == 0 && HSV_ACT_MMA_AUTO && L >= 256)) {
     const int rc = hsv::act1d_mma_launch(x, out, alpha, beta, B, C, L, in_scale, st);
-    if (rc != 1) return rc;
+    if (rc != 1) {
+      note_launch(0, 1, 1);
+      return rc;
+    }
     HSV_REQUIRE(g_act_mma != 2, "act1d: shape not eligible for the forced tensor-core variant");
   }
   return R == 25 ? launch<25, 1>(x, out, alpha, beta, B, C, L, in_scale, st)

@@ -40,3 +40,15 @@ extern "C" int hsv_device_supported(void) {
 }
 
 extern "C" int64_t hsv_blk16_rows(int64_t L) { return hsv::blk16_rows(L); }
+
+namespace hsv {
+int g_last_launch[2][16] = {};
+}
+
+extern "C" int hsv_last_launch_config(int family, int *out, int n) {
+  HSV_REQUIRE(family == 0 || family == 1, "last_launch_config: family must be 0 (conv) or 1 (activation), got %d", family);
+  HSV_REQUIRE(n >= 0 && (out || n == 0), "last_launch_config: null output");
+  const int have = family == 0 ? hsv::LAST_CONV_N : hsv::LAST_ACT_N;
+  for (int i = 0; i < n && i < have; ++i) out[i] = hsv::g_last_launch[family][i];
+  return have;
+}

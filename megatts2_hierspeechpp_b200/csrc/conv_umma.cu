@@ -1058,6 +1058,18 @@ int g_persist = 1;  // persistent variant for eligible launches (hsv_set_umma_de
 
 constexpr int PERSIST_EPW = 4;
 
+// hsv_last_launch_config, family 0: kind (0 one-tile, 1 persistent, 2 fused activation, 3 operand-writing epilogue),
+// msub, warps per CTA, vec_epi, nphase, n_tile, stages, G, resident, nabuf, grid x / y / z, running launch count
+void note_launch(int kind, const Params &p, int warps, dim3 grid) {
+  const bool persist = kind == 1;  // resident / nabuf are only set (and read) by the persistent variant
+  const int v[hsv::LAST_CONV_N - 1] = {kind, p.msub, warps, p.vec_epi, p.tt.nphase, p.n_tile, p.stages, p.G,
+                                       persist ? p.resident : 0, persist ? p.nabuf : 0, (int)grid.x, (int)grid.y,
+                                       (int)grid.z};
+  int *last = hsv::g_last_launch[0];
+  for (int i = 0; i < hsv::LAST_CONV_N - 1; ++i) last[i] = v[i];
+  ++last[hsv::LAST_CONV_N - 1];
+}
+
 int launch_persist(Params p, int B, cudaStream_t st, const char *what) {
   static int max_dyn[64] = {0};
   int dev = 0;
@@ -1126,6 +1138,7 @@ int launch_persist(Params p, int B, cudaStream_t st, const char *what) {
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = hsv::g_pdl ? 1 : 0;
+  note_launch(1, p, 2 + 4 * PERSIST_EPW, cfg.gridDim);
   cudaError_t e = cudaLaunchKernelEx(&cfg, conv_umma_persist_kernel<PERSIST_EPW>, p);
   if (e != cudaSuccess) {
     cudaGetLastError();
@@ -1242,6 +1255,7 @@ int launch_variant(const Params &p, dim3 grid, size_t smem, cudaStream_t st, con
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = hsv::g_pdl ? 1 : 0;
+  note_launch(RR > 0 ? 2 : (BLK ? 3 : 0), p, NW, grid);
   cudaError_t e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<MSUB, MINB, SMALLN, RR, NW, BLK>, p);
   if (e != cudaSuccess) {
     cudaGetLastError();

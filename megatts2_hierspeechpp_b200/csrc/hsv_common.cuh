@@ -73,4 +73,10 @@ extern int g_pdl;  // 0 = plain stream order (bring-up switch), 1 = PDL on the a
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
+// What the most recent host-side launch decision of a kernel family chose (hsv_last_launch_config, common.cu):
+// [0] = the tcgen05 conv (conv_umma.cu), [1] = the fused activation (act1d.cu).  Process-global bookkeeping, written
+// just before the launch; it never changes what is launched.
+constexpr int LAST_CONV_N = 14, LAST_ACT_N = 4;
+extern int g_last_launch[2][16];
+
 }  // namespace hsv
