@@ -81,6 +81,15 @@ int hsv_last_launch_config(int family, int *out, int n);
  */
 int hsv_act1d_snakebeta(const float *x, void *out, const float *alpha, const float *beta,
                         int B, int C, int64_t L, int out_mode, float in_scale, void *stream);
+/* The same for a ragged batch (utterances of different lengths padded to L):
+ *   valid_len [B] int32, device (NULL = L for every item); values are clamped to [0, L] on the device.
+ * Item b is a sequence of Lv = valid_len[b] steps stored with row stride L: x at t >= Lv is never read, the
+ * edge replication happens at Lv, and outputs at Lv <= t < L are written as 0 (both out modes), so out[b, :, :Lv]
+ * equals, bit for bit, the call on that item alone with L = Lv.  Returns HSV_ERR_ARG when the tensor-core variant
+ * is forced (hsv_set_act_variant), which takes no lengths. */
+int hsv_act1d_snakebeta_ragged(const float *x, void *out, const float *alpha, const float *beta,
+                               const int32_t *valid_len, int B, int C, int64_t L, int out_mode, float in_scale,
+                               void *stream);
 
 /* ---- weight norm fold: torch._weight_norm(v, g, dim=0) as applied by the
  * forward pre-hook of torch.nn.utils.weight_norm on every conv of the path
@@ -175,6 +184,14 @@ int hsv_conv_transpose1d_umma(const void *a_blk16, const void *w_packed, const f
 int hsv_conv1d_direct(const float *x, const float *w, const float *bias, float *out,
                       int B, int Cin, int Cout, int64_t Lin, int64_t Lout, int k, int d, int pad,
                       int flags, void *stream);
+/* The same for a ragged batch: valid_len [B] int32, device (NULL = as hsv_conv1d_direct), clamped to [0, Lin].
+ * Item b uses x at t < valid_len[b] only (the rest counts as 0: values there never reach the result, though the float4
+ * staging of aligned rows may load the 16 bytes that straddle valid_len[b]) and writes 0 at t >= valid_len[b]; its first valid_len[b]
+ * outputs equal, bit for bit, hsv_conv1d_direct on that item alone with Lin = Lout = valid_len[b].  With valid_len,
+ * only the conv_post shape is supported (Cout <= 4, k = 7, d = 1, pad = 3, Lout == Lin); others return HSV_ERR_ARG. */
+int hsv_conv1d_direct_ragged(const float *x, const float *w, const float *bias, const int32_t *valid_len, float *out,
+                             int B, int Cin, int Cout, int64_t Lin, int64_t Lout, int k, int d, int pad, int flags,
+                             void *stream);
 
 /* ---- ConvTranspose1d (ups[i], hierspeechpp_speechsynthesizer.py:404-408,434):
  *   x [B,Cin,Lin], w [Cin,Cout,k] (folded), bias [Cout] -> out [B,Cout,u*Lin],
@@ -192,6 +209,13 @@ int hsv_conv_transpose1d_direct(const float *x, const float *w, const float *bia
  */
 int hsv_sr_pre_interp(const float *x, const float *w, const float *bias, float *out,
                       int B, int C, int64_t Lin, int64_t Lout, void *stream);
+/* The same for a ragged batch: valid_len_in [B] / valid_len_out [B] int32, device (each NULL = Lin / Lout), clamped
+ * to [0, Lin] / [0, Lout].  Item b is interpolated from Lin_b to Lout_b samples with its own scale
+ * (float)Lin_b / (float)Lout_b, conv_pre's zero padding sits at Lin_b, and outputs at t >= Lout_b are 0: out[b, :, :Lout_b]
+ * equals, bit for bit, hsv_sr_pre_interp on that item alone with Lin = Lin_b, Lout = Lout_b. */
+int hsv_sr_pre_interp_ragged(const float *x, const float *w, const float *bias, const int32_t *valid_len_in,
+                             const int32_t *valid_len_out, float *out, int B, int C, int64_t Lin, int64_t Lout,
+                             void *stream);
 
 /* Index probe for the bit-exact part of the parity contract: writes, for each
  * dst in [0,Lout): i0, i1 (int32) and lambda (fp32) of the linear interpolation. */
@@ -213,6 +237,10 @@ int hsv_pack_blk16(const float *x, void *out, int B, int C, int64_t L, int lrelu
  * (hierspeechpp_speechsynthesizer.py:440-446) taken by the consumer, each resblock writing its own tensor. */
 int hsv_pack_blk16_sum3(const float *x1, const float *x2, const float *x3, void *out, int B, int C, int64_t L,
                         int lrelu, float in_scale, void *stream);
+/* the same for a ragged batch: valid_len [B] int32, device (NULL = L for every item); rows t >= valid_len[b] of item
+ * b are written as zero without reading x (the zero padding of the item's own run). */
+int hsv_pack_blk16_sum3_ragged(const float *x1, const float *x2, const float *x3, const int32_t *valid_len, void *out,
+                               int B, int C, int64_t L, int lrelu, float in_scale, void *stream);
 /* inverse (tests / debugging): fp16 blk16 -> fp32 [B,C,L]. */
 int hsv_unpack_blk16(const void *in, float *x, int B, int C, int64_t L, void *stream);
 /* operand health (debugging aid; the reference keeps fp32 everywhere, the tensor-core operands here are fp16):

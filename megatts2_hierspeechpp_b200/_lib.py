@@ -23,6 +23,8 @@ SIGNATURES = {
     "hsv_last_launch_config": (c_int, [c_int, c_void_p, c_int]),
     "hsv_act1d_snakebeta": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_float,
                                     c_void_p]),
+    "hsv_act1d_snakebeta_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64,
+                                           c_int, c_float, c_void_p]),
     "hsv_weight_norm_fold": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "hsv_pack_conv_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "hsv_conv1d_umma": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_float,
@@ -38,15 +40,21 @@ SIGNATURES = {
                                           c_int64, c_int, c_int, c_int, c_void_p]),
     "hsv_conv1d_direct": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_int64,
                                   c_int, c_int, c_int, c_int, c_void_p]),
+    "hsv_conv1d_direct_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int64,
+                                         c_int64, c_int, c_int, c_int, c_int, c_void_p]),
     "hsv_conv_transpose1d_direct": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                             c_int64, c_int, c_int, c_void_p]),
     "hsv_sr_pre_interp": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int64, c_void_p]),
+    "hsv_sr_pre_interp_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                         c_int64, c_int64, c_void_p]),
     "hsv_interp_linear_table": (c_int, [c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsv_nearest_gather": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p]),
     "hsv_add3_bcast": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, c_void_p]),
     "hsv_pack_blk16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_float, c_void_p]),
     "hsv_pack_blk16_sum3": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_float,
                                     c_void_p]),
+    "hsv_pack_blk16_sum3_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int,
+                                           c_float, c_void_p]),
     "hsv_unpack_blk16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
     "hsv_blk16_stats": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
     "hsv_pack_blk16_act": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_int, c_void_p]),

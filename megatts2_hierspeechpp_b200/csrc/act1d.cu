@@ -18,6 +18,11 @@
 // 4 (mod 32) words, which makes every shared access of the walk conflict-free.
 // Results are staged in shared memory and written back coalesced, either as
 // fp32 [B,C,L] or as the fp16 "blk16" tensor-core operand layout.
+//
+// Ragged batches: with valid_len, row b is a sequence of Lv = valid_len[b]
+// steps stored with row stride L.  Lv takes the place of L in every clamp and
+// edge test, x at t >= Lv is never read, and outputs at Lv <= t < L are 0, so
+// the first Lv outputs equal those of the same row run alone at L = Lv.
 #include "act_core.cuh"
 
 namespace hsv {
@@ -29,16 +34,15 @@ namespace {
 
 using namespace hsv_act;
 
+// The kernel body, inlined twice by act1d_kernel: once with valid_len == nullptr (constant-folded: the full-length
+// path compiles to the code it had before lengths existed) and once for ragged batches.
 template <int R, int OUT_MODE>
-__global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, void *__restrict__ outp,
-                                                   const float *__restrict__ alpha,
-                                                   const float *__restrict__ beta, int C, int64_t L,
-                                                   int64_t nrows, int ntiles, int64_t Lp, float sc, int cw) {
+__device__ __forceinline__ void act1d_body(float *__restrict__ x_s, float *__restrict__ o_s, uint64_t &bar,
+                                           const float *__restrict__ x, void *__restrict__ outp,
+                                           const float *__restrict__ alpha, const float *__restrict__ beta,
+                                           const int32_t *__restrict__ valid_len, int C, int64_t L, int64_t nrows,
+                                           int ntiles, int64_t Lp, float sc, int cw) {
   using K = Cfg<R>;
-  // x_s[c][p] holds x[row0+c][t0 - XOFF + p]; XOFF = 8 keeps the tile start 16-byte aligned for TMA
-  __shared__ __align__(16) float x_s[ROWS * K::PITCH];
-  __shared__ __align__(16) float o_s[OUT_MODE == 0 ? ROWS * K::OPITCH : K::TILE * 4];
-  __shared__ __align__(8) uint64_t bar;
 
   const int tid = threadIdx.x;
   int tile, ch;        // time tile; channel of this thread's row
@@ -69,12 +73,26 @@ __global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, 
     be = __ldg(beta + ch);
   }
   hsv::pdl_wait();
+  // valid lengths are data of the forward (not static): read after the wait
+  // valid length of this thread's row (32-bit: one register across the kernel; with valid_len == nullptr every use
+  // below folds to L)
+  int lv = 0;
+  if (valid_len && row < nrows) {
+    const int v = __ldg(valid_len + (OUT_MODE == 1 ? (int64_t)blockIdx.z : row / C));
+    lv = v < 0 ? 0 : (v > L ? (int)L : v);
+  } else if (valid_len) {
+    lv = (int)L;
+  }
+  const int64_t Lv = valid_len ? (int64_t)lv : L;
 
   // ---- stage the x tile ----
   // interior tiles of 16-byte-aligned rows: one 1-D bulk TMA copy per row (no issue slots, no registers);
   // edge tiles / unaligned rows: plain loads with the replicate clamp of the 1x grid.
-  const bool fast = ((L & 3) == 0) && t0 >= K::XOFF && t0 + K::TILE + K::XOFF <= L && row0 + ROWS <= nrows &&
-                    ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+  // lanes 0..7 of every warp hold the valid lengths of rows 0..7 (c == lane % 8); with valid_len the tile must lie
+  // inside every row's valid part
+  bool fast = ((L & 3) == 0) && t0 >= K::XOFF && t0 + K::TILE + K::XOFF <= L && row0 + ROWS <= nrows &&
+              ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+  if (valid_len) fast = __all_sync(0xffffffffu, t0 + K::TILE + K::XOFF <= Lv) && fast;
   if (fast) {
     const uint32_t bar_a = static_cast<uint32_t>(__cvta_generic_to_shared(&bar));
     if (tid == 0) {
@@ -108,7 +126,6 @@ __global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, 
   } else {
     // all loads of a thread are issued before the first store (one exposed memory latency, not one per row)
     constexpr int NLD = (ROWS * K::XW + NT - 1) / NT;
-    const int Lm1 = (int)(L - 1);
     float v[NLD];
 #pragma unroll
     for (int i = 0; i < NLD; ++i) {
@@ -116,8 +133,9 @@ __global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, 
       const int cc = idx / K::XW, p = idx - cc * K::XW;
       const int64_t rw = row0 + cc;
       const int64_t t = t0 - K::XOFF + p;
+      const int Lm1 = (valid_len ? __shfl_sync(0xffffffffu, (int)Lv, cc & (ROWS - 1)) : (int)L) - 1;
       const int tc = t < 0 ? 0 : (t > Lm1 ? Lm1 : (int)t);
-      v[i] = (idx < ROWS * K::XW && rw < nrows) ? __ldg(x + rw * L + tc) : 0.f;
+      v[i] = (idx < ROWS * K::XW && rw < nrows && Lm1 >= 0) ? __ldg(x + rw * L + tc) : 0.f;
     }
 #pragma unroll
     for (int i = 0; i < NLD; ++i) {
@@ -131,17 +149,22 @@ __global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, 
   const int64_t ta = t0 + (int64_t)run * R;
   float outv[R];
   const bool active = row < nrows && ta < L;
-  if (active) {
+  if (row < nrows && ta < Lv) {
     const float *xw = x_s + c * K::PITCH + run * R + (K::XOFF - 5);
-    act_run<R>(xw, outv, al, be, ta, L, x + row * L, sc);
+    act_run<R>(xw, outv, al, be, ta, Lv, x + row * L, sc);
   }
 
   // ---- stage results, write back coalesced ----
   if (OUT_MODE == 0) {
     if (active) {
       float *o = o_s + c * K::OPITCH + run * R;
+      if (valid_len && ta + R > Lv) {   // the run reaches past the row's valid part: zero tail
 #pragma unroll
-      for (int j = 0; j < R; ++j) o[j] = outv[j];
+        for (int j = 0; j < R; ++j) o[j] = ta + j < Lv ? outv[j] : 0.f;
+      } else {
+#pragma unroll
+        for (int j = 0; j < R; ++j) o[j] = outv[j];
+      }
     }
     __syncthreads();
     float *out = reinterpret_cast<float *>(outp);
@@ -153,8 +176,13 @@ __global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, 
   } else {
     __half *o_h = reinterpret_cast<__half *>(o_s);  // [TILE][8]
     if (active) {
+      if (valid_len && ta + R > Lv) {
 #pragma unroll
-      for (int j = 0; j < R; ++j) o_h[(run * R + j) * 8 + c] = __float2half_rn(outv[j]);
+        for (int j = 0; j < R; ++j) o_h[(run * R + j) * 8 + c] = __float2half_rn(ta + j < Lv ? outv[j] : 0.f);
+      } else {
+#pragma unroll
+        for (int j = 0; j < R; ++j) o_h[(run * R + j) * 8 + c] = __float2half_rn(outv[j]);
+      }
     }
     __syncthreads();
     // rows row0..row0+7 are one 8-channel unit of one batch item (C % 8 == 0)
@@ -174,6 +202,25 @@ __global__ void __launch_bounds__(NT) act1d_kernel(const float *__restrict__ x, 
   }
 }
 
+template <int R, int OUT_MODE>
+// 7 CTAs per SM need <= 72 registers: the fp16-operand kernels (both bodies inlined) meet it only with the bound, the
+// fp32-output ones without it (with it, R = 25 spills)
+__global__ void __launch_bounds__(NT, OUT_MODE == 1 ? 7 : 0) act1d_kernel(const float *__restrict__ x, void *__restrict__ outp,
+                                                   const float *__restrict__ alpha,
+                                                   const float *__restrict__ beta,
+                                                   const int32_t *__restrict__ valid_len, int C, int64_t L,
+                                                   int64_t nrows, int ntiles, int64_t Lp, float sc, int cw) {
+  using K = Cfg<R>;
+  // x_s[c][p] holds x[row0+c][t0 - XOFF + p]; XOFF = 8 keeps the tile start 16-byte aligned for TMA
+  __shared__ __align__(16) float x_s[ROWS * K::PITCH];
+  __shared__ __align__(16) float o_s[OUT_MODE == 0 ? ROWS * K::OPITCH : K::TILE * 4];
+  __shared__ __align__(8) uint64_t bar;
+  if (valid_len)
+    act1d_body<R, OUT_MODE>(x_s, o_s, bar, x, outp, alpha, beta, valid_len, C, L, nrows, ntiles, Lp, sc, cw);
+  else
+    act1d_body<R, OUT_MODE>(x_s, o_s, bar, x, outp, alpha, beta, nullptr, C, L, nrows, ntiles, Lp, sc, cw);
+}
+
 int g_act_run = 0;      // bring-up aid: force the run length (17 or 25); 0 = automatic
 #ifndef HSV_ACT_MMA_AUTO
 #define HSV_ACT_MMA_AUTO 0   // policy of variant 0 (auto): 1 = tensor-core kernel for L >= 256 (set once it wins on B200)
@@ -190,8 +237,8 @@ void note_launch(int R, int mma, int out_mode) {
 }
 
 template <int R, int OUT_MODE>
-int launch(const float *x, void *out, const float *alpha, const float *beta, int B, int C, int64_t L, float sc,
-           cudaStream_t st) {
+int launch(const float *x, void *out, const float *alpha, const float *beta, const int32_t *valid_len, int B, int C,
+           int64_t L, float sc, cudaStream_t st) {
   using K = Cfg<R>;
   const int64_t nrows = (int64_t)B * C;
   const int64_t ntiles = (L + K::TILE - 1) / K::TILE;
@@ -217,7 +264,8 @@ int launch(const float *x, void *out, const float *alpha, const float *beta, int
   const int64_t Lp = hsv::blk16_rows(L);
   const int cw = OUT_MODE == 1 ? hsv::blk_cw(C) : 0;
   note_launch(R, 0, OUT_MODE);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, act1d_kernel<R, OUT_MODE>, x, out, alpha, beta, C, L, nrows, nt_i, Lp, sc, cw);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, act1d_kernel<R, OUT_MODE>, x, out, alpha, beta, valid_len, C, L, nrows, nt_i, Lp,
+                                     sc, cw);
   if (e != cudaSuccess) {
     cudaGetLastError();
     hsv::set_error("act1d_snakebeta: launch failed: %s", cudaGetErrorString(e));
@@ -237,6 +285,12 @@ extern "C" int hsv_set_act_variant(int v) {
 
 extern "C" int hsv_act1d_snakebeta(const float *x, void *out, const float *alpha, const float *beta, int B,
                                    int C, int64_t L, int out_mode, float in_scale, void *stream) {
+  return hsv_act1d_snakebeta_ragged(x, out, alpha, beta, nullptr, B, C, L, out_mode, in_scale, stream);
+}
+
+extern "C" int hsv_act1d_snakebeta_ragged(const float *x, void *out, const float *alpha, const float *beta,
+                                          const int32_t *valid_len, int B, int C, int64_t L, int out_mode,
+                                          float in_scale, void *stream) {
   if (B == 0 || L == 0) return HSV_OK;  // empty batch / sequence
   HSV_REQUIRE(x && out && alpha && beta, "act1d: null pointer");
   HSV_REQUIRE(B >= 0 && C > 0 && L >= 0, "act1d: bad shape B=%d C=%d L=%lld", B, C, (long long)L);
@@ -272,14 +326,15 @@ extern "C" int hsv_act1d_snakebeta(const float *x, void *out, const float *alpha
   }
   HSV_REQUIRE(R == 9 || R == 17 || R == 21 || R == 25, "act1d: run length must be 9, 17, 21 or 25");
   if (out_mode == 0)
-    return R == 25 ? launch<25, 0>(x, out, alpha, beta, B, C, L, in_scale, st)
-                   : (R == 21 ? launch<21, 0>(x, out, alpha, beta, B, C, L, in_scale, st)
-                              : (R == 17 ? launch<17, 0>(x, out, alpha, beta, B, C, L, in_scale, st)
-                                         : launch<9, 0>(x, out, alpha, beta, B, C, L, in_scale, st)));
+    return R == 25 ? launch<25, 0>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)
+                   : (R == 21 ? launch<21, 0>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)
+                              : (R == 17 ? launch<17, 0>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)
+                                         : launch<9, 0>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)));
   HSV_REQUIRE(C % 16 == 0, "act1d: blk16 output needs C %% 16 == 0 (C=%d)", C);
   // tensor-core FIR variant (act1d_mma.cu): every shape with at least half a tile of work per row; the CUDA-core
   // kernel keeps the tiny sequences (its tiles are 8 x 272 instead of 8 x 512)
-  if (g_act_mma == 2 || (g_act_mma == 0 && HSV_ACT_MMA_AUTO && L >= 256)) {
+  HSV_REQUIRE(!(valid_len && g_act_mma == 2), "act1d: the forced tensor-core variant takes no valid lengths");
+  if (g_act_mma == 2 || (g_act_mma == 0 && HSV_ACT_MMA_AUTO && L >= 256 && !valid_len)) {
     const int rc = hsv::act1d_mma_launch(x, out, alpha, beta, B, C, L, in_scale, st);
     if (rc != 1) {
       note_launch(0, 1, 1);
@@ -287,8 +342,8 @@ extern "C" int hsv_act1d_snakebeta(const float *x, void *out, const float *alpha
     }
     HSV_REQUIRE(g_act_mma != 2, "act1d: shape not eligible for the forced tensor-core variant");
   }
-  return R == 25 ? launch<25, 1>(x, out, alpha, beta, B, C, L, in_scale, st)
-                 : (R == 21 ? launch<21, 1>(x, out, alpha, beta, B, C, L, in_scale, st)
-                            : (R == 17 ? launch<17, 1>(x, out, alpha, beta, B, C, L, in_scale, st)
-                                       : launch<9, 1>(x, out, alpha, beta, B, C, L, in_scale, st)));
+  return R == 25 ? launch<25, 1>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)
+                 : (R == 21 ? launch<21, 1>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)
+                            : (R == 17 ? launch<17, 1>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)
+                                       : launch<9, 1>(x, out, alpha, beta, valid_len, B, C, L, in_scale, st)));
 }

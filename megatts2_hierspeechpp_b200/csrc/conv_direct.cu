@@ -95,22 +95,89 @@ conv1d_tiled_kernel(const float *__restrict__ x, const float *__restrict__ w, co
   }
 }
 
+// One output of a very short sequence (cond(g): Lin == Lout == 1): one warp per output element, lanes split the
+// Cin*k products, shuffle reduction.  xb = the batch item's [Cin] rows of stride ldx, of which [0, Lin) are read;
+// every lane returns the sum, lane 0 stores out = epilogue(sum).
+__device__ __forceinline__ void rowdot_out(const float *__restrict__ xb, const float *__restrict__ w,
+                                           const float *__restrict__ bias, float *o, int Cin, int64_t ldx,
+                                           int64_t Lin, int k, int d, int pad, int co, int64_t t, int flags,
+                                           int lane) {
+  float acc = 0.f;
+  for (int r = lane; r < Cin * k; r += 32) {
+    const int ci = r / k, j = r - ci * k;
+    const int64_t ts = t - pad + (int64_t)j * d;
+    if (ts >= 0 && ts < Lin) {
+      float v = __ldg(xb + (int64_t)ci * ldx + ts);
+      if (flags & HSV_CONV_LRELU_IN) v = v > 0.f ? v : 0.1f * v;
+      if (flags & HSV_CONV_LRELU001_IN) v = v > 0.f ? v : 0.01f * v;
+      if (flags & HSV_CONV_SILU_IN) v = v / (1.f + expf(-v));
+      acc = fmaf(__ldg(w + (int64_t)co * Cin * k + r), v, acc);
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) {
+    if (bias) acc += __ldg(bias + co);
+    if (flags & HSV_CONV_TANH) acc = tanhf(acc);
+    if (flags & HSV_CONV_ADD_OUT) acc += *o;
+    *o = acc;
+  }
+}
+
+// Ragged batch item of the thin kernels (Lout == Lin, pad 3, k 7): valid length of item b, clamped to [0, Lin).
+__device__ __forceinline__ int64_t thin_valid_len(const int32_t *valid_len, int b, int64_t Lin) {
+  if (!valid_len) return Lin;
+  const int v = __ldg(valid_len + b);
+  return v < 0 ? 0 : (v > Lin ? Lin : v);
+}
+
+// An item of at most 8 valid steps is computed the way hsv_conv1d_direct computes it alone (Lout <= 8: the warp
+// reduction above, a different summation order from the thin kernels), so it stays bit-identical to its own run.
+// CTA 0 of the item computes the Lv * Cout outputs, every CTA zeroes its part of [Lv, Lout).
+__device__ __forceinline__ void thin_short_item(const float *__restrict__ x, const float *__restrict__ w,
+                                                const float *__restrict__ bias, float *__restrict__ out, int b, int Cin, int Cout, int64_t Lin,
+                                                int64_t Lv, int flags, int64_t t0, int TT) {
+  const int lane = threadIdx.x & 31, nw = blockDim.x >> 5, wid = threadIdx.x >> 5;
+  if (blockIdx.x == 0) {
+    for (int q = wid; q < Cout * (int)Lv; q += nw) {
+      const int co = q / (int)Lv, t = q - co * (int)Lv;
+      rowdot_out(x + (int64_t)b * Cin * Lin, w, bias, out + ((int64_t)b * Cout + co) * Lin + t, Cin, Lin, Lv, 7, 1,
+                 3, co, t, flags, lane);
+    }
+  }
+  for (int q = threadIdx.x; q < Cout * TT; q += blockDim.x) {
+    const int co = q / TT;
+    const int64_t t = t0 + (q - co * TT);
+    if (t >= Lv && t < Lin) out[((int64_t)b * Cout + co) * Lin + t] = 0.f;
+  }
+}
+
 // thin conv for Cout <= 4 and d == 1 (conv_post 16|32|64 -> 1, k=7).  CTA = TT consecutive outputs of one batch
 // row: the input window of CC channels is staged in shared memory with coalesced, independent loads (the previous
 // version walked the channels serially from global memory: 20 us for the [16,160000] conv_post of the batch-1
 // vocoder, a dependent-load chain), then every thread produces 2 outputs per output channel from a register window
 // of K+1 samples per input channel.  Accumulation order (ci outer, tap inner, fmaf) as before.
+// valid_len (K == 7, Lout == Lin only): item b reads x[t < Lv] (the rest as 0) and writes 0 at t >= Lv.
 template <int K>
-__global__ void __launch_bounds__(256) conv1d_thin_smem_kernel(const float *__restrict__ x, const float *__restrict__ w,
-                                                               const float *__restrict__ bias, float *__restrict__ out,
-                                                               int Cin, int Cout, int64_t Lin, int64_t Lout, int pad,
-                                                               int flags) {
-  constexpr int TT = 512, CC = 16, W = TT + K - 1, WP = (W + 3) & ~3;
-  __shared__ __align__(16) float xs[CC][WP];
-  __shared__ float ws[4][CC * K];
+struct ThinSmem {
+  static constexpr int TT = 512, CC = 16, W = TT + K - 1, WP = (W + 3) & ~3;
+};
+
+// body of conv1d_thin_smem_kernel, inlined with valid_len == nullptr (the full-length path, constant-folded) and without
+template <int K>
+__device__ __forceinline__ void thin_smem_body(float (*__restrict__ xs)[ThinSmem<K>::WP], float (*__restrict__ ws)[16 * K],
+                                               const float *__restrict__ x, const float *__restrict__ w,
+                                               const float *__restrict__ bias, float *__restrict__ out,
+                                               const int32_t *__restrict__ valid_len, int Cin, int Cout, int64_t Lin,
+                                               int64_t Lout, int pad, int flags) {
+  constexpr int TT = ThinSmem<K>::TT, CC = ThinSmem<K>::CC, W = ThinSmem<K>::W;
   const int tid = threadIdx.x;
   const int b = blockIdx.y;
   const int64_t t0 = (int64_t)blockIdx.x * TT;
+  const int64_t Lv = thin_valid_len(valid_len, b, Lin);
+  if (valid_len && Lv <= 8) {
+    thin_short_item(x, w, bias, out, b, Cin, Cout, Lin, Lv, flags, t0, TT);
+    return;
+  }
   float acc[4][2];
 #pragma unroll
   for (int co = 0; co < 4; ++co) acc[co][0] = acc[co][1] = 0.f;
@@ -126,7 +193,7 @@ __global__ void __launch_bounds__(256) conv1d_thin_smem_kernel(const float *__re
         const int idx = i0 + 256 * q;
         const int c = idx / W, pp = idx - c * W;
         const int64_t ts = t0 - pad + pp;
-        v[q] = (idx < nc * W && ts >= 0 && ts < Lin) ? __ldg(x + ((int64_t)b * Cin + c0 + c) * Lin + ts) : 0.f;
+        v[q] = (idx < nc * W && ts >= 0 && ts < Lv) ? __ldg(x + ((int64_t)b * Cin + c0 + c) * Lin + ts) : 0.f;
       }
 #pragma unroll
       for (int q = 0; q < NB; ++q) {
@@ -176,10 +243,24 @@ __global__ void __launch_bounds__(256) conv1d_thin_smem_kernel(const float *__re
         float v = acc[co][r] + bv;
         if (flags & HSV_CONV_TANH) v = tanhf(v);
         if (flags & HSV_CONV_ADD_OUT) v += o[r];
-        o[r] = v;
+        o[r] = valid_len && t0 + 2 * tid + r >= Lv ? 0.f : v;
       }
     }
   }
+}
+
+template <int K>
+__global__ void __launch_bounds__(256) conv1d_thin_smem_kernel(const float *__restrict__ x, const float *__restrict__ w,
+                                                               const float *__restrict__ bias, float *__restrict__ out,
+                                                               const int32_t *__restrict__ valid_len, int Cin,
+                                                               int Cout, int64_t Lin, int64_t Lout, int pad,
+                                                               int flags) {
+  __shared__ __align__(16) float xs[ThinSmem<K>::CC][ThinSmem<K>::WP];
+  __shared__ float ws[4][ThinSmem<K>::CC * K];
+  if (valid_len)
+    thin_smem_body<K>(xs, ws, x, w, bias, out, valid_len, Cin, Cout, Lin, Lout, pad, flags);
+  else
+    thin_smem_body<K>(xs, ws, x, w, bias, out, nullptr, Cin, Cout, Lin, Lout, pad, flags);
 }
 
 // The same for 16-byte aligned tensors with Lin % 4 == 0 and pad == 3 (every conv_post of the path): the window is staged with
@@ -187,15 +268,27 @@ __global__ void __launch_bounds__(256) conv1d_thin_smem_kernel(const float *__re
 // division; every thread produces 4 outputs per output channel from three LDS.128 of inputs and two of weights per input
 // channel.  SpeechSR48 conv_post at batch 16 ([16,32,480000]): 577 us (scalar staging) / 364 us (the round-1 kernel) -> see
 // DESIGN.md §4; ~224 FMAs per output make it FMA-issue-bound once the staging is out of the way.
-__global__ void __launch_bounds__(128) conv1d_thin_vec_kernel(const float *__restrict__ x, const float *__restrict__ w,
-                                                              const float *__restrict__ bias, float *__restrict__ out,
-                                                              int Cin, int Cout, int64_t Lin, int64_t Lout, int flags) {
-  constexpr int K = 7, TT = 512, CC = 16, W4 = TT / 4 + 2, WP = 4 * W4;   // window = [t0 - 4, t0 + TT + 4)
-  __shared__ __align__(16) float xs[CC][WP];
-  __shared__ __align__(16) float ws[4][CC][8];
+// valid_len: as conv1d_thin_smem_kernel, except that a float4 straddling Lv is loaded whole and its lanes >= Lv are
+// zeroed in shared memory before use.
+constexpr int THIN_VEC_WP = 4 * (512 / 4 + 2);   // window = [t0 - 4, t0 + TT + 4)
+
+// body of conv1d_thin_vec_kernel, inlined with valid_len == nullptr (the full-length path, constant-folded) and without
+__device__ __forceinline__ void thin_vec_body(float (*__restrict__ xs)[THIN_VEC_WP], float (*__restrict__ ws)[16][8],
+                                              const float *__restrict__ x, const float *__restrict__ w,
+                                              const float *__restrict__ bias, float *__restrict__ out,
+                                              const int32_t *__restrict__ valid_len, int Cin, int Cout, int64_t Lin,
+                                              int64_t Lout, int flags) {
+  constexpr int K = 7, TT = 512, CC = 16, W4 = TT / 4 + 2;
   const int tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
   const int b = blockIdx.y;
   const int64_t t0 = (int64_t)blockIdx.x * TT;
+  const int64_t Lv = thin_valid_len(valid_len, b, Lin);
+  if (valid_len && Lv <= 8) {
+    thin_short_item(x, w, bias, out, b, Cin, Cout, Lin, Lv, flags, t0, TT);
+    return;
+  }
+  // window float4 that straddles Lv (-1: none; Lin % 4 == 0, so only a ragged item has one)
+  const int p4v = valid_len && (Lv & 3) && Lv > t0 - 4 && Lv < t0 + TT + 4 ? (int)((Lv - (t0 - 4)) >> 2) : -1;
   float acc[4][4];
 #pragma unroll
   for (int co = 0; co < 4; ++co) acc[co][0] = acc[co][1] = acc[co][2] = acc[co][3] = 0.f;
@@ -212,8 +305,8 @@ __global__ void __launch_bounds__(128) conv1d_thin_vec_kernel(const float *__res
       for (int i = 0; i < 5; ++i) {
         const int p4 = lane + 32 * i;
         const int64_t ts = t0 - 4 + 4 * (int64_t)p4;
-        v[cc * 5 + i] = (c < nc && p4 < W4 && ts >= 0 && ts < Lin) ? __ldg(reinterpret_cast<const float4 *>(row) + p4)
-                                                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[cc * 5 + i] = (c < nc && p4 < W4 && ts >= 0 && ts < Lv) ? __ldg(reinterpret_cast<const float4 *>(row) + p4)
+                                                                   : make_float4(0.f, 0.f, 0.f, 0.f);
       }
     }
 #pragma unroll
@@ -234,6 +327,13 @@ __global__ void __launch_bounds__(128) conv1d_thin_vec_kernel(const float *__res
         }
         if (c < nc && p4 < W4) *reinterpret_cast<float4 *>(&xs[c][4 * p4]) = u;
       }
+    }
+    if (p4v >= 0 && (p4v & 31) == lane) {
+      // the float4 that straddles Lv was staged by this thread: zero its steps >= Lv
+#pragma unroll
+      for (int cc = 0; cc < CC / 4; ++cc)
+        if (wrp + 4 * cc < nc)
+          for (int q = (int)(Lv & 3); q < 4; ++q) xs[wrp + 4 * cc][4 * p4v + q] = 0.f;
     }
     for (int idx = tid; idx < 4 * CC * 8; idx += 128) {
       const int co = idx / (CC * 8), r = idx - co * (CC * 8), c = r >> 3, j = r & 7;
@@ -277,8 +377,26 @@ __global__ void __launch_bounds__(128) conv1d_thin_vec_kernel(const float *__res
       const float4 prev = *reinterpret_cast<const float4 *>(o);
       r4.x += prev.x; r4.y += prev.y; r4.z += prev.z; r4.w += prev.w;
     }
+    if (valid_len && t + 4 > Lv) {
+      r4.x = t < Lv ? r4.x : 0.f;
+      r4.y = t + 1 < Lv ? r4.y : 0.f;
+      r4.z = t + 2 < Lv ? r4.z : 0.f;
+      r4.w = t + 3 < Lv ? r4.w : 0.f;
+    }
     *reinterpret_cast<float4 *>(o) = r4;
   }
+}
+
+__global__ void __launch_bounds__(128) conv1d_thin_vec_kernel(const float *__restrict__ x, const float *__restrict__ w,
+                                                              const float *__restrict__ bias, float *__restrict__ out,
+                                                              const int32_t *__restrict__ valid_len, int Cin,
+                                                              int Cout, int64_t Lin, int64_t Lout, int flags) {
+  __shared__ __align__(16) float xs[16][THIN_VEC_WP];
+  __shared__ __align__(16) float ws[4][16][8];
+  if (valid_len)
+    thin_vec_body(xs, ws, x, w, bias, out, valid_len, Cin, Cout, Lin, Lout, flags);
+  else
+    thin_vec_body(xs, ws, x, w, bias, out, nullptr, Cin, Cout, Lin, Lout, flags);
 }
 
 // generic thin conv (any k, d): one thread per (b, t)
@@ -314,8 +432,7 @@ __global__ void conv1d_thin_kernel(const float *__restrict__ x, const float *__r
   }
 }
 
-// very short sequences (cond(g): Lin == Lout == 1): one warp per output element, lanes split the
-// Cin*k products, shuffle reduction
+// very short sequences (cond(g): Lin == Lout == 1): see rowdot_out
 __global__ void conv1d_rowdot_kernel(const float *__restrict__ x, const float *__restrict__ w,
                                      const float *__restrict__ bias, float *__restrict__ out, int B, int Cin,
                                      int Cout, int64_t Lin, int64_t Lout, int k, int d, int pad, int flags) {
@@ -326,26 +443,8 @@ __global__ void conv1d_rowdot_kernel(const float *__restrict__ x, const float *_
   const int64_t t = wid % Lout;
   const int co = (int)((wid / Lout) % Cout);
   const int b = (int)(wid / (Lout * Cout));
-  float acc = 0.f;
-  for (int r = lane; r < Cin * k; r += 32) {
-    const int ci = r / k, j = r - ci * k;
-    const int64_t ts = t - pad + (int64_t)j * d;
-    if (ts >= 0 && ts < Lin) {
-      float v = __ldg(x + ((int64_t)b * Cin + ci) * Lin + ts);
-      if (flags & HSV_CONV_LRELU_IN) v = v > 0.f ? v : 0.1f * v;
-      if (flags & HSV_CONV_LRELU001_IN) v = v > 0.f ? v : 0.01f * v;
-      if (flags & HSV_CONV_SILU_IN) v = v / (1.f + expf(-v));
-      acc = fmaf(__ldg(w + (int64_t)co * Cin * k + r), v, acc);
-    }
-  }
-  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-  if (lane == 0) {
-    if (bias) acc += __ldg(bias + co);
-    if (flags & HSV_CONV_TANH) acc = tanhf(acc);
-    float *o = out + ((int64_t)b * Cout + co) * Lout + t;
-    if (flags & HSV_CONV_ADD_OUT) acc += *o;
-    *o = acc;
-  }
+  rowdot_out(x + (int64_t)b * Cin * Lin, w, bias, out + ((int64_t)b * Cout + co) * Lout + t, Cin, Lin, Lin, k, d, pad,
+             co, t, flags, lane);
 }
 
 // the same for a per-utterance vector (k == 1, Lin == Lout == 1, Cin % 4 == 0: cond(g), adaLN, cond_layer): float4
@@ -494,23 +593,38 @@ __device__ __forceinline__ void lin_src(int64_t dst, float scale, int64_t Lin, i
   lam = src - (float)a;
 }
 
+// vl_in / vl_out (nullable): per-item valid lengths; item b is then interpolated from Lin_b to Lout_b samples (its
+// own scale, bit-identical to a call with Lin = Lin_b, Lout = Lout_b) and its outputs at t >= Lout_b are 0.
 __global__ void sr_pre_interp_kernel(const float *__restrict__ x, const float *__restrict__ w,
-                                     const float *__restrict__ bias, float *__restrict__ out, int B, int C,
-                                     int64_t Lin, int64_t Lout, float scale) {
+                                     const float *__restrict__ bias, float *__restrict__ out,
+                                     const int32_t *__restrict__ vl_in, const int32_t *__restrict__ vl_out, int B,
+                                     int C, int64_t Lin, int64_t Lout, float scale) {
   const int64_t n = (int64_t)B * Lout;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int b = (int)(i / Lout);
     const int64_t t = i - (int64_t)b * Lout;
+    const float *xr = x + (int64_t)b * Lin;
+    int64_t Li = Lin;
+    float sc = scale;
+    if (vl_in || vl_out) {
+      const int vi = vl_in ? __ldg(vl_in + b) : (int)Lin, vo = vl_out ? __ldg(vl_out + b) : (int)Lout;
+      Li = vi < 0 ? 0 : (vi > Lin ? Lin : vi);
+      const int64_t Lo = vo < 0 ? 0 : (vo > Lout ? Lout : vo);
+      if (t >= Lo || Li == 0) {
+        for (int c = 0; c < C; ++c) out[((int64_t)b * C + c) * Lout + t] = 0.f;
+        continue;
+      }
+      sc = (float)Li / (float)Lo;
+    }
     int i0, i1;
     float lam;
-    lin_src(t, scale, Lin, i0, i1, lam);
-    const float *xr = x + (int64_t)b * Lin;
+    lin_src(t, sc, Li, i0, i1, lam);
     float xa[7], xb[7];
 #pragma unroll
     for (int j = 0; j < 7; ++j) {
       const int64_t ta = (int64_t)i0 - 3 + j, tb = (int64_t)i1 - 3 + j;
-      xa[j] = (ta >= 0 && ta < Lin) ? __ldg(xr + ta) : 0.f;
-      xb[j] = (tb >= 0 && tb < Lin) ? __ldg(xr + tb) : 0.f;
+      xa[j] = (ta >= 0 && ta < Li) ? __ldg(xr + ta) : 0.f;
+      xb[j] = (tb >= 0 && tb < Li) ? __ldg(xr + tb) : 0.f;
     }
     const float w0 = 1.0f - lam, w1 = lam;
     for (int c = 0; c < C; ++c) {
@@ -592,12 +706,19 @@ __global__ void weight_norm_fold_kernel(const float *__restrict__ v, const float
 // sum over the resblocks of a stage (each resblock stream writes its own tensor; no chained accumulation)
 // grid = (time blocks, channel groups of 8, batch): no index division (a flat index cost two 64-bit divisions per thread,
 // as many instructions as the rest of the kernel)
+// valid_len (nullable): rows t >= valid_len[b] of item b are written as zero without reading x
 __global__ void __launch_bounds__(256) pack_blk16_kernel(const float *__restrict__ x, const float *__restrict__ x2,
-                                                         const float *__restrict__ x3, uint4 *__restrict__ out, int C,
-                                                         int64_t L, int64_t Lp, int lrelu, float sc, int cw) {
+                                                         const float *__restrict__ x3,
+                                                         const int32_t *__restrict__ valid_len, uint4 *__restrict__ out,
+                                                         int C, int64_t L, int64_t Lp, int lrelu, float sc, int cw) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= L) return;
   const int q = blockIdx.y, bb = blockIdx.z;
+  if (valid_len && t >= __ldg(valid_len + bb)) {
+    *reinterpret_cast<uint4 *>(reinterpret_cast<uint8_t *>(out) + hsv::blk_unit_offset(cw, Lp, C, bb, 8 * q, HSV_BLK_PAD + t)) =
+        make_uint4(0u, 0u, 0u, 0u);
+    return;
+  }
   const int64_t off = ((int64_t)bb * C + 8 * q) * L + t;
   const float *xr = x + off;
   float v[8];
@@ -686,18 +807,27 @@ inline int grid_for(int64_t n, int threads) {
 extern "C" int hsv_conv1d_direct(const float *x, const float *w, const float *bias, float *out, int B, int Cin,
                                  int Cout, int64_t Lin, int64_t Lout, int k, int d, int pad, int flags,
                                  void *stream) {
+  return hsv_conv1d_direct_ragged(x, w, bias, nullptr, out, B, Cin, Cout, Lin, Lout, k, d, pad, flags, stream);
+}
+
+extern "C" int hsv_conv1d_direct_ragged(const float *x, const float *w, const float *bias, const int32_t *valid_len,
+                                        float *out, int B, int Cin, int Cout, int64_t Lin, int64_t Lout, int k, int d,
+                                        int pad, int flags, void *stream) {
   if (B == 0 || Lout <= 0) return HSV_OK;  // empty batch / sequence
   HSV_REQUIRE(x && w && out, "conv1d_direct: null pointer");
   HSV_REQUIRE(Cin > 0 && Cout > 0 && k >= 1 && k <= KMAX && d >= 1, "conv1d_direct: bad shape");
   HSV_REQUIRE((k - 1) * d <= HALO_MAX, "conv1d_direct: (k-1)*d=%d exceeds %d", (k - 1) * d, HALO_MAX);
   HSV_REQUIRE(Lout == Lin + 2 * (int64_t)pad - (int64_t)d * (k - 1), "conv1d_direct: Lout mismatch");
+  HSV_REQUIRE(!valid_len || (Cout <= 4 && k == 7 && d == 1 && pad == 3),
+              "conv1d_direct: valid lengths need Cout <= 4, k = 7, d = 1, Lout == Lin (Cout=%d k=%d d=%d pad=%d)",
+              Cout, k, d, pad);
   if (B == 0 || Lout <= 0) return HSV_OK;
   cudaStream_t st = hsv::as_stream(stream);
   if (k == 1 && Lin == 1 && pad == 0 && (Cin & 3) == 0 && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(w)) & 15) == 0) {
     const int64_t nwarps = (int64_t)B * Cout;
     HSV_REQUIRE(nwarps * 32 / 256 + 1 < (1ll << 31), "conv1d_direct: grid too large");
     conv1d_vecdot_kernel<<<(unsigned)((nwarps * 32 + 255) / 256), 256, 0, st>>>(x, w, bias, out, B, Cin, Cout, flags);
-  } else if (Lout <= 8) {
+  } else if (Lout <= 8 && !valid_len) {   // (with valid_len, short items take the warp reduction inside the thin kernels)
     const int64_t nwarps = (int64_t)B * Cout * Lout;
     HSV_REQUIRE(nwarps * 32 / 256 + 1 < (1ll << 31), "conv1d_direct: grid too large");
     conv1d_rowdot_kernel<<<(unsigned)((nwarps * 32 + 255) / 256), 256, 0, st>>>(x, w, bias, out, B, Cin, Cout, Lin,
@@ -707,8 +837,8 @@ extern "C" int hsv_conv1d_direct(const float *x, const float *w, const float *bi
     dim3 grid((unsigned)((Lout + 511) / 512), (unsigned)B);
     const bool vec = pad == 3 && (Lin & 3) == 0 && Lout == Lin &&
                      ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
-    if (vec) conv1d_thin_vec_kernel<<<grid, 128, 0, st>>>(x, w, bias, out, Cin, Cout, Lin, Lout, flags);
-    else conv1d_thin_smem_kernel<7><<<grid, 256, 0, st>>>(x, w, bias, out, Cin, Cout, Lin, Lout, pad, flags);
+    if (vec) conv1d_thin_vec_kernel<<<grid, 128, 0, st>>>(x, w, bias, out, valid_len, Cin, Cout, Lin, Lout, flags);
+    else conv1d_thin_smem_kernel<7><<<grid, 256, 0, st>>>(x, w, bias, out, valid_len, Cin, Cout, Lin, Lout, pad, flags);
   } else if (Cout <= 4) {
     conv1d_thin_kernel<<<grid_for((int64_t)B * Lout, 256), 256, 0, st>>>(x, w, bias, out, B, Cin, Cout, Lin,
                                                                         Lout, k, d, pad, flags);
@@ -743,13 +873,19 @@ extern "C" int hsv_conv_transpose1d_direct(const float *x, const float *w, const
 
 extern "C" int hsv_sr_pre_interp(const float *x, const float *w, const float *bias, float *out, int B, int C,
                                  int64_t Lin, int64_t Lout, void *stream) {
+  return hsv_sr_pre_interp_ragged(x, w, bias, nullptr, nullptr, out, B, C, Lin, Lout, stream);
+}
+
+extern "C" int hsv_sr_pre_interp_ragged(const float *x, const float *w, const float *bias, const int32_t *valid_len_in,
+                                        const int32_t *valid_len_out, float *out, int B, int C, int64_t Lin,
+                                        int64_t Lout, void *stream) {
   if (B == 0) return HSV_OK;
   HSV_REQUIRE(x && w && out, "sr_pre_interp: null pointer");
   HSV_REQUIRE(C > 0 && Lin > 0 && Lout > 0, "sr_pre_interp: bad shape");
   if (B == 0) return HSV_OK;
   const float scale = (float)Lin / (float)Lout;  // ATen area_pixel_compute_scale, align_corners=False
-  sr_pre_interp_kernel<<<grid_for((int64_t)B * Lout, 256), 256, 0, hsv::as_stream(stream)>>>(x, w, bias, out, B,
-                                                                                            C, Lin, Lout, scale);
+  sr_pre_interp_kernel<<<grid_for((int64_t)B * Lout, 256), 256, 0, hsv::as_stream(stream)>>>(
+      x, w, bias, out, valid_len_in, valid_len_out, B, C, Lin, Lout, scale);
   return hsv::check_launch("sr_pre_interp");
 }
 
@@ -786,27 +922,35 @@ extern "C" int hsv_weight_norm_fold(const float *v, const float *g, float *w, in
   return hsv::check_launch("weight_norm_fold");
 }
 
+namespace {
+// the three pack entry points share one launch; `name` prefixes their argument errors
+int pack_blk16_launch(const char *name, const float *x1, const float *x2, const float *x3, const int32_t *valid_len,
+                      void *out, int B, int C, int64_t L, int lrelu, float in_scale, void *stream) {
+  if (B == 0 || L == 0) return HSV_OK;
+  HSV_REQUIRE(x1 && out, "%s: null pointer", name);
+  HSV_REQUIRE(x2 || !x3, "%s: x3 without x2", name);
+  HSV_REQUIRE(C > 0 && C % 16 == 0, "%s: C %% 16 != 0 (C=%d)", name, C);
+  HSV_REQUIRE(B <= 65535 && C / 8 <= 65535, "%s: grid too large", name);
+  pack_blk16_kernel<<<dim3((unsigned)((L + 255) / 256), (unsigned)(C / 8), (unsigned)B), 256, 0, hsv::as_stream(stream)>>>(
+      x1, x2, x3, valid_len, reinterpret_cast<uint4 *>(out), C, L, hsv::blk16_rows(L), lrelu, in_scale,
+      hsv::blk_cw(C));
+  return hsv::check_launch(name);
+}
+}  // namespace
+
 extern "C" int hsv_pack_blk16(const float *x, void *out, int B, int C, int64_t L, int lrelu, float in_scale,
                               void *stream) {
-  if (B == 0 || L == 0) return HSV_OK;
-  HSV_REQUIRE(x && out, "pack_blk16: null pointer");
-  HSV_REQUIRE(C > 0 && C % 16 == 0, "pack_blk16: C %% 16 != 0 (C=%d)", C);
-  HSV_REQUIRE(B <= 65535 && C / 8 <= 65535, "pack_blk16: grid too large");
-  pack_blk16_kernel<<<dim3((unsigned)((L + 255) / 256), (unsigned)(C / 8), (unsigned)B), 256, 0, hsv::as_stream(stream)>>>(
-      x, nullptr, nullptr, reinterpret_cast<uint4 *>(out), C, L, hsv::blk16_rows(L), lrelu, in_scale, hsv::blk_cw(C));
-  return hsv::check_launch("pack_blk16");
+  return pack_blk16_launch("pack_blk16", x, nullptr, nullptr, nullptr, out, B, C, L, lrelu, in_scale, stream);
 }
 
 extern "C" int hsv_pack_blk16_sum3(const float *x1, const float *x2, const float *x3, void *out, int B, int C,
                                    int64_t L, int lrelu, float in_scale, void *stream) {
-  if (B == 0 || L == 0) return HSV_OK;
-  HSV_REQUIRE(x1 && out, "pack_blk16_sum3: null pointer");
-  HSV_REQUIRE(x2 || !x3, "pack_blk16_sum3: x3 without x2");
-  HSV_REQUIRE(C > 0 && C % 16 == 0, "pack_blk16_sum3: C %% 16 != 0 (C=%d)", C);
-  HSV_REQUIRE(B <= 65535 && C / 8 <= 65535, "pack_blk16_sum3: grid too large");
-  pack_blk16_kernel<<<dim3((unsigned)((L + 255) / 256), (unsigned)(C / 8), (unsigned)B), 256, 0, hsv::as_stream(stream)>>>(
-      x1, x2, x3, reinterpret_cast<uint4 *>(out), C, L, hsv::blk16_rows(L), lrelu, in_scale, hsv::blk_cw(C));
-  return hsv::check_launch("pack_blk16_sum3");
+  return pack_blk16_launch("pack_blk16_sum3", x1, x2, x3, nullptr, out, B, C, L, lrelu, in_scale, stream);
+}
+
+extern "C" int hsv_pack_blk16_sum3_ragged(const float *x1, const float *x2, const float *x3, const int32_t *valid_len,
+                                          void *out, int B, int C, int64_t L, int lrelu, float in_scale, void *stream) {
+  return pack_blk16_launch("pack_blk16_sum3_ragged", x1, x2, x3, valid_len, out, B, C, L, lrelu, in_scale, stream);
 }
 
 extern "C" int hsv_unpack_blk16(const void *in, float *x, int B, int C, int64_t L, void *stream) {

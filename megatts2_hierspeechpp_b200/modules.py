@@ -274,6 +274,65 @@ FUSE_MAX_CHANNELS = [int(__import__("os").environ.get("HSV_FUSE_MAX_C", "0"))]
 # kernel), there the saved launch on the critical path is worth more than the slower in-CTA activation
 FUSE_MAX_ELEMS = [int(__import__("os").environ.get("HSV_FUSE_MAX_ELEMS", str(1 << 62)))]
 
+# ----------------------------------------------------------------------------------------------
+# ragged batches: utterances of different lengths padded to one T
+# ----------------------------------------------------------------------------------------------
+def _lengths_tensor(lengths, B: int, T: int, device) -> Optional[torch.Tensor]:
+    """``lengths`` (per utterance, in the module's input time units) as a contiguous int32 [B] tensor on ``device``.
+    A CUDA tensor is only checked for shape / device / dtype -- never read back, so the call stays free of host syncs and
+    capturable (the kernels clamp its values to the tensor length); a host sequence is range-checked (1 <= len <= T)."""
+    if lengths is None:
+        return None
+    device = torch.device(device)
+    if isinstance(lengths, torch.Tensor):
+        if lengths.device != device:
+            raise ValueError(f"lengths is on {lengths.device}, the input is on {device}")
+        if tuple(lengths.shape) != (B,):
+            raise ValueError(f"lengths must have shape ({B},), got {tuple(lengths.shape)}")
+        if lengths.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f"lengths must be int32 or int64, got {lengths.dtype}")
+        return lengths.to(torch.int32).contiguous()
+    vals = [int(v) for v in lengths]
+    if len(vals) != B:
+        raise ValueError(f"lengths has {len(vals)} entries for a batch of {B}")
+    bad = [v for v in vals if not 1 <= v <= T]
+    if bad:
+        raise ValueError(f"lengths must lie in [1, {T}], got {bad[:4]}")
+    return torch.tensor(vals, dtype=torch.int32, device=device)
+
+
+def _length_table(lengths, B: int, T: int, device, mults: Sequence[int]) -> Optional[torch.Tensor]:
+    """int32 [len(mults), B] on the device: row i = the valid lengths at the stage whose length is mults[i] x the input's
+    (computed once per forward; its rows are the ``valid_len`` of that stage's kernels)."""
+    ln = _lengths_tensor(lengths, B, T, device)
+    return None if ln is None else torch.stack([ln * m for m in mults])
+
+
+def _scale_lengths(lengths, m: int):
+    """``lengths`` in units m times finer (a device tensor stays on the device)."""
+    if lengths is None or isinstance(lengths, torch.Tensor):
+        return None if lengths is None else lengths * m
+    return [int(v) * m for v in lengths]
+
+
+def _frame_mask(vl: torch.Tensor, L: int) -> torch.Tensor:
+    """fp32 [B, L] 0/1 mask of the valid steps (the operand-writing conv epilogues multiply by it: v * 1.0f is exact)."""
+    return (torch.arange(L, device=vl.device, dtype=torch.int32).unsqueeze(0) < vl.unsqueeze(1)).float()
+
+
+def _vl(valid_len: Optional[torch.Tensor]) -> dict:
+    # the ops keep their unragged call when there are no lengths
+    return {} if valid_len is None else {"valid_len": valid_len}
+
+
+def _hops(rates: Sequence[int]) -> List[int]:
+    """Length of the input and of every up-sampling stage's output, in input steps."""
+    out = [1]
+    for u in rates:
+        out.append(out[-1] * u)
+    return out
+
+
 _MAIN_SLOT = 3   # blk16 workspace slot of the main stream (slots 0..2 belong to the per-resblock streams)
 _DB_SLOT = 15   # second operand workspace of the DBlock's conv chain
 _PRE_SLOT = 7    # ... of Generator.pre when Vocoder runs it beside the SourceNetwork (4..6: front.py, 8+: tests)
@@ -281,18 +340,21 @@ _PRE_SLOT = 7    # ... of Generator.pre when Vocoder runs it beside the SourceNe
 
 def _dense_conv(x: torch.Tensor, f: _Folded, k: int, d: int = 1, lrelu: bool = False,
                 residual: Optional[torch.Tensor] = None, slot: Optional[int] = None,
-                out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                out: Optional[torch.Tensor] = None, valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
     """'same' Conv1d of an fp32 [B,C,L] tensor: tcgen05 path when both channel counts are multiples of
     16 (pack to the fp16 operand layout, optional leaky_relu(0.1) fused into the pack), fp32 direct
-    kernel otherwise."""
+    kernel otherwise.  ``valid_len`` (int32 [B]): the operand is zero past each item's length, so the output below it
+    equals the item's own run (the output past it is not meaningful)."""
     B, C, L = x.shape
     cout = f.conv.out_channels
     if C % 16 == 0 and cout % 16 == 0 and ((k - 1) // 2) * d <= ops.BLK_PAD:
         buf = ops.blk16_buffer(B, C, L, x.device, _MAIN_SLOT if slot is None else slot)
-        ops.pack_blk16(x, buf, lrelu)
+        ops.pack_blk16(x, buf, lrelu, **_vl(valid_len))
         ops.check_saturation(buf, C, L)
         wp, nt = f.packed_weight(_row_tiles(B, L))
         return ops.conv1d_umma(buf, wp, f.bias(), L, C, cout, k, d, nt, residual=residual, out=out)
+    if valid_len is not None:
+        raise NotImplementedError("per-utterance lengths need channel counts that are multiples of 16 here")
     pad = ((k - 1) // 2) * d
     if residual is not None:
         if out is None:
@@ -305,18 +367,21 @@ def _dense_conv(x: torch.Tensor, f: _Folded, k: int, d: int = 1, lrelu: bool = F
 
 
 def _dense_convT(x: torch.Tensor, f: _Folded, k: int, u: int, add: Optional[torch.Tensor] = None,
-                 scale: float = 1.0) -> torch.Tensor:
+                 scale: float = 1.0, valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
     """ConvTranspose1d(k, stride u, padding (k-u)//2) of the fp32 [B,C,L] tensor ``x * scale`` (+ optional add).
     ``x`` may be the list of per-resblock outputs of the previous stage (``sum_of_blocks(..., separate=True)``): their
-    sum is taken inside the operand pack."""
+    sum is taken inside the operand pack.  ``valid_len`` (int32 [B], input steps): the operand is zero past each item's
+    length, so the output below u * length equals the item's own run."""
     B, C, L = (x[0] if isinstance(x, (list, tuple)) else x).shape
     cout = f.conv.out_channels
     if C % 16 == 0 and cout % 16 == 0:
         buf = ops.blk16_buffer(B, C, L, f.weight().device, _MAIN_SLOT)
-        ops.pack_blk16(x, buf, scale=scale)
+        ops.pack_blk16(x, buf, scale=scale, **_vl(valid_len))
         ops.check_saturation(buf, C, L)
         wp, nt = f.packedT_weight(u, _row_tiles(B, L))
         return ops.conv_transpose1d_umma(buf, wp, f.bias(), L, C, cout, k, u, nt, add=add)
+    if valid_len is not None:
+        raise NotImplementedError("per-utterance lengths need channel counts that are multiples of 16 here")
     if scale != 1.0 or isinstance(x, (list, tuple)):
         raise NotImplementedError("channel counts that are not multiples of 16 are not supported on this path")
     return ops.conv_transpose1d(x, f.weight(), f.bias(), u, add=add)
@@ -347,15 +412,18 @@ class AMPBlock1(nn.Module):
         _bump_on_load(self)
 
     def run(self, x: torch.Tensor, slot: int = 0, acc: Optional[torch.Tensor] = None, acc_mode: int = ops.ACC_NONE,
-            before_final=None) -> Optional[torch.Tensor]:
+            before_final=None, valid_len: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
         """x fp32 [B,C,L] (not modified).  Returns the block output, or None when the result is only
         accumulated into ``acc`` (sum over resblocks).  ``before_final`` is called right before the
-        last conv is enqueued (used to order accumulation across streams)."""
+        last conv is enqueued (used to order accumulation across streams).  ``valid_len`` (int32 [B]): item b is
+        x[b, :, :valid_len[b]]; the output below that equals the item's own run, past it it is not meaningful."""
         B, C, L = x.shape
         if C != self.channels or C % 16:
             raise ValueError(f"AMP block expects {self.channels} channels (multiple of 16), got {C}")
         k = self.kernel_size
         fused = C in ops.FUSED_CIN and C <= FUSE_MAX_CHANNELS[0] and B * C * L <= FUSE_MAX_ELEMS[0]
+        if fused and valid_len is not None:
+            raise NotImplementedError("the fused act+conv half-layer (HSV_FUSE_MAX_C) takes no per-utterance lengths")
         buf = None if fused else ops.blk16_buffer(B, C, L, x.device, slot)
         xt = torch.empty_like(x)
         cur = x
@@ -381,10 +449,10 @@ class AMPBlock1(nn.Module):
                 continue
             w1, nt1 = self._f1[i].packed_weight(_row_tiles(B, L))
             w2, nt2 = self._f2[i].packed_weight(_row_tiles(B, L))
-            ops.act1d_blk16(cur, *a1.params(), buf)
+            ops.act1d_blk16(cur, *a1.params(), buf, **_vl(valid_len))
             ops.check_saturation(buf, C, L)
             ops.conv1d_umma(buf, w1, self._f1[i].bias(), L, C, C, k, d, nt1, out=xt)
-            ops.act1d_blk16(xt, *a2.params(), buf)
+            ops.act1d_blk16(xt, *a2.params(), buf, **_vl(valid_len))
             ops.check_saturation(buf, C, L)
             if last and before_final is not None:
                 before_final()
@@ -417,7 +485,8 @@ SEPARATE_MAX_ELEMS = [1 << 23]
 _SEPARATE = [__import__("os").environ.get("HSV_SEPARATE_SUMS", "1") != "0"]   # A/B switch of the consumer-side resblock sums
 
 
-def sum_of_blocks(x: torch.Tensor, blocks: Sequence[AMPBlock1], parallel: bool = False, separate: bool = False):
+def sum_of_blocks(x: torch.Tensor, blocks: Sequence[AMPBlock1], parallel: bool = False, separate: bool = False,
+                  valid_len: Optional[torch.Tensor] = None):
     """(xs, scale) with xs = sum_j resblock_j(x) and scale = 1/num_kernels
     (hierspeechpp_speechsynthesizer.py:440-446).  The sum is accumulated in the epilogue of each block's
     last conv (store, then red.add in stream order: deterministic); the division is applied by the
@@ -426,10 +495,12 @@ def sum_of_blocks(x: torch.Tensor, blocks: Sequence[AMPBlock1], parallel: bool =
     ``separate=True`` (multi-stream mode only, up to three blocks): every block writes its own tensor and the LIST is
     returned; the consumer's operand pack adds them in the same fixed order ((x1 + x2) + x3, bit-identical to the
     chained accumulation, same bytes moved).  The last convs of the blocks then run concurrently instead of one
-    after the other: at batch 1 that chain was ~10 us at the end of every stage."""
+    after the other: at batch 1 that chain was ~10 us at the end of every stage.
+
+    ``valid_len`` (int32 [B]) is passed to every block (``AMPBlock1.run``)."""
     nk = len(blocks)
     if nk == 1:
-        return blocks[0].run(x), 1.0
+        return blocks[0].run(x, **_vl(valid_len)), 1.0
     if separate and parallel and nk <= 3 and _SEPARATE[0] and x.numel() <= SEPARATE_MAX_ELEMS[0]:
         main = torch.cuda.current_stream()
         fork = torch.cuda.Event()
@@ -440,7 +511,7 @@ def sum_of_blocks(x: torch.Tensor, blocks: Sequence[AMPBlock1], parallel: bool =
             s = streams[j]
             s.wait_event(fork)
             with torch.cuda.stream(s):
-                outs.append(blk.run(x, slot=j))
+                outs.append(blk.run(x, slot=j, **_vl(valid_len)))
                 ev = torch.cuda.Event()
                 ev.record(s)
             main.wait_event(ev)
@@ -449,7 +520,7 @@ def sum_of_blocks(x: torch.Tensor, blocks: Sequence[AMPBlock1], parallel: bool =
     modes = [ops.ACC_SET] + [ops.ACC_ADD] * (nk - 1)
     if not parallel:
         for j, blk in enumerate(blocks):
-            blk.run(x, slot=0, acc=xs, acc_mode=modes[j])
+            blk.run(x, slot=0, acc=xs, acc_mode=modes[j], **_vl(valid_len))
         return xs, 1.0 / nk
     # one stream per resblock; the accumulating epilogues are chained with events
     main = torch.cuda.current_stream()
@@ -463,7 +534,8 @@ def sum_of_blocks(x: torch.Tensor, blocks: Sequence[AMPBlock1], parallel: bool =
         with torch.cuda.stream(s):
             prev = done[j - 1] if j > 0 else None
             blk.run(x, slot=j, acc=xs, acc_mode=modes[j],
-                    before_final=(lambda p=prev, st=s: st.wait_event(p)) if prev is not None else None)
+                    before_final=(lambda p=prev, st=s: st.wait_event(p)) if prev is not None else None,
+                    **_vl(valid_len))
             done[j].record(s)
     for ev in done:
         main.wait_event(ev)
@@ -499,15 +571,17 @@ class DBlock(nn.Module):
         self._fc = [_Folded(c) for c in self.conv]
         _bump_on_load(self)
 
-    def forward(self, x, side=None):
+    def forward(self, x, side=None, *, valid_len: Optional[torch.Tensor] = None):
         """``side`` = (stream, workspace slot): run the residual 1x1 conv there, beside the first two convs of the
-        main branch (it is only needed by the third)."""
+        main branch (it is only needed by the third).  ``valid_len`` (int32 [B], OUTPUT steps, i.e. input steps /
+        factor): the output below it equals each item's own run."""
         x = _as_input(x)
         size = x.shape[-1] // self.factor
         # nearest down-sampling commutes with the 1x1 conv: gather first (4x less work, same values)
         xd = ops.nearest_gather(x, size)
+        mask = None if valid_len is None else _frame_mask(valid_len, size)
         if side is None:
-            res = _dense_conv(xd, self._fr, 1)
+            res = _dense_conv(xd, self._fr, 1, valid_len=valid_len)
             ready = None
         else:
             st, slot = side
@@ -517,7 +591,7 @@ class DBlock(nn.Module):
             fork.record(main)
             st.wait_event(fork)
             with torch.cuda.stream(st):
-                _dense_conv(xd, self._fr, 1, slot=slot, out=res)
+                _dense_conv(xd, self._fr, 1, slot=slot, out=res, valid_len=valid_len)
                 ready.record(st)
         B, cin, L = xd.shape
         hid = self.conv[0].out_channels
@@ -526,14 +600,15 @@ class DBlock(nn.Module):
             # fp16 operand (leaky_relu applied in the epilogue)
             rt = _row_tiles(B, L)
             b0 = ops.blk16_buffer(B, cin, L, xd.device, _MAIN_SLOT)
-            ops.pack_blk16(xd, b0, True)
+            ops.pack_blk16(xd, b0, True, **_vl(valid_len))
             ops.check_saturation(b0, cin, L)
             b1 = ops.blk16_buffer(B, hid, L, xd.device, _MAIN_SLOT)
             b2 = ops.blk16_buffer(B, hid, L, xd.device, _DB_SLOT)
+            # with lengths, the mask gives each operand the zero tail of the item's own run
             w0, n0 = self._fc[0].packed_weight(rt)
-            ops.conv1d_umma_blk(b0, w0, self._fc[0].bias(), L, cin, hid, 3, 1, n0, b1, ops.BLK_LRELU)
+            ops.conv1d_umma_blk(b0, w0, self._fc[0].bias(), L, cin, hid, 3, 1, n0, b1, ops.BLK_LRELU, mask=mask)
             w1, n1 = self._fc[1].packed_weight(rt)
-            ops.conv1d_umma_blk(b1, w1, self._fc[1].bias(), L, hid, hid, 3, 2, n1, b2, ops.BLK_LRELU)
+            ops.conv1d_umma_blk(b1, w1, self._fc[1].bias(), L, hid, hid, 3, 2, n1, b2, ops.BLK_LRELU, mask=mask)
             ops.check_saturation(b2, hid, L)
             if ready is not None:
                 torch.cuda.current_stream().wait_event(ready)
@@ -543,7 +618,7 @@ class DBlock(nn.Module):
         for i, d in enumerate((1, 2, 4)):
             if i == 2 and ready is not None:
                 torch.cuda.current_stream().wait_event(ready)
-            h = _dense_conv(h, self._fc[i], 3, d, lrelu=True, residual=res if i == 2 else None)
+            h = _dense_conv(h, self._fc[i], 3, d, lrelu=True, residual=res if i == 2 else None, valid_len=valid_len)
         return h
 
     def remove_weight_norm(self):
@@ -559,11 +634,16 @@ class _VocoderBase(nn.Module):
         super().__init__()
         _bump_on_load(self)
 
-    def _stage(self, x, i, separate: bool = False):
+    def _stage(self, x, i, separate: bool = False, valid_len: Optional[torch.Tensor] = None):
         """``separate``: the consumer of this stage is an operand pack (the next stage's ConvTranspose1d), which can
         take the per-resblock tensors as a list."""
         nk = self.num_kernels
-        return sum_of_blocks(x, [self.resblocks[i * nk + j] for j in range(nk)], self.parallel_blocks, separate)
+        return sum_of_blocks(x, [self.resblocks[i * nk + j] for j in range(nk)], self.parallel_blocks, separate,
+                             valid_len)
+
+    def _length_table(self, lengths, x: torch.Tensor) -> Optional[torch.Tensor]:
+        """Valid lengths of the input and of every up-sampling stage's output (rows of an int32 [stages + 1, B])."""
+        return _length_table(lengths, x.shape[0], x.shape[-1], x.device, _hops(self.upsample_rates))
 
 
 class SourceNetwork(_VocoderBase):
@@ -599,20 +679,27 @@ class SourceNetwork(_VocoderBase):
         self._f_post = _Folded(self.conv_post)
         self._f_cond = _Folded(self.cond)
 
-    def forward(self, x, g, need_pred: bool = True):
+    def forward(self, x, g, need_pred: bool = True, *, lengths=None):
         """Returns (e, e_) like the reference (:290-308).  ``need_pred=False`` skips the f0 predictor
-        ``conv_post`` (e_ is returned as None): ``Generator`` only consumes the hidden state e."""
+        ``conv_post`` (e_ is returned as None): ``Generator`` only consumes the hidden state e.
+
+        ``lengths`` (frames of x per utterance: int CUDA tensor [B] or host sequence): a padded batch of utterances of
+        different lengths; item b's outputs below 4 * lengths[b] equal its own unpadded run, the rest is 0."""
         x, g = _as_input(x), _as_input(g)
-        xp = _dense_conv(x, self._f_pre, 7)
+        V = self._length_table(lengths, x)
+        vl = (lambda i: None) if V is None else (lambda i: V[i])
+        xp = _dense_conv(x, self._f_pre, 7, valid_len=vl(0))
         cg = ops.conv1d_direct(g, self._f_cond.weight(), self._f_cond.bias())
         x = ops.add3_bcast(xp, None, cg, out=xp)
         sc = 1.0
         for i in range(self.num_upsamples):
-            x = _dense_convT(x, self._f_ups[i], self.ups[i].kernel_size[0], self.upsample_rates[i], scale=sc)
-            x, sc = self._stage(x, i, separate=i < self.num_upsamples - 1)
+            x = _dense_convT(x, self._f_ups[i], self.ups[i].kernel_size[0], self.upsample_rates[i], scale=sc,
+                             valid_len=vl(i))
+            x, sc = self._stage(x, i, separate=i < self.num_upsamples - 1, valid_len=vl(i + 1))
         self.activation_post.check_filters()
-        x = ops.act1d(x, *self.activation_post.params(), scale=sc)
-        x_ = ops.conv1d_direct(x, self._f_post.weight(), None, pad=3) if need_pred else None
+        n = self.num_upsamples
+        x = ops.act1d(x, *self.activation_post.params(), scale=sc, **_vl(vl(n)))
+        x_ = ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, **_vl(vl(n))) if need_pred else None
         return x, x_
 
 
@@ -649,20 +736,26 @@ class Generator(_VocoderBase):
         self._f_cond = _Folded(self.cond) if gin_channels != 0 else None
         self._f_proj = _Folded(self.proj)
 
-    def pre(self, x, g, out=None, slot: Optional[int] = None):
+    def pre(self, x, g, out=None, slot: Optional[int] = None, valid_len: Optional[torch.Tensor] = None):
         """``conv_pre(x)`` and ``cond(g)`` (:428, :430): the part of forward that does not need the pitch hidden state,
         so ``Vocoder`` can run it beside the SourceNetwork.  ``out`` = (xp, cg) preallocated by the caller."""
         x, g = _as_input(x), _as_input(g)
-        xp = _dense_conv(x, self._f_pre, 7, slot=slot, out=None if out is None else out[0])
+        xp = _dense_conv(x, self._f_pre, 7, slot=slot, out=None if out is None else out[0], valid_len=valid_len)
         cg = ops.conv1d_direct(g, self._f_cond.weight(), self._f_cond.bias(), out=None if out is None else out[1])
         return xp, cg
 
-    def forward(self, x, pitch, g=None, _pre=None):
+    def forward(self, x, pitch, g=None, _pre=None, *, lengths=None, _table=None):
+        """``lengths`` (frames of x per utterance: int CUDA tensor [B] or host sequence): a padded batch of utterances
+        of different lengths (pitch: the SourceNetwork's hidden state of the same batch); item b's waveform below
+        prod(upsample_rates) * lengths[b] equals its own unpadded run, the rest is 0.  ``_table``: the length table
+        ``vocode`` already built for ``_pre``."""
         x, pitch = _as_input(x), _as_input(pitch)
         if g is None:
             # the reference evaluates self.cond(g) unconditionally (:430) and fails on g=None
             raise ValueError("Generator.forward needs the speaker embedding g")
-        xp, cg = self.pre(x, g) if _pre is None else _pre
+        V = _table if _table is not None else self._length_table(lengths, x)
+        vl = (lambda i: None) if V is None else (lambda i: V[i])
+        xp, cg = self.pre(x, g, valid_len=vl(0)) if _pre is None else _pre
         proj = proj_ready = None
         if self.parallel_blocks and _PRE_OVERLAP[0]:
             # multi-stream mode: proj(pitch) (:437) and the DBlock's residual conv run beside the DBlock's main branch
@@ -674,27 +767,28 @@ class Generator(_VocoderBase):
             fork.record(main)
             s0.wait_event(fork)
             with torch.cuda.stream(s0):
-                _dense_conv(pitch, self._f_proj, 7, slot=0, out=proj)
+                _dense_conv(pitch, self._f_proj, 7, slot=0, out=proj, valid_len=vl(1))
                 proj_ready.record(s0)
-            dn = self.downs(pitch, side=(s1, 1))
+            dn = self.downs(pitch, side=(s1, 1), valid_len=vl(0))
         else:
-            dn = self.downs(pitch)
+            dn = self.downs(pitch, valid_len=vl(0))
         x = ops.add3_bcast(xp, dn, cg, out=xp)
         sc = 1.0
         for i in range(self.num_upsamples):
             add = None
             if i == 0:
                 if proj is None:
-                    add = _dense_conv(pitch, self._f_proj, 7)
+                    add = _dense_conv(pitch, self._f_proj, 7, valid_len=vl(1))
                 else:
                     torch.cuda.current_stream().wait_event(proj_ready)
                     add = proj
             x = _dense_convT(x, self._f_ups[i], self.ups[i].kernel_size[0], self.upsample_rates[i], add=add,
-                             scale=sc)
-            x, sc = self._stage(x, i, separate=i < self.num_upsamples - 1)
+                             scale=sc, valid_len=vl(i))
+            x, sc = self._stage(x, i, separate=i < self.num_upsamples - 1, valid_len=vl(i + 1))
         self.activation_post.check_filters()
-        x = ops.act1d(x, *self.activation_post.params(), scale=sc)
-        return ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, flags=ops.CONV_TANH)
+        n = self.num_upsamples
+        x = ops.act1d(x, *self.activation_post.params(), scale=sc, **_vl(vl(n)))
+        return ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, flags=ops.CONV_TANH, **_vl(vl(n)))
 
     def remove_weight_norm(self):
         for l in self.ups:
@@ -739,16 +833,24 @@ class SpeechSRGenerator(_VocoderBase):
         self._f_pre = _Folded(self.conv_pre)
         self._f_post = _Folded(self.conv_post)
 
-    def forward(self, x, g=None):
+    def forward(self, x, g=None, *, lengths=None):
+        """``lengths`` (input samples per utterance: int CUDA tensor [B] or host sequence): a padded batch of utterances
+        of different lengths; item b's output below int(lengths[b] * scale) equals its own unpadded run, the rest is 0."""
         if g is not None:
             raise NotImplementedError("SpeechSR is unconditional in the reference (gin_channels=0)")
         x = _as_input(x)
         L = x.shape[-1]
-        x = ops.sr_pre_interp(x, self._f_pre.weight(), self._f_pre.bias(), int(L * self.scale))
-        x, sc = self._stage(x, 0)
+        ln = _lengths_tensor(lengths, x.shape[0], L, x.device)
+        vin = vout = None
+        if ln is not None:
+            # int(L * 1.5) == (3 L) // 2 and int(L * 3) == 3 L, in integer arithmetic on the device
+            vin, vout = ln, (ln * 3 // 2 if self.scale == 1.5 else ln * int(self.scale))
+        x = ops.sr_pre_interp(x, self._f_pre.weight(), self._f_pre.bias(), int(L * self.scale),
+                              **_vl(None if ln is None else (vin, vout)))
+        x, sc = self._stage(x, 0, valid_len=vout)
         self.activation_post.check_filters()
-        x = ops.act1d(x, *self.activation_post.params(), scale=sc)
-        return ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, flags=ops.CONV_TANH)
+        x = ops.act1d(x, *self.activation_post.params(), scale=sc, **_vl(vout))
+        return ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, flags=ops.CONV_TANH, **_vl(vout))
 
     def remove_weight_norm(self):
         for l in self.resblocks:
@@ -784,8 +886,8 @@ class _SpeechSRSynthesizer(nn.Module):
         self.dec = self._gen_cls(1, resblock, resblock_kernel_sizes, resblock_dilation_sizes, upsample_rates,
                                  upsample_initial_channel, upsample_kernel_sizes)
 
-    def forward(self, x):
-        return self.dec(x)
+    def forward(self, x, *, lengths=None):
+        return self.dec(x, lengths=lengths)
 
     @torch.no_grad()
     def infer(self, x, max_len=None):
@@ -800,17 +902,18 @@ class SpeechSR48(_SpeechSRSynthesizer):
     _gen_cls = SpeechSR48Generator
 
 
-def vocode(sn: "SourceNetwork", dec: "Generator", z, g, need_pred: bool = False):
+def vocode(sn: "SourceNetwork", dec: "Generator", z, g, need_pred: bool = False, *, lengths=None):
     """``e, e_ = sn(z, g); return dec(z, e, g), e_`` (hierspeechpp_speechsynthesizer.py:648-649, :697-698).
 
     In multi-stream mode (``dec.parallel_blocks``) ``dec.conv_pre(z)`` and ``dec.cond(g)``, which do not depend on the
     SourceNetwork, run beside it on their own stream and operand workspace slot; their outputs are allocated on the
-    caller's stream."""
+    caller's stream.  ``lengths``: frames of z per utterance (see ``Generator.forward``)."""
     if not (dec.parallel_blocks and z.is_cuda and _PRE_OVERLAP[0]):
-        e, e_ = sn(z, g, need_pred=need_pred)
-        return dec(z, e, g=g), e_
+        e, e_ = sn(z, g, need_pred=need_pred, lengths=lengths)
+        return dec(z, e, g=g, lengths=lengths), e_
     z_, g_ = _as_input(z), _as_input(g)
     B, _, T = z_.shape
+    V = dec._length_table(lengths, z_)
     c0 = dec.conv_pre.out_channels
     xp = torch.empty(B, c0, T, dtype=torch.float32, device=z_.device)
     cg = torch.empty(B, c0, 1, dtype=torch.float32, device=z_.device)
@@ -820,11 +923,11 @@ def vocode(sn: "SourceNetwork", dec: "Generator", z, g, need_pred: bool = False)
     fork.record(main)
     side.wait_event(fork)
     with torch.cuda.stream(side):
-        dec.pre(z_, g_, out=(xp, cg), slot=_PRE_SLOT)
+        dec.pre(z_, g_, out=(xp, cg), slot=_PRE_SLOT, valid_len=None if V is None else V[0])
         done.record(side)
-    e, e_ = sn(z_, g_, need_pred=need_pred)
+    e, e_ = sn(z_, g_, need_pred=need_pred, lengths=None if V is None else V[0])
     main.wait_event(done)
-    return dec(z_, e, g=g_, _pre=(xp, cg)), e_
+    return dec(z_, e, g=g_, _pre=(xp, cg), _table=V), e_
 
 
 class Vocoder(nn.Module):
@@ -839,8 +942,10 @@ class Vocoder(nn.Module):
         self.dec = Generator(**c)
         self.sn = SourceNetwork(c["upsample_initial_channel"] // 2)
 
-    def forward(self, z, g):
-        return vocode(self.sn, self.dec, z, g)[0]
+    def forward(self, z, g, lengths=None):
+        """``lengths`` (frames of z per utterance: int CUDA tensor [B] or host sequence): a padded batch of utterances of
+        different lengths; item b's waveform [:320 * lengths[b]] equals its own unpadded run, the rest is 0."""
+        return vocode(self.sn, self.dec, z, g, lengths=lengths)[0]
 
 
 class VocoderSR(nn.Module):
@@ -862,9 +967,12 @@ class VocoderSR(nn.Module):
         self.sr = (SpeechSR24 if which == 24 else SpeechSR48)(100, 40, **SR_CFG)
         self.which = which
 
-    def forward(self, z, g, pcm16: bool = False):
-        wav16 = self.vocoder(z, g)
-        out = self.sr(wav16)
+    def forward(self, z, g, pcm16: bool = False, lengths=None):
+        """``lengths``: frames of z per utterance (see ``Vocoder.forward``); the padding of each output row is 0, which
+        leaves its per-utterance PCM peak unchanged."""
+        wav16 = self.vocoder(z, g, lengths=lengths)
+        hop = _hops(self.vocoder.dec.upsample_rates)[-1]
+        out = self.sr(wav16, lengths=_scale_lengths(lengths, hop))
         if pcm16:
             from .runtime import to_pcm16
             return to_pcm16(out, per_utterance=True)

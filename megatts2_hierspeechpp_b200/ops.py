@@ -108,39 +108,57 @@ def clear_workspace():
     WORKSPACE_EPOCH[0] += 1
 
 
+def _req_len(valid_len: Optional[torch.Tensor], B: int, device, name: str = "valid_len"):
+    """Per-item valid lengths of a ragged batch: a contiguous int32 CUDA tensor [B] on the data's device (values are
+    clamped to [0, L] by the kernels)."""
+    if valid_len is None:
+        return
+    _req(valid_len, name, torch.int32, 1)
+    if valid_len.numel() != B:
+        raise ValueError(f"{name}: expected {B} elements, got {valid_len.numel()}")
+    if valid_len.device != torch.device(device):
+        raise ValueError(f"{name}: on {valid_len.device}, the data is on {device}")
+
+
 def act1d(x: torch.Tensor, alpha: torch.Tensor, beta: torch.Tensor, out: Optional[torch.Tensor] = None,
-          scale: float = 1.0):
-    """Fused Activation1d(SnakeBeta) of ``x * scale``: fp32 [B,C,L] -> fp32 [B,C,L]."""
+          scale: float = 1.0, valid_len: Optional[torch.Tensor] = None):
+    """Fused Activation1d(SnakeBeta) of ``x * scale``: fp32 [B,C,L] -> fp32 [B,C,L].  ``valid_len`` (int32 [B]): item b
+    is its first valid_len[b] steps, as if run alone; the rest of its output is 0 and the rest of its input unread."""
     _req(x, "x", ndim=3); _req(alpha, "alpha"); _req(beta, "beta")
     B, C, L = x.shape
     if alpha.numel() != C or beta.numel() != C:
         raise ValueError(f"alpha/beta must have {C} elements")
+    _req_len(valid_len, B, x.device)
     if out is None:
         out = torch.empty_like(x)
     else:
         _req(out, "out", ndim=3)
     lib = _lib.load()
-    _lib.check(lib.hsv_act1d_snakebeta(_p(x), _p(out), _p(alpha), _p(beta), B, C, L, 0, float(scale), _stream()),
-               "hsv_act1d_snakebeta")
+    _lib.check(lib.hsv_act1d_snakebeta_ragged(_p(x), _p(out), _p(alpha), _p(beta), _p(valid_len), B, C, L, 0,
+                                              float(scale), _stream()), "hsv_act1d_snakebeta")
     return out
 
 
-def act1d_blk16(x: torch.Tensor, alpha: torch.Tensor, beta: torch.Tensor, buf: torch.Tensor, scale: float = 1.0):
-    """Fused Activation1d(SnakeBeta) of ``x * scale``: fp32 [B,C,L] -> fp16 blk16 operand (into ``buf``)."""
+def act1d_blk16(x: torch.Tensor, alpha: torch.Tensor, beta: torch.Tensor, buf: torch.Tensor, scale: float = 1.0,
+                valid_len: Optional[torch.Tensor] = None):
+    """Fused Activation1d(SnakeBeta) of ``x * scale``: fp32 [B,C,L] -> fp16 blk16 operand (into ``buf``).
+    ``valid_len``: as ``act1d`` (operand rows past an item's length are written as zero)."""
     _req(x, "x", ndim=3); _req(alpha, "alpha"); _req(beta, "beta"); _req(buf, "buf", torch.float16, 4)
     B, C, L = x.shape
     if tuple(buf.shape) != blk16_shape(B, C, L):
         raise ValueError(f"blk16 buffer shape {tuple(buf.shape)} does not match x {tuple(x.shape)}")
+    _req_len(valid_len, B, x.device)
     lib = _lib.load()
-    _lib.check(lib.hsv_act1d_snakebeta(_p(x), _p(buf), _p(alpha), _p(beta), B, C, L, 1, float(scale), _stream()),
-               "hsv_act1d_snakebeta")
+    _lib.check(lib.hsv_act1d_snakebeta_ragged(_p(x), _p(buf), _p(alpha), _p(beta), _p(valid_len), B, C, L, 1,
+                                              float(scale), _stream()), "hsv_act1d_snakebeta")
     return buf
 
 
-def pack_blk16(x, buf: torch.Tensor, lrelu: bool = False, scale: float = 1.0):
+def pack_blk16(x, buf: torch.Tensor, lrelu: bool = False, scale: float = 1.0, valid_len: Optional[torch.Tensor] = None):
     """fp32 [B,C,L] -> fp16 blk16 operand of ``x * scale`` (optionally leaky_relu(0.1) of it).  ``x`` may be a list of up
     to three equally shaped tensors: the operand is then ``((x1 + x2) + x3) * scale`` (the sum over a stage's resblocks
-    taken by the consumer, ``modules.sum_of_blocks(..., separate=True)``)."""
+    taken by the consumer, ``modules.sum_of_blocks(..., separate=True)``).  ``valid_len`` (int32 [B]): operand rows at
+    t >= valid_len[b] are written as zero without reading x."""
     xs = list(x) if isinstance(x, (list, tuple)) else [x]
     if not 1 <= len(xs) <= 3:
         raise ValueError("pack_blk16: one to three addends")
@@ -153,7 +171,12 @@ def pack_blk16(x, buf: torch.Tensor, lrelu: bool = False, scale: float = 1.0):
     if tuple(buf.shape) != blk16_shape(B, C, L):
         raise ValueError("blk16 buffer shape mismatch")
     lib = _lib.load()
-    if len(xs) == 1:
+    if valid_len is not None:
+        _req_len(valid_len, B, xs[0].device)
+        xs = xs + [None] * (3 - len(xs))
+        _lib.check(lib.hsv_pack_blk16_sum3_ragged(_p(xs[0]), _p(xs[1]), _p(xs[2]), _p(valid_len), _p(buf), B, C, L,
+                                                  int(lrelu), float(scale), _stream()), "hsv_pack_blk16_sum3_ragged")
+    elif len(xs) == 1:
         _lib.check(lib.hsv_pack_blk16(_p(xs[0]), _p(buf), B, C, L, int(lrelu), float(scale), _stream()), "hsv_pack_blk16")
     else:
         _lib.check(lib.hsv_pack_blk16_sum3(_p(xs[0]), _p(xs[1]), _p(xs[2]) if len(xs) == 3 else None, _p(buf), B, C, L,
@@ -438,7 +461,9 @@ def conv_transpose1d_umma(a_blk: torch.Tensor, w_packed: torch.Tensor, bias: Opt
 
 
 def conv1d_direct(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], d: int = 1, pad: int = 0,
-                  flags: int = 0, out: Optional[torch.Tensor] = None):
+                  flags: int = 0, out: Optional[torch.Tensor] = None, valid_len: Optional[torch.Tensor] = None):
+    """fp32 Conv1d on CUDA cores.  ``valid_len`` (int32 [B], conv_post shapes only: Cout <= 4, k = 7, pad = 3): item b
+    reads x[..., :valid_len[b]] only and its output past that is 0."""
     _req(x, "x", ndim=3); _req(w, "w", ndim=3)
     if bias is not None:
         _req(bias, "bias")
@@ -455,9 +480,14 @@ def conv1d_direct(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor]
         _req(out, "out", ndim=3)
         if tuple(out.shape) != (B, cout, Lout):
             raise ValueError("out shape mismatch")
+    _req_len(valid_len, B, x.device)
     lib = _lib.load()
-    _lib.check(lib.hsv_conv1d_direct(_p(x), _p(w), _p(bias), _p(out), B, cin, cout, Lin, Lout, k, d, pad, flags,
-                                     _stream()), "hsv_conv1d_direct")
+    if valid_len is not None:
+        _lib.check(lib.hsv_conv1d_direct_ragged(_p(x), _p(w), _p(bias), _p(valid_len), _p(out), B, cin, cout, Lin, Lout,
+                                                k, d, pad, flags, _stream()), "hsv_conv1d_direct_ragged")
+    else:
+        _lib.check(lib.hsv_conv1d_direct(_p(x), _p(w), _p(bias), _p(out), B, cin, cout, Lin, Lout, k, d, pad, flags,
+                                         _stream()), "hsv_conv1d_direct")
     return out
 
 
@@ -481,7 +511,10 @@ def conv_transpose1d(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tens
     return out
 
 
-def sr_pre_interp(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], Lout: int):
+def sr_pre_interp(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], Lout: int,
+                  valid_len: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+    """SpeechSR conv_pre + linear interpolation to Lout.  ``valid_len`` = (len_in, len_out), int32 [B] each: item b is
+    interpolated from len_in[b] to len_out[b] samples as if run alone; its output past len_out[b] is 0."""
     _req(x, "x", ndim=3); _req(w, "w", ndim=3)
     B, one, Lin = x.shape
     C = w.shape[0]
@@ -489,7 +522,14 @@ def sr_pre_interp(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor]
         raise ValueError("sr_pre_interp expects x [B,1,L] and w [C,1,7]")
     out = torch.empty(B, C, Lout, dtype=torch.float32, device=x.device)
     lib = _lib.load()
-    _lib.check(lib.hsv_sr_pre_interp(_p(x), _p(w), _p(bias), _p(out), B, C, Lin, Lout, _stream()), "hsv_sr_pre_interp")
+    if valid_len is not None:
+        vin, vout = valid_len
+        _req_len(vin, B, x.device, "valid_len[0]"); _req_len(vout, B, x.device, "valid_len[1]")
+        _lib.check(lib.hsv_sr_pre_interp_ragged(_p(x), _p(w), _p(bias), _p(vin), _p(vout), _p(out), B, C, Lin, Lout,
+                                                _stream()), "hsv_sr_pre_interp_ragged")
+    else:
+        _lib.check(lib.hsv_sr_pre_interp(_p(x), _p(w), _p(bias), _p(out), B, C, Lin, Lout, _stream()),
+                   "hsv_sr_pre_interp")
     return out
 
 

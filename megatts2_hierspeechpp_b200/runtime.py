@@ -158,6 +158,24 @@ def bucket_by_length(indices: Sequence[int], lengths: Sequence[int], max_batch: 
     return out
 
 
+def ragged_batches(indices: Sequence[int], lengths: Sequence[int], max_batch: int,
+                   frame_multiple: int = 50) -> List[Tuple[List[int], int]]:
+    """Micro-batches of utterances of different lengths for the ``lengths=`` path of the vocoder / SpeechSR modules:
+    [(ids, T_padded)], sorted longest first and cut into consecutive runs of at most ``max_batch``; each batch is padded
+    to its longest utterance rounded up to a multiple of ``frame_multiple``, which bounds the number of distinct
+    padded shapes (one captured CUDA graph each) while keeping the padded fraction small.  Deterministic (ties keep
+    index order); the batches partition ``indices``."""
+    if max_batch < 1 or frame_multiple < 1:
+        raise ValueError("max_batch and frame_multiple must be >= 1")
+    order = sorted(indices, key=lambda i: (-int(lengths[i]), i))
+    out = []
+    for s in range(0, len(order), max_batch):
+        ids = order[s:s + max_batch]
+        longest = int(lengths[ids[0]])
+        out.append((ids, -(-longest // frame_multiple) * frame_multiple))
+    return out
+
+
 def gather_packed(flat: torch.Tensor, dst: int = 0):
     """The collective under ``gather_waveforms``: every rank contributes one 1-D buffer of the SAME size and dtype
     (pad to the largest shard), rank ``dst`` gets a [world, n] tensor, the others None.  No metadata exchange, no
