@@ -121,6 +121,14 @@ int hsv_pack_conv_weight(const float *w, void *packed, int Cout, int Cin, int k,
 int hsv_conv1d_umma(const void *a_blk16, const void *w_packed, const float *bias,
                     const float *residual, float *out, float *acc, int acc_mode, float acc_div,
                     int B, int Cin, int Cout, int64_t L, int k, int d, int n_tile, void *stream);
+/* The same with an explicit batch stride of the operand: a_bchunks = operand chunks (CW channels x
+ * hsv_blk16_rows(L) rows each) from one batch item to the next (0 = Cin / CW, a dense buffer).  A channel
+ * range [c0, c0 + Cin) of a wider blk16 buffer with the same CW is then read in place at any batch size:
+ * a_blk16 = the buffer + the byte offset of chunk c0 / CW of item 0, a_bchunks = the wider buffer's chunks
+ * per item (split-K passes over one packed operand).  Results equal a dense copy of the range, bit for bit. */
+int hsv_conv1d_umma_astride(const void *a_blk16, int64_t a_bchunks, const void *w_packed, const float *bias,
+                            const float *residual, float *out, float *acc, int acc_mode, int B, int Cin, int Cout,
+                            int64_t L, int k, int d, int n_tile, void *stream);
 
 /* hsv_conv1d_umma_blk16: the same convolution with an OPERAND-WRITING epilogue: (conv + bias + bc[b]) -> activation ->
  * * mask -> fp16 blk16 buffer that the next hsv_conv1d_umma reads (no fp32 round trip, no pack launch).
@@ -269,7 +277,9 @@ int hsv_peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws, int rows, 
  *   commons.py:108-114);  2: gelu_tanh(x) * mask (FFN_Conv, modules.py:382-388);  3: mish(x) * mask (styleencoder.py:6-10)
  *   x_channels = channels per batch item of x (a channel prefix of a wider tensor can be packed).
  * hsv_ln_mod_blk16: LayerNorm over channels (eps, no affine) [* mask] -> x*(1+scale[b,c]) + shift[b,c] (modules.py:346,
- *   405-410); inmask: x*mask first; premask: normalised*mask before the modulation; mod_stride = batch stride of shift/scale.
+ *   405-410); inmask: x*mask first; premask bit 0: normalised*mask before the modulation, bit 1 (HSV_LN_ZERO_MASKED):
+ *   operand rows where mask == 0 are written as zero (the rows past an item of a ragged batch, which its own run
+ *   does not have: a following k > 1 conv then sees its zero padding); mod_stride = batch stride of shift/scale.
  * hsv_frame_op: element-wise ops (op codes in csrc/frame_ops.cu): 1 wn_res, 2 wn_last, 3 gate_add, 4 couple, 5 sample,
  *   6 mask, 7 add, 8 glu_res, 9 mish, 10 flip, 11 add_bcast.
  * hsv_mha: softmax(q k^T * scale) v per (batch, head); q/k/v channel-major [heads*D, T] with batch strides (so the fused
@@ -284,6 +294,7 @@ int hsv_pack_blk16_act(const float *x, const float *bcast, const float *mask, vo
  * output += rs[:, C:], blk = fp16 blk16 operand of the new x.  rs is [B, 2C, T]. */
 int hsv_wn_res_pack(float *x, const float *rs, const float *mask, float *output, void *blk, int B, int C, int64_t L,
                     void *stream);
+#define HSV_LN_ZERO_MASKED 2
 int hsv_ln_mod_blk16(const float *x, const float *shift, const float *scale, const float *mask, void *out, int B, int C,
                      int64_t L, float eps, int inmask, int premask, int64_t mod_stride, void *stream);
 /* hsv_gate_ln_mod_blk16: x = x + gate[b,c] * y * mask (in place, modules.py:408-409) fused with hsv_ln_mod_blk16 of the new x:
@@ -300,11 +311,31 @@ int hsv_mha(const float *q, const float *k, const float *v, float *out, const in
 int hsv_mha_blk16(const float *q, const float *k, const float *v, void *out_blk16, const int *lens, int B, int heads, int D,
                   int Tq, int Tk, int64_t q_bstride, int64_t k_bstride, int64_t v_bstride, float scale, int prescale_q,
                   void *stream);
+/* hsv_mha (out_mode 0) / hsv_mha_blk16 (out_mode 1) for a ragged batch of self-attention (Tq == Tk, lens NULL):
+ *   valid_len [B] int32, device (NULL = as hsv_mha / hsv_mha_blk16), clamped to [0, Tk].  Item b has n = valid_len[b]
+ *   queries and keys stored with row pitch Tk; it runs as its own launch with Tq = Tk = n (keys past n are never read
+ *   and weigh nothing), so out[b, :, :n] equals that launch bit for bit, and its rows [n, Tq) are written as 0 in
+ *   both out modes.  Unlike lens (masked_fill(-1e4) over the padded length), the padding does not take part at all.
+ *   Tensor-core kernel only: returns HSV_ERR_ARG with valid_len under hsv_set_mha_variant(1). */
+int hsv_mha_ragged(const float *q, const float *k, const float *v, void *out, int out_mode, const int *lens,
+                   const int32_t *valid_len, int B, int heads, int D, int Tq, int Tk, int64_t q_bstride,
+                   int64_t k_bstride, int64_t v_bstride, float scale, int prescale_q, void *stream);
 /* test hook: 0 = tensor-core attention (csrc/mha_mma.cu, default), 1 = the fp32 CUDA-core kernel. Process-global. */
 int hsv_set_mha_variant(int v);
 int hsv_conv1d_c1_strided(const float *x, const float *w, const float *bias, const float *mask, float *out, int B,
                           int Cout, int64_t Lin, int64_t Lout, int k, int stride, int pad, void *stream);
+/* the same for a ragged batch: valid_len [B] int32, device (NULL = as above), in OUTPUT frames, clamped to [0, Lout].
+ * Item b reads x[b, 0, :stride * valid_len[b]] only (samples past it are the conv's zero padding, as in its own run with
+ * Lin = stride * valid_len[b]) and writes 0 at t >= valid_len[b]. */
+int hsv_conv1d_c1_strided_ragged(const float *x, const float *w, const float *bias, const float *mask,
+                                 const int32_t *valid_len, float *out, int B, int Cout, int64_t Lin, int64_t Lout, int k,
+                                 int stride, int pad, void *stream);
 int hsv_masked_mean(const float *x, const float *mask, float *out, int B, int C, int64_t L, void *stream);
+/* the same for a ragged batch: valid_len [B] int32, device (NULL = as above), clamped to [0, L].  Item b sums
+ * x[b, c, :valid_len[b]] in the order of its own call with L = valid_len[b] (and an all-ones mask) and divides by
+ * valid_len[b]; mask is not read. */
+int hsv_masked_mean_ragged(const float *x, const float *mask, const int32_t *valid_len, float *out, int B, int C,
+                           int64_t L, void *stream);
 
 /* ---- f0-driven harmonic sine source (BASELINE.json north_star item 3; NSF / HiFTNet-style SineGen -- the
  * reference repository has no counterpart on this path, SURVEY.md §0.3).  The phase accumulator is 64-bit fixed point

@@ -29,6 +29,8 @@ SIGNATURES = {
     "hsv_pack_conv_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "hsv_conv1d_umma": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_float,
                                 c_int, c_int, c_int, c_int64, c_int, c_int, c_int, c_void_p]),
+    "hsv_conv1d_umma_astride": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                        c_int, c_int, c_int64, c_int, c_int, c_int, c_void_p]),
     "hsv_conv1d_umma_blk16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_int, c_int,
                                       c_int, c_int64, c_int, c_int, c_int, c_void_p]),
     "hsv_conv1d_umma_wn_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
@@ -67,12 +69,17 @@ SIGNATURES = {
                              c_float, c_int64, c_void_p]),
     "hsv_mha_blk16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64,
                               c_int64, c_int64, c_float, c_int, c_void_p]),
+    "hsv_mha_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
+                               c_int, c_int, c_int64, c_int64, c_int64, c_float, c_int, c_void_p]),
     "hsv_set_mha_variant": (c_int, [c_int]),
     "hsv_mha": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64,
                         c_int64, c_int64, c_float, c_int, c_void_p]),
     "hsv_conv1d_c1_strided": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int64,
                                       c_int, c_int, c_int, c_void_p]),
+    "hsv_conv1d_c1_strided_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                             c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
     "hsv_masked_mean": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
+    "hsv_masked_mean_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
     "hsv_sinegen_workspace": (c_int64, [c_int, c_int64, c_int]),
     "hsv_sinegen": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int, c_float, c_int, c_float,
                             c_void_p]),

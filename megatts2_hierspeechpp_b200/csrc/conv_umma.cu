@@ -66,6 +66,7 @@ struct Params {
   int msub;          // 128-row sub-tiles per CTA (1, 2 or 4): every weight K-step feeds msub MMAs
   int cw;            // channels per operand row (64 / 32 / 16)
   int nchunks;       // Cin / cw
+  int a_bchunks;     // operand chunks between batch items of A (nchunks, more when A is a channel range of a wider buffer)
   int R;             // rows per chunk of the shared A tile = 128*msub + hlo8 + h_hi
   int hlo8;          // halo rows before the tile, rounded up to a multiple of 8 (swizzle phase alignment)
   uint32_t a_pitch;  // bytes between chunks of the shared A tile (multiple of 1024)
@@ -489,7 +490,7 @@ __global__ void __launch_bounds__(32 * NW, MINB) conv_umma_kernel(const __grid_c
     if constexpr (RR == 0) {
       const int64_t row0 = (int64_t)HSV_BLK_PAD + (int64_t)tile * TILE_M * MSUB - p.hlo8;  // multiple of 8
       for (int c = 0; c < p.nchunks; ++c) {
-        const uint8_t *src = p.a + (((int64_t)b * p.nchunks + c) * p.Lp + row0) * rowbytes;
+        const uint8_t *src = p.a + ((int64_t)(b * p.a_bchunks + c) * p.Lp + row0) * rowbytes;   // B * a_bchunks < 2^31
         mbar_expect_tx(bar_a + 8 * c, a_chunk_bytes);
         bulk_g2s(a_s + c * p.a_pitch, src, a_chunk_bytes, bar_a + 8 * c);
       }
@@ -882,7 +883,7 @@ __global__ void __launch_bounds__(64 + 128 * EPW, 1) conv_umma_persist_kernel(co
         const int64_t row0 = (int64_t)HSV_BLK_PAD + (int64_t)tile * TILE_M - p.hlo8;
         mbar_expect_tx(bar0 + 8 * (PB_A_F + buf), a_chunk_bytes * (uint32_t)p.nchunks);
         for (int c = 0; c < p.nchunks; ++c) {
-          const uint8_t *src = p.a + (((int64_t)b * p.nchunks + c) * p.Lp + row0) * rowbytes;
+          const uint8_t *src = p.a + (((int64_t)b * p.a_bchunks + c) * p.Lp + row0) * rowbytes;
           bulk_g2s(a_s + buf * a_tile_bytes + c * p.a_pitch, src, a_chunk_bytes, bar0 + 8 * (PB_A_F + buf));
         }
       };
@@ -1282,7 +1283,7 @@ struct BlkOut {    // operand-writing epilogue (see Params)
 int launch(const TapTable &tt, const void *a_blk16, const void *w_packed, const float *bias,
            const float *residual, float *out, float *acc, int acc_mode, int B, int Cin, int Cout, int64_t L,
            int64_t Lout, int n_tile, cudaStream_t st, const char *what, const FusedAct *fa = nullptr,
-           const BlkOut *bo = nullptr) {
+           const BlkOut *bo = nullptr, int64_t a_bchunks = 0) {
   Params p;
   p.out_blk = bo ? bo->out : nullptr;
   p.blk_mode = bo ? bo->mode : 0;
@@ -1305,6 +1306,8 @@ int launch(const TapTable &tt, const void *a_blk16, const void *w_packed, const 
   p.n_tile = n_tile; p.nco_tiles = Cout / n_tile;
   p.cw = hsv::blk_cw(Cin);
   p.nchunks = Cin / p.cw;
+  p.a_bchunks = (int)(a_bchunks > 0 ? a_bchunks : p.nchunks);
+  HSV_REQUIRE((int64_t)B * p.a_bchunks < (int64_t)1 << 31, "%s: batch x operand chunks too large", what);
   HSV_REQUIRE(p.nchunks <= MAX_CHUNKS, "%s: Cin=%d needs %d operand chunks (max %d)", what, Cin, p.nchunks, MAX_CHUNKS);
   const int rowbytes = p.cw * 2;
   p.hlo8 = (tt.h_lo + 7) & ~7;
@@ -1503,11 +1506,14 @@ extern "C" int hsv_pack_convT_weight(const float *w, void *packed, int Cin, int 
               "pack_convT_weight");
 }
 
-extern "C" int hsv_conv1d_umma(const void *a_blk16, const void *w_packed, const float *bias,
-                               const float *residual, float *out, float *acc, int acc_mode, float /*acc_div: reserved*/,
-                               int B, int Cin, int Cout, int64_t L, int k, int d, int n_tile, void *stream) {
+extern "C" int hsv_conv1d_umma_astride(const void *a_blk16, int64_t a_bchunks, const void *w_packed, const float *bias,
+                                       const float *residual, float *out, float *acc, int acc_mode, int B, int Cin,
+                                       int Cout, int64_t L, int k, int d, int n_tile, void *stream) {
   if (B == 0 || L == 0) return HSV_OK;  // empty batch / sequence
   if (int rc = check_common("conv1d_umma", a_blk16, w_packed, Cin, Cout, n_tile)) return rc;
+  HSV_REQUIRE(a_bchunks == 0 || (a_bchunks >= Cin / hsv::blk_cw(Cin) && a_bchunks <= 65535),
+              "conv1d_umma: A batch stride of %lld chunks outside [%d (Cin=%d), 65535]", (long long)a_bchunks,
+              Cin / hsv::blk_cw(Cin), Cin);
   HSV_REQUIRE(k >= 1 && k <= MAX_TAPS && (k & 1) && d >= 1, "conv1d_umma: k must be odd and <= %d (k=%d d=%d)",
               MAX_TAPS, k, d);
   HSV_REQUIRE(((k - 1) / 2) * d <= HSV_BLK_PAD, "conv1d_umma: halo %d exceeds blk16 padding %d",
@@ -1515,7 +1521,14 @@ extern "C" int hsv_conv1d_umma(const void *a_blk16, const void *w_packed, const 
   HSV_REQUIRE(acc_mode >= 0 && acc_mode <= 2 && (acc_mode == 0 || acc), "conv1d_umma: bad acc_mode/acc");
   HSV_REQUIRE(out || acc_mode, "conv1d_umma: no output");
   return launch(conv_taps(k, d), a_blk16, w_packed, bias, residual, out, acc, acc_mode, B, Cin, Cout, L, L, n_tile,
-                hsv::as_stream(stream), "conv1d_umma");
+                hsv::as_stream(stream), "conv1d_umma", nullptr, nullptr, a_bchunks);
+}
+
+extern "C" int hsv_conv1d_umma(const void *a_blk16, const void *w_packed, const float *bias,
+                               const float *residual, float *out, float *acc, int acc_mode, float /*acc_div: reserved*/,
+                               int B, int Cin, int Cout, int64_t L, int k, int d, int n_tile, void *stream) {
+  return hsv_conv1d_umma_astride(a_blk16, 0, w_packed, bias, residual, out, acc, acc_mode, B, Cin, Cout, L, k, d, n_tile,
+                                 stream);
 }
 
 extern "C" int hsv_conv1d_umma_blk16(const void *a_blk16, const void *w_packed, const float *bias, void *out_blk16, int mode,

@@ -118,7 +118,9 @@ __global__ void wn_res_pack_kernel(float *__restrict__ x, const float *__restric
 // groups; thread (tx, g) owns the C/8 consecutive channels of group g at step tx (C % 64 == 0: whole 16-byte units).
 // With y != nullptr the preceding gated residual update is fused in (modules.py:408-409): x = x + gate[b,c] * y * mask is
 // written back to x (fp32, in place) and the normalisation runs on the new x.
-template <int CPT>   // channels per thread = C / 8
+// ZROWS: operand rows where mask == 0 are written as zero (HSV_LN_ZERO_MASKED; a separate instantiation, so the
+// other launches run none of it)
+template <int CPT, bool ZROWS>   // channels per thread = C / 8
 __global__ void __launch_bounds__(256) ln_mod_kernel(float *x, const float *__restrict__ y, const float *__restrict__ gate,
                                                      int64_t gate_stride, const float *__restrict__ shift,
                                                      const float *__restrict__ scale, const float *__restrict__ mask,
@@ -169,7 +171,14 @@ __global__ void __launch_bounds__(256) ln_mod_kernel(float *x, const float *__re
   for (int q = 0; q < 8; ++q) var += red[q][tx];
   const float rstd = rsqrtf(var / (float)C + eps);
   if (!ok) return;
-  const float pm = premask ? mk : 1.f;
+  if (ZROWS && mk == 0.f) {               // rows past an item of a ragged batch: the zero padding of its own run
+#pragma unroll
+    for (int u = 0; u < CPT / 8; ++u)
+      *reinterpret_cast<uint4 *>(reinterpret_cast<uint8_t *>(out) +
+                                 hsv::blk_unit_offset(cw, Lp, C, b, g * CPT + u * 8, HSV_BLK_PAD + t)) = make_uint4(0, 0, 0, 0);
+    return;
+  }
+  const float pm = (premask & 1) ? mk : 1.f;
 #pragma unroll
   for (int u = 0; u < CPT / 8; ++u) {
     __half2 h[4];
@@ -443,19 +452,31 @@ int mha_launch(const float *q, const float *k, const float *v, float *out, const
 
 // Conv1d with ONE input channel and a stride (PosteriorSFEncoder.pre_filter: Conv1d(1, 192, 9, stride 4, padding 4),
 // hierspeechpp_speechsynthesizer.py:187,196): out[b, co, t] = bias[co] + sum_j w[co, j] * x[b, t*stride + j - pad]
+// VLEN: item b is its first vlen[b] output frames and stride * vlen[b] input samples (the rest of its input is the
+// conv's zero padding and is never read, its output there is 0)
+template <bool VLEN>
 __global__ void conv1d_c1_strided_kernel(const float *__restrict__ x, const float *__restrict__ w,
                                          const float *__restrict__ bias, const float *__restrict__ mask,
-                                         float *__restrict__ out, int B, int Cout, int64_t Lin, int64_t Lout, int k,
-                                         int stride, int pad) {
+                                         const int *__restrict__ vlen, float *__restrict__ out, int B, int Cout,
+                                         int64_t Lin, int64_t Lout, int k, int stride, int pad) {
   const int64_t n = (int64_t)B * Cout * Lout;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t bc = i / Lout, t = i - bc * Lout;
     const int64_t bb = bc / Cout;
     const int co = (int)(bc - bb * Cout);
+    int64_t lin = Lin;
+    if (VLEN) {
+      const int64_t nv = min((int64_t)max(__ldg(vlen + bb), 0), Lout);
+      if (t >= nv) {
+        out[i] = 0.f;
+        continue;
+      }
+      lin = min(nv * stride, Lin);
+    }
     float acc = 0.f;
     for (int j = 0; j < k; ++j) {
       const int64_t s = t * stride + j - pad;
-      if (s >= 0 && s < Lin) acc = fmaf(__ldg(w + co * k + j), __ldg(x + bb * Lin + s), acc);
+      if (s >= 0 && s < lin) acc = fmaf(__ldg(w + co * k + j), __ldg(x + bb * Lin + s), acc);
     }
     acc += bias ? __ldg(bias + co) : 0.f;
     out[i] = acc * (mask ? __ldg(mask + bb * Lout + t) : 1.f);
@@ -463,10 +484,14 @@ __global__ void conv1d_c1_strided_kernel(const float *__restrict__ x, const floa
 }
 
 // out[b, c] = sum_t x[b, c, t] / denom[b]   (StyleEncoder.temporal_avg_pool: the sum runs over ALL frames)
-__global__ void masked_mean_kernel(const float *__restrict__ x, float *__restrict__ out, int64_t L) {
+// VLEN: the sum of item b runs over t < vlen[b] only, in the order of its own launch with L = vlen[b]
+template <bool VLEN>
+__global__ void masked_mean_kernel(const float *__restrict__ x, const int *__restrict__ vlen, float *__restrict__ out,
+                                   int C, int64_t L) {
   const int64_t row = blockIdx.x;            // b * C + c
+  const int64_t n = VLEN ? min((int64_t)max(__ldg(vlen + row / C), 0), L) : L;
   float s = 0.f;
-  for (int64_t t = threadIdx.x; t < L; t += blockDim.x) s += __ldg(x + row * L + t);
+  for (int64_t t = threadIdx.x; t < n; t += blockDim.x) s += __ldg(x + row * L + t);
   __shared__ float red[32];
   for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
@@ -477,12 +502,17 @@ __global__ void masked_mean_kernel(const float *__restrict__ x, float *__restric
     out[row] = tot;
   }
 }
-__global__ void mean_div_kernel(float *__restrict__ out, const float *__restrict__ mask, int C, int64_t L) {
+__global__ void mean_div_kernel(float *__restrict__ out, const float *__restrict__ mask, const int *__restrict__ vlen,
+                                int C, int64_t L) {
   const int b = blockIdx.x;
   __shared__ float len_s;
   if (threadIdx.x == 0) {
     float l = 0.f;
-    for (int64_t t = 0; t < L; ++t) l += mask ? mask[(int64_t)b * L + t] : 1.f;
+    if (vlen) {                              // an item's own run: a mask of n ones sums to n exactly (n < 2^24)
+      l = (float)min((int64_t)max(vlen[b], 0), L);
+    } else {
+      for (int64_t t = 0; t < L; ++t) l += mask ? mask[(int64_t)b * L + t] : 1.f;
+    }
     len_s = l;
   }
   __syncthreads();
@@ -521,17 +551,28 @@ static int ln_mod_launch(float *x, const float *y, const float *gate, int64_t ga
   HSV_REQUIRE(x && shift && scale && out, "%s: null pointer", what);
   HSV_REQUIRE(C == 192 || C == 256 || C == 128 || C == 64, "%s: C must be 64, 128, 192 or 256 (C=%d)", what, C);
   HSV_REQUIRE(B <= 65535, "%s: batch too large", what);
+  HSV_REQUIRE(!(premask & HSV_LN_ZERO_MASKED) || mask, "%s: zeroing masked rows needs a mask", what);
   dim3 grid((unsigned)((L + 31) / 32), (unsigned)B);
   cudaStream_t st = hsv::as_stream(stream);
   uint4 *o = reinterpret_cast<uint4 *>(out);
   const int64_t Lp = hsv::blk16_rows(L);
   const int cw = hsv::blk_cw(C);
-#define HSV_LN(CPT) \
-  ln_mod_kernel<CPT><<<grid, 256, 0, st>>>(x, y, gate, gate_stride, shift, scale, mask, o, C, L, Lp, cw, eps, inmask, premask, mod_stride)
-  if (C == 192) HSV_LN(24);
-  else if (C == 256) HSV_LN(32);
-  else if (C == 128) HSV_LN(16);
-  else HSV_LN(8);
+#define HSV_LN(CPT)                                                                                                       \
+  if (premask & HSV_LN_ZERO_MASKED)                                                                                         \
+    ln_mod_kernel<CPT, true><<<grid, 256, 0, st>>>(x, y, gate, gate_stride, shift, scale, mask, o, C, L, Lp, cw, eps, inmask, \
+                                                   premask, mod_stride);                                                    \
+  else                                                                                                                      \
+    ln_mod_kernel<CPT, false><<<grid, 256, 0, st>>>(x, y, gate, gate_stride, shift, scale, mask, o, C, L, Lp, cw, eps, inmask, \
+                                                    premask, mod_stride)
+  if (C == 192) {
+    HSV_LN(24);
+  } else if (C == 256) {
+    HSV_LN(32);
+  } else if (C == 128) {
+    HSV_LN(16);
+  } else {
+    HSV_LN(8);
+  }
 #undef HSV_LN
   return hsv::check_launch(what);
 }
@@ -564,9 +605,9 @@ extern "C" int hsv_frame_op(int op, const float *a, const float *b, const float 
 }
 
 namespace hsv {
-int mha_mma_launch(const float *q, const float *k, const float *v, void *out, int blk, const int *lens, int B, int heads,
-                   int D, int Tq, int Tk, int64_t qbs, int64_t kbs, int64_t vbs, float scale, int prescale,
-                   cudaStream_t st);
+int mha_mma_launch(const float *q, const float *k, const float *v, void *out, int blk, const int *lens, const int *vlen,
+                   int B, int heads, int D, int Tq, int Tk, int64_t qbs, int64_t kbs, int64_t vbs, float scale,
+                   int prescale, cudaStream_t st);
 }
 static int g_mha_variant = 0;   // 0: tensor cores (mha_mma.cu), 1: the fp32 CUDA-core kernel of this file (test hook)
 extern "C" int hsv_set_mha_variant(int v) {
@@ -574,25 +615,31 @@ extern "C" int hsv_set_mha_variant(int v) {
   return HSV_OK;
 }
 
-extern "C" int hsv_mha(const float *q, const float *k, const float *v, float *out, const int *lens, int B, int heads,
-                       int D, int Tq, int Tk, int64_t q_bstride, int64_t k_bstride, int64_t v_bstride, float scale,
-                       int prescale_q, void *stream) {
+extern "C" int hsv_mha_ragged(const float *q, const float *k, const float *v, void *out, int out_mode, const int *lens,
+                              const int32_t *valid_len, int B, int heads, int D, int Tq, int Tk, int64_t q_bstride,
+                              int64_t k_bstride, int64_t v_bstride, float scale, int prescale_q, void *stream) {
+  const char *what = out_mode ? "mha_blk16" : "mha";
   if (B == 0 || Tq == 0) return HSV_OK;
-  HSV_REQUIRE(q && k && v && out, "mha: null pointer");
-  HSV_REQUIRE(D == 96 || D == 128 || D == 64, "mha: head dim must be 64, 96 or 128 (D=%d)", D);
-  HSV_REQUIRE(Tk > 0 && heads > 0 && heads <= 65535 && B <= 65535, "mha: bad shape");
+  HSV_REQUIRE(q && k && v && out, "%s: null pointer", what);
+  HSV_REQUIRE(D == 96 || D == 128 || D == 64, "%s: head dim must be 64, 96 or 128 (D=%d)", what, D);
+  HSV_REQUIRE(Tk > 0 && heads > 0 && heads <= (out_mode ? 32767 : 65535) && B <= 65535 && (heads * D) % 16 == 0,
+              "%s: bad shape", what);
+  HSV_REQUIRE(out_mode == 0 || out_mode == 1, "%s: out_mode %d", what, out_mode);
+  HSV_REQUIRE(!valid_len || (!lens && Tq == Tk), "%s: valid_len is self-attention per item (Tq == Tk, no lens)", what);
+  HSV_REQUIRE(!valid_len || g_mha_variant == 0, "%s: the fp32 CUDA-core variant takes no valid_len", what);
   cudaStream_t st = hsv::as_stream(stream);
-  if (g_mha_variant == 0) {
-    const int rc = hsv::mha_mma_launch(q, k, v, out, 0, lens, B, heads, D, Tq, Tk, q_bstride, k_bstride, v_bstride, scale,
-                                       prescale_q, st);
+  if (g_mha_variant == 0 || out_mode) {
+    const int rc = hsv::mha_mma_launch(q, k, v, out, out_mode, lens, valid_len, B, heads, D, Tq, Tk, q_bstride, k_bstride,
+                                       v_bstride, scale, prescale_q, st);
     if (rc != 1) return rc;
   }
+  float *o = reinterpret_cast<float *>(out);
   // few (batch, head, query tile) items: 8-row tiles spread the work over more SMs
   const bool small = (int64_t)B * heads * ((Tq + 15) / 16) < 148;
 #define HSV_MHA(DD)                                                                                               \
-  return small ? mha_launch<DD, 2>(q, k, v, out, lens, B, heads, Tq, Tk, q_bstride, k_bstride, v_bstride, scale, \
+  return small ? mha_launch<DD, 2>(q, k, v, o, lens, B, heads, Tq, Tk, q_bstride, k_bstride, v_bstride, scale,   \
                                    prescale_q, st)                                                                 \
-               : mha_launch<DD, 4>(q, k, v, out, lens, B, heads, Tq, Tk, q_bstride, k_bstride, v_bstride, scale, \
+               : mha_launch<DD, 4>(q, k, v, o, lens, B, heads, Tq, Tk, q_bstride, k_bstride, v_bstride, scale,   \
                                    prescale_q, st)
   if (D == 96) { HSV_MHA(96); }
   if (D == 128) { HSV_MHA(128); }
@@ -600,33 +647,53 @@ extern "C" int hsv_mha(const float *q, const float *k, const float *v, float *ou
 #undef HSV_MHA
 }
 
+extern "C" int hsv_mha(const float *q, const float *k, const float *v, float *out, const int *lens, int B, int heads,
+                       int D, int Tq, int Tk, int64_t q_bstride, int64_t k_bstride, int64_t v_bstride, float scale,
+                       int prescale_q, void *stream) {
+  return hsv_mha_ragged(q, k, v, out, 0, lens, nullptr, B, heads, D, Tq, Tk, q_bstride, k_bstride, v_bstride, scale,
+                        prescale_q, stream);
+}
+
 extern "C" int hsv_mha_blk16(const float *q, const float *k, const float *v, void *out_blk16, const int *lens, int B,
                              int heads, int D, int Tq, int Tk, int64_t q_bstride, int64_t k_bstride, int64_t v_bstride,
                              float scale, int prescale_q, void *stream) {
-  if (B == 0 || Tq == 0) return HSV_OK;
-  HSV_REQUIRE(q && k && v && out_blk16, "mha_blk16: null pointer");
-  HSV_REQUIRE(Tk > 0 && heads > 0 && heads <= 32767 && B <= 65535 && (heads * D) % 16 == 0, "mha_blk16: bad shape");
-  const int rc = hsv::mha_mma_launch(q, k, v, out_blk16, 1, lens, B, heads, D, Tq, Tk, q_bstride, k_bstride, v_bstride,
-                                     scale, prescale_q, hsv::as_stream(stream));
-  HSV_REQUIRE(rc != 1, "mha_blk16: head dim must be 64, 96 or 128 (D=%d)", D);
-  return rc;
+  return hsv_mha_ragged(q, k, v, out_blk16, 1, lens, nullptr, B, heads, D, Tq, Tk, q_bstride, k_bstride, v_bstride, scale,
+                        prescale_q, stream);
+}
+
+extern "C" int hsv_conv1d_c1_strided_ragged(const float *x, const float *w, const float *bias, const float *mask,
+                                            const int32_t *valid_len, float *out, int B, int Cout, int64_t Lin,
+                                            int64_t Lout, int k, int stride, int pad, void *stream) {
+  if (B == 0 || Lout == 0) return HSV_OK;
+  HSV_REQUIRE(x && w && out && k >= 1 && stride >= 1 && pad >= 0, "conv1d_c1_strided: bad arguments");
+  const int grid = grid_for((int64_t)B * Cout * Lout, 256);
+  cudaStream_t st = hsv::as_stream(stream);
+  if (valid_len)
+    conv1d_c1_strided_kernel<true><<<grid, 256, 0, st>>>(x, w, bias, mask, valid_len, out, B, Cout, Lin, Lout, k, stride,
+                                                         pad);
+  else
+    conv1d_c1_strided_kernel<false><<<grid, 256, 0, st>>>(x, w, bias, mask, nullptr, out, B, Cout, Lin, Lout, k, stride,
+                                                          pad);
+  return hsv::check_launch("conv1d_c1_strided");
 }
 
 extern "C" int hsv_conv1d_c1_strided(const float *x, const float *w, const float *bias, const float *mask, float *out,
                                      int B, int Cout, int64_t Lin, int64_t Lout, int k, int stride, int pad,
                                      void *stream) {
-  if (B == 0 || Lout == 0) return HSV_OK;
-  HSV_REQUIRE(x && w && out && k >= 1 && stride >= 1 && pad >= 0, "conv1d_c1_strided: bad arguments");
-  conv1d_c1_strided_kernel<<<grid_for((int64_t)B * Cout * Lout, 256), 256, 0, hsv::as_stream(stream)>>>(
-      x, w, bias, mask, out, B, Cout, Lin, Lout, k, stride, pad);
-  return hsv::check_launch("conv1d_c1_strided");
+  return hsv_conv1d_c1_strided_ragged(x, w, bias, mask, nullptr, out, B, Cout, Lin, Lout, k, stride, pad, stream);
 }
 
-extern "C" int hsv_masked_mean(const float *x, const float *mask, float *out, int B, int C, int64_t L, void *stream) {
+extern "C" int hsv_masked_mean_ragged(const float *x, const float *mask, const int32_t *valid_len, float *out, int B,
+                                      int C, int64_t L, void *stream) {
   if (B == 0 || C == 0) return HSV_OK;
   HSV_REQUIRE(x && out && L > 0, "masked_mean: bad arguments");
   cudaStream_t st = hsv::as_stream(stream);
-  masked_mean_kernel<<<(unsigned)(B * C), 128, 0, st>>>(x, out, L);
-  mean_div_kernel<<<B, 128, 0, st>>>(out, mask, C, L);
+  if (valid_len) masked_mean_kernel<true><<<(unsigned)(B * C), 128, 0, st>>>(x, valid_len, out, C, L);
+  else masked_mean_kernel<false><<<(unsigned)(B * C), 128, 0, st>>>(x, nullptr, out, C, L);
+  mean_div_kernel<<<B, 128, 0, st>>>(out, mask, valid_len, C, L);
   return hsv::check_launch("masked_mean");
+}
+
+extern "C" int hsv_masked_mean(const float *x, const float *mask, float *out, int B, int C, int64_t L, void *stream) {
+  return hsv_masked_mean_ragged(x, mask, nullptr, out, B, C, L, stream);
 }

@@ -66,11 +66,14 @@ __device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], 
 
 // BLK: the result is written as the fp16 blk16 operand of the following proj conv (out = blk16 buffer of heads*D channels)
 // instead of fp32 [B, heads*D, Tq]
-template <int D, bool BLK>
+// VLEN: per-item lengths (self-attention of a ragged batch): item b has n = vlen[b] queries and keys, stored with the row
+// pitches Tq / Tk.  It runs exactly as its own launch with Tq = Tk = n (same key tiles, same zero fill and -inf past n),
+// and its rows [n, Tq) are written as zero; a query tile wholly past n does no key work.
+template <int D, bool BLK, bool VLEN>
 __global__ void __cluster_dims__(1, NSPLIT, 1) __launch_bounds__(32 * NWARP)
 mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const float *__restrict__ v, void *__restrict__ out,
-               const int *__restrict__ lens, int Tq, int Tk, int64_t qbs, int64_t kbs, int64_t vbs, int heads, float scale,
-               int prescale, int fast) {
+               const int *__restrict__ lens, const int *__restrict__ vlen, int Tq, int Tk, int64_t qbs, int64_t kbs,
+               int64_t vbs, int heads, float scale, int prescale, int fast) {
   constexpr int KS = D / 16;                      // k-steps of Q K^T
   constexpr int NT = D / 8;                       // n-tiles of P V
   constexpr int STAGE = D * (KP + VP);            // words per (K, V) stage of one warp
@@ -86,8 +89,64 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
   const float *kb = k + (int64_t)b * kbs + (int64_t)h * D * Tk;
   const float *vb = v + (int64_t)b * vbs + (int64_t)h * D * Tk;
   const int len = lens ? lens[b] : 0x7fffffff;
-  const int ntiles = (Tk + KT - 1) / KT;
+  // logical query / key counts of this item (the row pitches stay Tq / Tk)
+  const int nv = VLEN ? min(max(vlen[b], 0), min(Tq, Tk)) : 0;
+  const int tq = VLEN ? nv : Tq, tk = VLEN ? nv : Tk;
+  const int ntiles = (tk + KT - 1) / KT;
   float *my = sm + w * 2 * STAGE;                 // this warp's two stages
+
+  // merged values per thread.  fp32 output: value i = (d, r) with rows fastest (64-byte segments of a channel row);
+  // blk16 output: a thread owns whole 16-byte units (8 consecutive channels of one row): unit u = tid + 128 * (i / 8)
+  constexpr int NUNIT = QT * D / 8;
+  constexpr int PER = BLK ? 8 * ((NUNIT + 32 * NWARP - 1) / (32 * NWARP)) : QT * D / (32 * NWARP);
+  auto where = [&](int i, int &d, int &r) -> bool {
+    if (BLK) {
+      const int u = tid + 32 * NWARP * (i >> 3);
+      d = 8 * (u / QT) + (i & 7);
+      r = u % QT;
+      return u < NUNIT;
+    }
+    const int idx = tid + 32 * NWARP * i;
+    d = idx / QT;
+    r = idx - d * QT;
+    return true;
+  };
+  // CTA 0's store of the tile's rows [q0, min(q0 + QT, Tq))
+  auto store = [&](const float (&accv)[PER]) {
+    if (BLK) {
+      const int C = heads * D;
+      const int cw = hsv::blk_cw(C);
+      const int64_t Lp = hsv::blk16_rows(Tq);
+#pragma unroll
+      for (int j = 0; j < PER / 8; ++j) {
+        int d, r;
+        if (!where(8 * j, d, r) || q0 + r >= Tq) continue;
+        __half2 hh[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) hh[e] = __floats2half2_rn(accv[8 * j + 2 * e], accv[8 * j + 2 * e + 1]);
+        *reinterpret_cast<uint4 *>(reinterpret_cast<uint8_t *>(out) +
+                                   hsv::blk_unit_offset(cw, Lp, C, b, h * D + d, HSV_BLK_PAD + q0 + r)) =
+            *reinterpret_cast<uint4 *>(hh);
+      }
+    } else {
+      float *ob = reinterpret_cast<float *>(out) + ((int64_t)b * heads + h) * D * Tq;
+#pragma unroll
+      for (int i = 0; i < PER; ++i) {
+        int d, r;
+        where(i, d, r);
+        if (q0 + r < Tq) ob[(int64_t)d * Tq + q0 + r] = accv[i];
+      }
+    }
+  };
+  if (VLEN && q0 >= tq) {                         // every row of the tile is past the item: zero rows, no key work
+    if (split == 0) {
+      float zero[PER];
+#pragma unroll
+      for (int i = 0; i < PER; ++i) zero[i] = 0.f;
+      store(zero);
+    }
+    return;                                       // both CTAs of the cluster leave here (same q0, same b)
+  }
 
   // per-lane constants of the tile copy: chunk ch = lane + 32 i  ->  d = (lane >> 2) + 8 i, 4 keys at (lane & 3) * 4
   const int ld_d0 = lane >> 2, ld_x4 = (lane & 3) * 4;
@@ -97,7 +156,7 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
   const int64_t ld_step = (int64_t)8 * Tk;
   auto load_tile = [&](int t, int stage) {
     const int k0 = t * KT;
-    if (fast && k0 + KT <= Tk) {
+    if (fast && k0 + KT <= tk) {
       const float *gk = ld_k + k0, *gv = ld_v + k0;
       const uint32_t sk = ld_sk + stage * (STAGE * 4), sv = ld_sv + stage * (STAGE * 4);
 #pragma unroll
@@ -113,7 +172,7 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
       const uint32_t sk0 = (uint32_t)__cvta_generic_to_shared(my + stage * STAGE);
       const uint32_t sv0 = sk0 + D * KP * 4;
       const int j = lane & (KT - 1), dq = lane / KT;             // 16 keys x 2 rows per warp step
-      const int ok = (k0 + j < Tk) ? 4 : 0;
+      const int ok = (k0 + j < tk) ? 4 : 0;
       const int64_t col = ok ? k0 + j : 0;                       // keep the (unused) source address in bounds
 #pragma unroll 8
       for (int d = dq; d < D; d += 32 / KT) {
@@ -129,7 +188,7 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
   // ---- Q tile [D][16 rows] -> shared (cp.async, same [d][t] form as a K tile), then the first K / V tile ----
   float *Qs = sm + NWARP * 2 * STAGE + QT * (D + 1) + 2 * QT;     // behind the peer's landing zone; pitch KP
   {
-    const bool qfast = (Tq % 4 == 0) && q0 + QT <= Tq && ((reinterpret_cast<uintptr_t>(q) & 15) == 0) && (qbs % 4 == 0);
+    const bool qfast = (Tq % 4 == 0) && q0 + QT <= tq && ((reinterpret_cast<uintptr_t>(q) & 15) == 0) && (qbs % 4 == 0);
     if (qfast) {
       for (int ch = tid; ch < D * 4; ch += 32 * NWARP) {
         const int d = ch >> 2, x4 = (ch & 3) * 4;
@@ -138,7 +197,7 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
     } else {                                                     // ragged / unaligned: 4-byte copies, zero fill past Tq
       const uint32_t sq0 = (uint32_t)__cvta_generic_to_shared(Qs);
       const int r = tid & (QT - 1);
-      const int ok = (q0 + r < Tq) ? 4 : 0;
+      const int ok = (q0 + r < tq) ? 4 : 0;
       const int64_t col = ok ? q0 + r : 0;
 #pragma unroll 4
       for (int d = tid / QT; d < D; d += 32 * NWARP / QT)
@@ -210,7 +269,7 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
         const int qi = q0 + g + 8 * (e >> 1);
         float a = prescale ? s[nt][e] : s[nt][e] * scale;
         if (lens && (qi >= len || j >= len)) a = -1e4f;      // masked_fill(mask == 0, -1e4)
-        if (j >= Tk) a = -INFINITY;                          // padding of the last key tile
+        if (j >= tk) a = -INFINITY;                          // padding of the last key tile
         s[nt][e] = a;
         mx[e >> 1] = fmaxf(mx[e >> 1], a);
       }
@@ -307,22 +366,6 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
     Cl[r] = l;
   }
   __syncthreads();
-  // merged values per thread.  fp32 output: value i = (d, r) with rows fastest (64-byte segments of a channel row);
-  // blk16 output: a thread owns whole 16-byte units (8 consecutive channels of one row): unit u = tid + 128 * (i / 8)
-  constexpr int NUNIT = QT * D / 8;
-  constexpr int PER = BLK ? 8 * ((NUNIT + 32 * NWARP - 1) / (32 * NWARP)) : QT * D / (32 * NWARP);
-  auto where = [&](int i, int &d, int &r) -> bool {
-    if (BLK) {
-      const int u = tid + 32 * NWARP * (i >> 3);
-      d = 8 * (u / QT) + (i & 7);
-      r = u % QT;
-      return u < NUNIT;
-    }
-    const int idx = tid + 32 * NWARP * i;
-    d = idx / QT;
-    r = idx - d * QT;
-    return true;
-  };
   float accv[PER];
 #pragma unroll
   for (int i = 0; i < PER; ++i) {
@@ -357,42 +400,20 @@ mha_mma_kernel(const float *__restrict__ q, const float *__restrict__ k, const f
     const float f0 = __expf(m0 - m), f1 = m1 == -INFINITY ? 0.f : __expf(m1 - m);
     const float l = fmaf(Cl[r], f0, Rl[r] * f1);
     accv[i] = fmaf(accv[i], f0, Ro[r * (D + 1) + d] * f1) / l;
+    if (VLEN && q0 + r >= tq) accv[i] = 0.f;       // rows past the item
   }
-  if (BLK) {
-    const int C = heads * D;
-    const int cw = hsv::blk_cw(C);
-    const int64_t Lp = hsv::blk16_rows(Tq);
-#pragma unroll
-    for (int j = 0; j < PER / 8; ++j) {
-      int d, r;
-      if (!where(8 * j, d, r) || q0 + r >= Tq) continue;
-      __half2 hh[4];
-#pragma unroll
-      for (int e = 0; e < 4; ++e) hh[e] = __floats2half2_rn(accv[8 * j + 2 * e], accv[8 * j + 2 * e + 1]);
-      *reinterpret_cast<uint4 *>(reinterpret_cast<uint8_t *>(out) +
-                                 hsv::blk_unit_offset(cw, Lp, C, b, h * D + d, HSV_BLK_PAD + q0 + r)) =
-          *reinterpret_cast<uint4 *>(hh);
-    }
-  } else {
-    float *ob = reinterpret_cast<float *>(out) + ((int64_t)b * heads + h) * D * Tq;
-#pragma unroll
-    for (int i = 0; i < PER; ++i) {
-      int d, r;
-      where(i, d, r);
-      if (q0 + r < Tq) ob[(int64_t)d * Tq + q0 + r] = accv[i];
-    }
-  }
+  store(accv);
 }
 
-template <int D, bool BLK>
-int launch(const float *q, const float *k, const float *v, void *out, const int *lens, int B, int heads, int Tq, int Tk,
-           int64_t qbs, int64_t kbs, int64_t vbs, float scale, int prescale, cudaStream_t st) {
+template <int D, bool BLK, bool VLEN>
+int launch(const float *q, const float *k, const float *v, void *out, const int *lens, const int *vlen, int B, int heads,
+           int Tq, int Tk, int64_t qbs, int64_t kbs, int64_t vbs, float scale, int prescale, cudaStream_t st) {
   static_assert((QT * D) % (32 * NWARP) == 0 && D % 8 == 0, "merge mapping");
   const size_t stages = sizeof(float) * NWARP * 2 * D * (KP + VP);           // >= the CTA-level merge area that reuses it
   const size_t smem = stages + sizeof(float) * (QT * (D + 1) + 2 * QT + D * KP);   // + the peer's landing zone + Q tile
   static bool done = false;
   if (!done) {
-    cudaError_t e = cudaFuncSetAttribute(mha_mma_kernel<D, BLK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(mha_mma_kernel<D, BLK, VLEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) {
       cudaGetLastError();
       hsv::set_error("mha_mma: cudaFuncSetAttribute(%zu): %s", smem, cudaGetErrorString(e));
@@ -403,8 +424,8 @@ int launch(const float *q, const float *k, const float *v, void *out, const int 
   auto al = [](const void *p_) { return (reinterpret_cast<uintptr_t>(p_) & 15) == 0; };
   const int fast = (Tk % 4 == 0) && al(k) && al(v) && (kbs % 4 == 0) && (vbs % 4 == 0);
   dim3 grid((unsigned)((Tq + QT - 1) / QT), (unsigned)(heads * NSPLIT), (unsigned)B);   // cluster dims (1, NSPLIT, 1)
-  mha_mma_kernel<D, BLK><<<grid, 32 * NWARP, smem, st>>>(q, k, v, out, lens, Tq, Tk, qbs, kbs, vbs, heads, scale,
-                                                       prescale, fast);
+  mha_mma_kernel<D, BLK, VLEN><<<grid, 32 * NWARP, smem, st>>>(q, k, v, out, lens, vlen, Tq, Tk, qbs, kbs, vbs, heads,
+                                                             scale, prescale, fast);
   return hsv::check_launch("mha_mma");
 }
 
@@ -413,12 +434,17 @@ int launch(const float *q, const float *k, const float *v, void *out, const int 
 namespace hsv {
 // returns 1 when the shape is not taken by this kernel (the caller falls back to the fp32 CUDA-core kernel).
 // blk != 0: ``out`` is the fp16 blk16 operand buffer of heads*D channels x Tq rows (zero padding rows untouched).
-int mha_mma_launch(const float *q, const float *k, const float *v, void *out, int blk, const int *lens, int B, int heads,
-                   int D, int Tq, int Tk, int64_t qbs, int64_t kbs, int64_t vbs, float scale, int prescale,
-                   cudaStream_t st) {
+// vlen != nullptr: per-item lengths (mha_mma_kernel's VLEN); a separate instantiation, so a launch without them runs
+// none of that code.
+int mha_mma_launch(const float *q, const float *k, const float *v, void *out, int blk, const int *lens, const int *vlen,
+                   int B, int heads, int D, int Tq, int Tk, int64_t qbs, int64_t kbs, int64_t vbs, float scale,
+                   int prescale, cudaStream_t st) {
 #define HSV_MHA_MMA(DD)                                                                                              \
-  return blk ? launch<DD, true>(q, k, v, out, lens, B, heads, Tq, Tk, qbs, kbs, vbs, scale, prescale, st)            \
-             : launch<DD, false>(q, k, v, out, lens, B, heads, Tq, Tk, qbs, kbs, vbs, scale, prescale, st)
+  if (vlen)                                                                                                          \
+    return blk ? launch<DD, true, true>(q, k, v, out, lens, vlen, B, heads, Tq, Tk, qbs, kbs, vbs, scale, prescale, st) \
+               : launch<DD, false, true>(q, k, v, out, lens, vlen, B, heads, Tq, Tk, qbs, kbs, vbs, scale, prescale, st); \
+  return blk ? launch<DD, true, false>(q, k, v, out, lens, nullptr, B, heads, Tq, Tk, qbs, kbs, vbs, scale, prescale, st) \
+             : launch<DD, false, false>(q, k, v, out, lens, nullptr, B, heads, Tq, Tk, qbs, kbs, vbs, scale, prescale, st)
   if (D == 96) { HSV_MHA_MMA(96); }
   if (D == 128) { HSV_MHA_MMA(128); }
   if (D == 64) { HSV_MHA_MMA(64); }

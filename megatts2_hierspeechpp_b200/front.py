@@ -22,8 +22,8 @@ from torch import nn
 from torch.nn import Conv1d
 
 from . import ops
-from .modules import (_Folded, _as_input, _bump_on_load, _row_tiles, _side_streams, _weight_norm, Generator,
-                      SourceNetwork, vocode)
+from .modules import (_Folded, _as_input, _bump_on_load, _frame_mask, _lengths_tensor, _row_tiles, _side_streams,
+                      _vl, _weight_norm, Generator, SourceNetwork, vocode)
 
 _S_X, _S_G, _S_W = 4, 5, 6      # blk16 workspace slots of this module family (0..3 and 7 belong to the vocoder)
 _WN_TAIL = __import__("os").environ.get("HSV_WN_TAIL", "1") != "0"   # A/B switch: WN layer tail in the res_skip conv's epilogue
@@ -138,12 +138,13 @@ class _FoldedSlice:
 
 
 def _conv(x: torch.Tensor, f: _Folded, k: int = 1, d: int = 1, mode: int = ops.PACK_MASK, C: Optional[int] = None,
-          slot: int = _S_X, mask=None, bcast=None) -> torch.Tensor:
+          slot: int = _S_X, mask=None, bcast=None, strided: bool = False) -> torch.Tensor:
     """pack (with a fused activation) -> tcgen05 conv.  ``C`` = operand channels when x is wider (prefix / gate).
 
     The tcgen05 kernel keeps the whole [128 x Cin] operand tile in shared memory (Cin <= 512): wider layers
     (pre_source 1024 -> 192, FFN fc2 768 -> 192) run as split-K passes over input-channel slices, each pass adding
-    the previous result in its epilogue (fp32)."""
+    the previous result in its epilogue (fp32).  ``strided``: at any batch size, ONE pack of all channels and passes
+    that read its channel ranges in place (the launches of the batch-1 path; per-item batches use it)."""
     B, cx, L = x.shape
     C = cx if C is None else C
     cout = f.conv.out_channels if hasattr(f.conv, "out_channels") else f.conv.out_features
@@ -162,7 +163,7 @@ def _conv(x: torch.Tensor, f: _Folded, k: int = 1, d: int = 1, mode: int = ops.P
         f._slices = ((C, nsplit), [_FoldedSlice(f, i * per, (i + 1) * per) for i in range(nsplit)])
     out = None
     whole = None
-    if B == 1 and per % ops.blk_cw(C) == 0 and ops.blk_cw(per) == ops.blk_cw(C):
+    if (B == 1 or strided) and per % ops.blk_cw(C) == 0 and ops.blk_cw(per) == ops.blk_cw(C):
         # one batch item: the channel chunks of a blk16 buffer are its outermost dimension, so ONE pack of all C channels
         # serves every pass as a dense sub-buffer
         whole = ops.blk16_buffer(B, C, L, x.device, slot)
@@ -191,15 +192,17 @@ def _slices_of(f: _Folded, C: int):
     return per, f._slices[1]
 
 
-def _conv_packed(buf: torch.Tensor, f: _Folded, C: int, L: int, k: int = 1, d: int = 1) -> torch.Tensor:
+def _conv_packed(buf: torch.Tensor, f: _Folded, C: int, L: int, k: int = 1, d: int = 1,
+                 strided: bool = False) -> torch.Tensor:
     """tcgen05 conv of an already packed operand of C channels; wider than 512: split-K over channel sub-buffers
-    (batch 1 only: the channel chunks are the outermost dimension of the buffer)."""
+    (batch 1, where the channel chunks are the outermost dimension of the buffer, or ``strided``: the passes read
+    the channel ranges in place through the operand's batch stride)."""
     B = buf.shape[0]
     cout = f.conv.out_channels if hasattr(f.conv, "out_channels") else f.conv.out_features
     if C <= 512:
         return _conv_buf(buf, f, L, C, cout, k, d)
-    if B != 1:
-        raise NotImplementedError("split-K over a packed buffer needs batch 1")
+    if B != 1 and not strided:
+        raise NotImplementedError("split-K over a packed buffer needs batch 1 or strided=True")
     per, slices = _slices_of(f, C)
     nchunk = buf.shape[1] * per // C
     out = None
@@ -327,14 +330,25 @@ class PosteriorSFEncoder(nn.Module):
         self._f_proj = _Folded(self.proj)
         _bump_on_load(self)
 
-    def forward(self, x_src, x_ftr, x_mask, g=None):
+    def forward(self, x_src, x_ftr, x_mask, g=None, *, eps=None, noise_scale: float = 1.0, lengths=None):
+        """``eps``: the noise of z = (m + eps * exp(logs) * noise_scale) * mask, fp32 [B, out_channels, T] (default: one
+        ``torch.randn_like(m)`` draw, the reference's :201).  ``lengths`` (frames per item: int CUDA tensor [B] or host
+        sequence): a padded batch whose item b equals its own unpadded run with ``x_mask`` = ones (f0 past
+        4 * lengths[b] is never read, nor is any other input past the item); ``x_mask`` is then derived from them."""
         x_src, x_ftr = _as_input(x_src), _as_input(x_ftr)
-        mask = _mask2d(x_mask)
         B, _, T = x_src.shape
+        vl = _lengths_tensor(lengths, B, T, x_src.device)
+        if vl is not None:
+            x_mask = _frame_mask(vl, T).unsqueeze(1)
+        mask = _mask2d(x_mask)
         H = self.hidden_channels
-        xs = _conv(x_src, self._f_src)
+        if vl is None:
+            xs = _conv(x_src, self._f_src)
+        else:   # the batch-1 split-K launches at every B; padding never enters the operand
+            xs = _conv(x_src, self._f_src, mask=mask, strided=True)
         ops.frame_op(ops.OP_MASK, xs, None, None, mask, xs, None, B, H, T)
-        xf = ops.conv1d_c1_strided(x_ftr, self.pre_filter.weight.detach(), self.pre_filter.bias.detach(), 4, 4, mask)
+        xf = ops.conv1d_c1_strided(x_ftr, self.pre_filter.weight.detach(), self.pre_filter.bias.detach(), 4, 4, mask,
+                                   **_vl(vl))
         if xf.shape[-1] != T:
             raise ValueError(f"f0 has {x_ftr.shape[-1]} frames, expected 4 x {T}")
         if self.parallel_blocks:
@@ -357,10 +371,21 @@ class PosteriorSFEncoder(nn.Module):
         stats = _conv(x, self._f_proj)
         ops.frame_op(ops.OP_MASK, stats, None, None, mask, stats, None, B, 2 * self.out_channels, T)
         m, logs = torch.split(stats, self.out_channels, dim=1)
-        eps = torch.randn_like(m)                      # the reference's draw (:201), same generator, same shape
+        if eps is None:
+            eps = torch.randn_like(m)                  # the reference's draw (:201), same generator, same shape
+        else:
+            _check_eps(eps, B, self.out_channels, T, stats.device)
         z = torch.empty(B, self.out_channels, T, dtype=torch.float32, device=stats.device)
-        ops.frame_op(ops.OP_SAMPLE, stats, eps.contiguous(), None, mask, z, None, B, self.out_channels, T, s=1.0)
+        ops.frame_op(ops.OP_SAMPLE, stats, eps.contiguous(), None, mask, z, None, B, self.out_channels, T,
+                     s=float(noise_scale))
         return z, m, logs
+
+
+def _check_eps(eps, B: int, C: int, T: int, device):
+    if not isinstance(eps, torch.Tensor) or eps.dtype != torch.float32 or eps.device != torch.device(device):
+        raise ValueError(f"eps must be a float32 tensor on {device}")
+    if tuple(eps.shape) != (B, C, T):
+        raise ValueError(f"eps must have shape {(B, C, T)}, got {tuple(eps.shape)}")
 
 
 # ----------------------------------------------------------------------------------------------
@@ -382,16 +407,19 @@ class Attention(nn.Module):
         self._f_qkv = _FoldedLinear(self.qkv)
         self._f_proj = _FoldedLinear(self.proj)
 
-    def run(self, buf: torch.Tensor, C: int, T: int) -> torch.Tensor:
-        """buf = packed (normalised, modulated) input; returns proj(attention) fp32 [B, C, T]."""
+    def run(self, buf: torch.Tensor, C: int, T: int, vl: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """buf = packed (normalised, modulated) input; returns proj(attention) fp32 [B, C, T].  ``vl``: per-item lengths
+        (int32 [B]): item b attends over its own frames only, as its own run does."""
         B = buf.shape[0]
         qkv = _conv_buf(buf, self._f_qkv, T, C, 3 * C)
         D = C // self.num_heads
         flat = qkv.view(-1)
+        if vl is not None and not (ops.MHA_VARIANT[0] == 0 and D in (64, 96, 128)):
+            raise NotImplementedError("per-item lengths need the tensor-core attention (head dim 64, 96 or 128)")
         if ops.MHA_VARIANT[0] == 0 and D in (64, 96, 128):
             # the tensor-core attention writes the proj conv's fp16 operand directly
             ab = ops.mha(flat, flat[C * T:], flat[2 * C * T:], B, self.num_heads, D, T, T, 3 * C * T, 3 * C * T, 3 * C * T,
-                         self.scale, prescale_q=False, out_blk=ops.blk16_buffer(B, C, T, qkv.device, _S_G))
+                         self.scale, prescale_q=False, out_blk=ops.blk16_buffer(B, C, T, qkv.device, _S_G), **_vl(vl))
             ops.check_saturation(ab, C, T)
             return _conv_buf(ab, self._f_proj, T, C, C)
         att = ops.mha(flat, flat[C * T:], flat[2 * C * T:], B, self.num_heads, D, T, T, 3 * C * T, 3 * C * T, 3 * C * T,
@@ -414,18 +442,19 @@ class FFN_Conv(nn.Module):
         self.kernel = kernel
         self._f1, self._f2 = _Folded(self.fc1), _Folded(self.fc2)
 
-    def run(self, buf: torch.Tensor, C: int, T: int, mask) -> torch.Tensor:
-        """fc2(gelu(fc1(buf)) * mask); the trailing * mask is the caller's."""
+    def run(self, buf: torch.Tensor, C: int, T: int, mask, per_item: bool = False) -> torch.Tensor:
+        """fc2(gelu(fc1(buf)) * mask); the trailing * mask is the caller's.  ``per_item``: the batch-1 launches at any
+        batch size (a per-item batch must compute what each item's own run computes)."""
         B = buf.shape[0]
         Hh = self.fc1.out_channels
-        if B == 1 or Hh <= 512:
+        if B == 1 or Hh <= 512 or per_item:
             # fc1's epilogue applies GELU * mask and writes fc2's fp16 operand; fc2 wider than 512 input channels runs as
-            # split-K passes over channel sub-buffers (dense at batch 1)
+            # split-K passes over channel sub-buffers (dense at batch 1, read in place through the batch stride else)
             hb = ops.blk16_buffer(B, Hh, T, buf.device, _S_W)
             wp, nt = self._f1.packed_weight(_row_tiles(B, T))
             ops.conv1d_umma_blk(buf, wp, self._f1.bias(), T, C, Hh, self.kernel, 1, nt, hb, ops.BLK_GELU, mask=mask)
             ops.check_saturation(hb, Hh, T)
-            return _conv_packed(hb, self._f2, Hh, T)
+            return _conv_packed(hb, self._f2, Hh, T, strided=per_item)
         h = _conv_buf(buf, self._f1, T, C, Hh, self.kernel, 1)
         return _conv(h, self._f2, mode=ops.PACK_GELU, slot=_S_W, mask=mask)
 
@@ -443,7 +472,7 @@ class DiTConVBlock(nn.Module):
         self._f_ada = _FoldedLinear(self.adaLN_modulation[1])
 
     def run(self, x: torch.Tensor, c: torch.Tensor, mask, mod: Optional[torch.Tensor] = None,
-            masked_input: bool = False, pending=None, defer: bool = False):
+            masked_input: bool = False, pending=None, defer: bool = False, vl: Optional[torch.Tensor] = None):
         """x fp32 [B, C, T] (updated in place), c [B, C] conditioning, mask [B, T] or None.  Returns (x, pending).
 
         ``mod``: this block's adaLN vector [B, 6C] (rows may be strided) when the caller evaluated all blocks'
@@ -451,7 +480,8 @@ class DiTConVBlock(nn.Module):
         x*m + g*y*m re-masked is the same bits), so the leading mask pass is skipped.  Every gated residual update
         ``x += gate * y * mask`` (:408-409) is fused into the LayerNorm/modulate/pack launch that follows it:
         ``pending`` = the (y, gate) of the previous block's MLP branch still to be applied, ``defer`` = hand this block's
-        own last update to the next block the same way instead of applying it here."""
+        own last update to the next block the same way instead of applying it here.  ``vl``: per-item lengths (int32 [B],
+        ``mask`` their frame mask): attention over each item's own frames, fc1's operand zero past them."""
         B, C, T = x.shape
         if mask is not None and not masked_input:
             ops.frame_op(ops.OP_MASK, x, None, None, mask, x, None, B, C, T)
@@ -466,9 +496,11 @@ class DiTConVBlock(nn.Module):
             if pending[1].stride(0) != ms:
                 raise RuntimeError("DiTConVBlock: pending gate and this block's modulation must share a batch stride")
             ops.gate_ln_mod_blk16(x, pending[0], pending[1], sh1, sc1, buf, ms, mask, 1e-6, premask=True)
-        y = self.attn.run(buf, C, T)
-        ops.gate_ln_mod_blk16(x, y, g1, sh2, sc2, buf, ms, mask, 1e-6, premask=False)
-        y = self.mlp.run(buf, C, T, mask)
+        y = self.attn.run(buf, C, T, vl)
+        # per item: fc1 (k = 5) must see the zero padding of each item's own run past its length
+        ops.gate_ln_mod_blk16(x, y, g1, sh2, sc2, buf, ms, mask, 1e-6, premask=False,
+                              **({} if vl is None else {"zero_masked": True}))
+        y = self.mlp.run(buf, C, T, mask, per_item=vl is not None)
         if defer:
             return x, (y, g2)
         ops.frame_op(ops.OP_GATE_ADD, x, y, g2, mask, x, None, B, C, T, cstride=ms)
@@ -496,12 +528,16 @@ class ResidualCouplingLayer_Transformer_simple(nn.Module):
         self._f_pre, self._f_post = _Folded(self.pre), _Folded(self.post)
         _bump_on_load(self)
 
-    def forward(self, x, x_mask, g=None, reverse=False, mods=None):
+    def forward(self, x, x_mask, g=None, reverse=False, mods=None, *, lengths=None):
         """``mods``: [B, n_layers, 6H] adaLN vectors of this layer's blocks, when the owning
-        ``ResidualCouplingBlock_Transformer`` evaluated them for all its flows at once."""
+        ``ResidualCouplingBlock_Transformer`` evaluated them for all its flows at once.  ``lengths``: as
+        ``ResidualCouplingBlock_Transformer.forward``."""
         if not reverse:
             raise NotImplementedError("inference path: reverse=True only")
         x = _as_input(x)
+        vl = _lengths_tensor(lengths, x.shape[0], x.shape[-1], x.device)
+        if vl is not None:
+            x_mask = _frame_mask(vl, x.shape[-1])
         mask = _mask2d(x_mask)
         B, C, T = x.shape
         half, H = self.half_channels, self.hidden_channels
@@ -510,7 +546,7 @@ class ResidualCouplingLayer_Transformer_simple(nn.Module):
         nb = len(self.enc_block)
         for j, blk in enumerate(self.enc_block):
             h, pending = blk.run(h, g, mask, None if mods is None else mods[:, j], masked_input=j > 0, pending=pending,
-                                 defer=j < nb - 1)
+                                 defer=j < nb - 1, vl=vl)
         m = _conv(h, self._f_post)
         out = x.clone()
         ops.frame_op(ops.OP_COUPLE, out, m, None, mask, out, None, B, half, T)   # x1 = (x1 - m) * mask
@@ -548,10 +584,15 @@ class ResidualCouplingBlock_Transformer(nn.Module):
                                       for blk in self.flows[i].enc_block])
         _bump_on_load(self)
 
-    def forward(self, x, x_mask, g=None, reverse=False):
+    def forward(self, x, x_mask, g=None, reverse=False, *, lengths=None):
+        """``lengths`` (frames per item: int CUDA tensor [B] or host sequence): a padded batch whose item b equals its own
+        unpadded run (x_mask = ones) bit for bit, with 0 past its length; ``x_mask`` is then derived from them."""
         if not reverse:
             raise NotImplementedError("inference path: reverse=True only")
         B = x.shape[0]
+        vl = _lengths_tensor(lengths, B, x.shape[-1], x.device)
+        if vl is not None:
+            x_mask = _frame_mask(vl, x.shape[-1]).unsqueeze(1)
         c = _vec(_vec(_as_input(g).reshape(B, -1), self._f_c0), self._f_c2, silu=True)
         # every DiT block's adaLN modulation depends on c only: ONE launch for all n_flows * n_layers blocks
         # (concatenated weights, cached per checkpoint) instead of one per block on the critical path
@@ -560,7 +601,7 @@ class ResidualCouplingBlock_Transformer(nn.Module):
         for idx in reversed(range(len(self.flows))):
             flow = self.flows[idx]
             if idx % 2 == 0:
-                x = flow(x, x_mask, g=c, reverse=True, mods=mods[:, idx // 2])
+                x = flow(x, x_mask, g=c, reverse=True, mods=mods[:, idx // 2], lengths=vl)
             else:
                 x = flow(x, x_mask, g=c, reverse=True)
         return x
@@ -615,13 +656,15 @@ class MultiHeadAttention(nn.Module):
                 self.conv_k.bias.copy_(self.conv_q.bias)
         self._fq, self._fk, self._fv, self._fo = (_Folded(c) for c in (self.conv_q, self.conv_k, self.conv_v, self.conv_o))
 
-    def run(self, x, lens):
+    def run(self, x, lens, vl: Optional[torch.Tensor] = None):
+        """``lens``: the reference's masked_fill(-1e4) over the padded length; ``vl`` instead: per-item lengths, each
+        item attending over its own frames only, as its own run does."""
         B, C, T = x.shape
         buf = ops.blk16_buffer(B, C, T, x.device, _S_X)
         ops.pack_blk16_act(x, buf, C, ops.PACK_MASK)
         q, k, v = (_conv_buf(buf, f, T, C, C) for f in (self._fq, self._fk, self._fv))
         att = ops.mha(q, k, v, B, self.n_heads, self.k_channels, T, T, C * T, C * T, C * T,
-                      1.0 / math.sqrt(self.k_channels), prescale_q=True, lens=lens)
+                      1.0 / math.sqrt(self.k_channels), prescale_q=True, lens=lens, **_vl(vl))
         return _conv(att, self._fo, slot=_S_G)
 
 
@@ -641,21 +684,28 @@ class StyleEncoder(nn.Module):
         self._f_s0, self._f_s3, self._f_fc = _Folded(self.spectral[0]), _Folded(self.spectral[3]), _Folded(self.fc)
         _bump_on_load(self)
 
-    def forward(self, x, mask=None):
+    def forward(self, x, mask=None, *, lengths=None):
+        """``lengths`` (frames per item: int CUDA tensor [B] or host sequence): a padded batch whose item b equals, bit for
+        bit, its own unpadded run (mask = ones); ``mask`` is then derived from them and x past an item is never used."""
         x = _as_input(x)
         B, _, T = x.shape
         H = self.hidden_dim
+        vl = _lengths_tensor(lengths, B, T, x.device)
+        if vl is not None:
+            mask = _frame_mask(vl, T)
         m2 = _mask2d(mask)
-        lens = None if m2 is None else m2.sum(dim=1).to(torch.int32)        # prefix masks (commons.sequence_mask)
-        h = _conv(x, self._f_s0)                                            # spectral.0
+        lens = None if m2 is None or vl is not None else m2.sum(dim=1).to(torch.int32)   # prefix masks (sequence_mask)
+        # per item: the input's padding is masked out of the first operand, and the first GLU block's output too (its
+        # own run's second GLU conv sees zero padding there)
+        h = _conv(x, self._f_s0, mask=None if vl is None else m2)           # spectral.0
         h = _conv(h, self._f_s3, mode=ops.PACK_MISH)                        # mish -> spectral.3
         ops.frame_op(ops.OP_MISH, h, None, None, m2, h, None, B, H, T)      # mish(...) * mask
-        h = self.temporal[0].run(h, None)
+        h = self.temporal[0].run(h, None if vl is None else m2)
         h = self.temporal[1].run(h, m2)                                     # temporal(x) * mask
-        y = self.slf_attn.run(h, lens)
+        y = self.slf_attn.run(h, lens, vl)
         ops.frame_op(ops.OP_ADD, h, y, None, None, h, None, B, H, T)
         h = _conv(h, self._f_fc)
-        return ops.masked_mean(h, m2)
+        return ops.masked_mean(h, m2, **_vl(vl))
 
 
 # ----------------------------------------------------------------------------------------------
@@ -688,7 +738,14 @@ class HierSpeechSynthesizer(nn.Module):
         self.emb_g = StyleEncoder(in_dim=80, hidden_dim=256, out_dim=gin_channels)
 
     @torch.no_grad()
-    def infer(self, x_mel, w2v, length, f0):
+    def infer(self, x_mel, w2v, length, f0, *, per_item=False, eps=None):
+        """``per_item``: see ``voice_conversion_noise_control``; x_mel [B, 80, T] shares ``length`` with w2v, and ``eps``
+        is the draw inside ``enc_p_l`` (:201).  Returns (waveform, pitch prediction) as the reference does."""
+        if per_item:
+            vl, _ = self._per_item_args(w2v, length, f0, x_mel, None, w2v.shape[0], eps)
+            g = self.emb_g(_as_input(x_mel), lengths=vl).unsqueeze(-1)
+            return self._convert(w2v, vl, f0, g, eps, 1.0, need_pred=True)
+        _no_eps(eps)
         x_mask = torch.unsqueeze(sequence_mask(length, x_mel.size(2)), 1).to(x_mel.dtype)
         g = self.emb_g(x_mel, x_mask).unsqueeze(-1)
         z, _, _ = self.enc_p_l(w2v, f0, x_mask, g=g)
@@ -698,9 +755,29 @@ class HierSpeechSynthesizer(nn.Module):
 
     @torch.no_grad()
     def voice_conversion_noise_control(self, src, src_length, trg_mel, trg_length, f0, noise_scale=0.333, uncond=False,
-                                       denoise_ratio=0):
+                                       denoise_ratio=0, *, per_item=False, eps=None):
+        """``per_item=True``: B utterances of different lengths padded into one batch, each computed exactly as this
+        method (``per_item=False``) computes it alone -- batch 1, unpadded, its own prompts, the same noise -- bit for bit.
+
+        * ``src`` [B, 1024, T] padded; ``src_length`` = frames per item: an int CUDA tensor [B] (never read back, so the
+          call stays capturable) or a host sequence (range-checked to [1, T]).  ``f0`` [B, 1, 4T].
+        * ``trg_mel`` [2B, 80, Tm]: rows [0, B) are each item's prompt, rows [B, 2B) its denoised prompt (B = 1 is the
+          reference's [2, 80, Tm] layout); ``trg_length`` [2B].  Item b uses (1 - r) g[b] + r g[B + b].  (Equality with
+          the item's own call holds when its two prompts have the same length: the own call pads them to each other.)
+        * ``eps``: fp32 CUDA [B, 192, T], the noise multiplying exp(logs_p) (the reference's second draw, :687); item b
+          uses eps[b, :, :len[b]].  With ``eps=None`` one ``randn`` of the padded shape is drawn: capturable, but then an
+          item's noise depends on the batch it is in.
+        * Nothing past an item's length is read (any finite padding gives the same result); the waveform is
+          [B, 1, 320 T] with item b's samples past 320 len[b] exactly 0."""
         if uncond:
             raise NotImplementedError("classifier-free guidance branch (cfg=True models) is not on this path")
+        if per_item:
+            B = src.shape[0]
+            vl, tl = self._per_item_args(src, src_length, f0, trg_mel, trg_length, 2 * B, eps)
+            g = self.emb_g(_as_input(trg_mel), lengths=tl).unsqueeze(-1)
+            g = ((1 - denoise_ratio) * g[:B] + denoise_ratio * g[B:]).contiguous()
+            return self._convert(src, vl, f0, g, eps, noise_scale)[0]
+        _no_eps(eps)
         trg_mask = torch.unsqueeze(sequence_mask(trg_length, trg_mel.size(2)), 1).to(trg_mel.dtype)
         g = self.emb_g(trg_mel, trg_mask).unsqueeze(-1)
         g_org, g_denoise = g[:1, :, :], g[1:, :, :]
@@ -716,9 +793,16 @@ class HierSpeechSynthesizer(nn.Module):
         return vocode(self.sn, self.dec, z, g_interpolation)[0]
 
     @torch.no_grad()
-    def voice_conversion(self, src, src_length, trg_mel, trg_length, f0, noise_scale=0.333, uncond=False):
+    def voice_conversion(self, src, src_length, trg_mel, trg_length, f0, noise_scale=0.333, uncond=False, *,
+                         per_item=False, eps=None):
+        """``per_item``: see ``voice_conversion_noise_control``, with one prompt per item: ``trg_mel`` [B, 80, Tm]."""
         if uncond:
             raise NotImplementedError("classifier-free guidance branch (cfg=True models) is not on this path")
+        if per_item:
+            vl, tl = self._per_item_args(src, src_length, f0, trg_mel, trg_length, src.shape[0], eps)
+            g = self.emb_g(_as_input(trg_mel), lengths=tl).unsqueeze(-1)
+            return self._convert(src, vl, f0, g, eps, noise_scale)[0]
+        _no_eps(eps)
         trg_mask = torch.unsqueeze(sequence_mask(trg_length, trg_mel.size(2)), 1).to(trg_mel.dtype)
         g = self.emb_g(trg_mel, trg_mask).unsqueeze(-1)
         y_mask = torch.unsqueeze(sequence_mask(src_length, src.size(2)), 1).to(trg_mel.dtype)
@@ -730,3 +814,39 @@ class HierSpeechSynthesizer(nn.Module):
         z = self.flow_l(z, y_mask, g=g, reverse=True)
         z = self.flow(z, y_mask, g=g, reverse=True)
         return vocode(self.sn, self.dec, z, g)[0]
+
+    # ---- per-item batches
+    def _per_item_args(self, src, src_length, f0, mel, mel_length, rows: int, eps):
+        """Checks every argument of a per-item call before anything runs; returns the int32 lengths of the source and
+        of the prompts (``mel_length=None``: the prompts share the source's lengths and T, as ``infer``'s x_mel)."""
+        if src.dim() != 3:
+            raise ValueError(f"the source must be [B, C, T], got {tuple(src.shape)}")
+        B, _, T = src.shape
+        vl = _lengths_tensor(src_length, B, T, src.device)
+        Tm = T if mel_length is None else (mel.shape[-1] if mel.dim() == 3 else -1)
+        if tuple(mel.shape) != (rows, self.emb_g.in_dim, Tm):
+            want = f"[{rows}, {self.emb_g.in_dim}, {'T' if mel_length is None else 'Tm'}]"
+            raise ValueError(f"the prompt mel must be {want}, got {tuple(mel.shape)}")
+        tl = vl if mel_length is None else _lengths_tensor(mel_length, rows, Tm, src.device)
+        if tuple(f0.shape) != (B, 1, 4 * T):
+            raise ValueError(f"f0 must be [{B}, 1, {4 * T}], got {tuple(f0.shape)}")
+        if eps is not None:
+            _check_eps(eps, B, self.enc_p_l.out_channels, T, src.device)
+        return vl, tl
+
+    def _convert(self, src, src_length, f0, g, eps, noise_scale: float, need_pred: bool = False):
+        """enc_p_l -> flow_l -> flow -> vocoder of a per-item batch (g [B, gin, 1] per item); returns vocode's pair."""
+        src, f0 = _as_input(src), _as_input(f0)
+        B, _, T = src.shape
+        vl = _lengths_tensor(src_length, B, T, src.device)
+        if eps is None:
+            eps = torch.randn(B, self.enc_p_l.out_channels, T, dtype=torch.float32, device=src.device)
+        z, _, _ = self.enc_p_l(src, f0, None, g=g, eps=eps, noise_scale=noise_scale, lengths=vl)
+        z = self.flow_l(z, None, g=g, reverse=True, lengths=vl)
+        z = self.flow(z, None, g=g, reverse=True, lengths=vl)
+        return vocode(self.sn, self.dec, z, g, need_pred, lengths=vl)
+
+
+def _no_eps(eps):
+    if eps is not None:
+        raise ValueError("eps= is taken with per_item=True (per_item=False draws the reference's noise itself)")

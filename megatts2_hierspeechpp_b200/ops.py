@@ -296,8 +296,12 @@ def conv1d_umma(a_blk: torch.Tensor, w_packed: torch.Tensor, bias: Optional[torc
                 cout: int, k: int, d: int, n_tile: int, residual: Optional[torch.Tensor] = None,
                 out: Optional[torch.Tensor] = None, acc: Optional[torch.Tensor] = None, acc_mode: int = ACC_NONE,
                 acc_div: float = 1.0, want_out: bool = True):
-    """tcgen05 implicit-GEMM Conv1d.  Returns ``out`` (fp32 [B,Cout,L]) or None if want_out=False."""
-    _req(a_blk, "a_blk16", torch.float16, 4); _req(w_packed, "w_packed", torch.float16)
+    """tcgen05 implicit-GEMM Conv1d.  Returns ``out`` (fp32 [B,Cout,L]) or None if want_out=False.
+
+    ``a_blk`` may also be a channel range of a wider blk16 buffer, ``buf[:, c0 // CW:(c0 + cin) // CW]`` with the same
+    CW (a split-K pass over one packed operand): read in place through the A operand's batch stride."""
+    _req_blk_view(a_blk, "a_blk16")
+    _req(w_packed, "w_packed", torch.float16)
     B = a_blk.shape[0]
     if tuple(a_blk.shape) != blk16_shape(B, cin, L):
         raise ValueError(f"a_blk16 shape {tuple(a_blk.shape)} does not match Cin={cin}, L={L}")
@@ -315,9 +319,24 @@ def conv1d_umma(a_blk: torch.Tensor, w_packed: torch.Tensor, bias: Optional[torc
     if acc is not None and tuple(acc.shape) != (B, cout, L):
         raise ValueError("acc shape mismatch")
     lib = _lib.load()
-    _lib.check(lib.hsv_conv1d_umma(_p(a_blk), _p(w_packed), _p(bias), _p(residual), _p(out), _p(acc), acc_mode,
-                                   float(acc_div), B, cin, cout, L, k, d, n_tile, _stream()), "hsv_conv1d_umma")
+    if a_blk.is_contiguous():
+        _lib.check(lib.hsv_conv1d_umma(_p(a_blk), _p(w_packed), _p(bias), _p(residual), _p(out), _p(acc), acc_mode,
+                                       float(acc_div), B, cin, cout, L, k, d, n_tile, _stream()), "hsv_conv1d_umma")
+    else:
+        _lib.check(lib.hsv_conv1d_umma_astride(_p(a_blk), a_blk.stride(0) // a_blk.stride(1), _p(w_packed), _p(bias),
+                                               _p(residual), _p(out), _p(acc), acc_mode, B, cin, cout, L, k, d, n_tile,
+                                               _stream()), "hsv_conv1d_umma_astride")
     return out
+
+
+def _req_blk_view(t: torch.Tensor, name: str):
+    """A blk16 operand: a contiguous buffer, or a chunk range of one (dense inside each batch item, any batch stride)."""
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float16 and t.dim() == 4) or t.is_contiguous():
+        _req(t, name, torch.float16, 4)
+        return
+    _, nc, rows, cw = t.shape
+    if t.stride(3) != 1 or t.stride(2) != cw or t.stride(1) != rows * cw or t.stride(0) % t.stride(1):
+        raise ValueError(f"{name}: a non-contiguous operand must be a chunk range of a contiguous blk16 buffer")
 
 
 BLK_NONE, BLK_GATE, BLK_GELU, BLK_LRELU = 0, 1, 2, 3
@@ -645,9 +664,14 @@ def wn_res_pack(x: torch.Tensor, rs: torch.Tensor, mask: Optional[torch.Tensor],
     return buf
 
 
+LN_ZERO_MASKED = 2
+
+
 def ln_mod_blk16(x: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor, buf: torch.Tensor, mod_stride: int,
-                 mask: Optional[torch.Tensor] = None, eps: float = 1e-6, inmask: bool = False, premask: bool = False):
-    """LayerNorm over channels (no affine) [* mask] -> x * (1 + scale[b]) + shift[b] -> fp16 blk16."""
+                 mask: Optional[torch.Tensor] = None, eps: float = 1e-6, inmask: bool = False, premask: bool = False,
+                 zero_masked: bool = False):
+    """LayerNorm over channels (no affine) [* mask] -> x * (1 + scale[b]) + shift[b] -> fp16 blk16.  ``zero_masked``:
+    operand rows where mask == 0 are written as zero (rows past an item of a ragged batch)."""
     _req(x, "x", ndim=3); _req_vec(shift, "shift"); _req_vec(scale, "scale"); _req(buf, "buf", torch.float16, 4)
     B, C, L = x.shape
     if tuple(buf.shape) != blk16_shape(B, C, L):
@@ -655,16 +679,19 @@ def ln_mod_blk16(x: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor, buf:
     if mask is not None:
         _req(mask, "mask")
     lib = _lib.load()
+    if zero_masked and mask is None:
+        raise ValueError("ln_mod_blk16: zero_masked needs a mask")
     _lib.check(lib.hsv_ln_mod_blk16(_p(x), _p(shift), _p(scale), _p(mask), _p(buf), B, C, L, float(eps), int(inmask),
-                                    int(premask), int(mod_stride), _stream()), "hsv_ln_mod_blk16")
+                                    int(premask) | (LN_ZERO_MASKED if zero_masked else 0), int(mod_stride), _stream()),
+               "hsv_ln_mod_blk16")
     return buf
 
 
 def gate_ln_mod_blk16(x: torch.Tensor, y: torch.Tensor, gate: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor,
                       buf: torch.Tensor, mod_stride: int, mask: Optional[torch.Tensor] = None, eps: float = 1e-6,
-                      premask: bool = False):
+                      premask: bool = False, zero_masked: bool = False):
     """x += gate[b] * y * mask (in place), then ``ln_mod_blk16`` of the new x: one launch.  gate/shift/scale are row views
-    of one modulation tensor (batch stride ``mod_stride``)."""
+    of one modulation tensor (batch stride ``mod_stride``); ``zero_masked`` as ``ln_mod_blk16``."""
     _req(x, "x", ndim=3); _req(y, "y", ndim=3); _req_vec(gate, "gate"); _req_vec(shift, "shift"); _req_vec(scale, "scale")
     _req(buf, "buf", torch.float16, 4)
     B, C, L = x.shape
@@ -672,8 +699,12 @@ def gate_ln_mod_blk16(x: torch.Tensor, y: torch.Tensor, gate: torch.Tensor, shif
         raise ValueError("gate_ln_mod_blk16: shape mismatch")
     if mask is not None:
         _req(mask, "mask")
+    elif zero_masked:
+        raise ValueError("gate_ln_mod_blk16: zero_masked needs a mask")
     _lib.check(_lib.load().hsv_gate_ln_mod_blk16(_p(x), _p(y), _p(gate), int(mod_stride), _p(shift), _p(scale), _p(mask),
-                                                 _p(buf), B, C, L, float(eps), int(premask), int(mod_stride), _stream()),
+                                                 _p(buf), B, C, L, float(eps),
+                                                 int(premask) | (LN_ZERO_MASKED if zero_masked else 0), int(mod_stride),
+                                                 _stream()),
                "hsv_gate_ln_mod_blk16")
     return buf
 
@@ -691,16 +722,32 @@ def frame_op(op: int, a, b=None, c=None, mask=None, out=None, out2=None, B=0, C=
 
 def mha(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, heads: int, D: int, Tq: int, Tk: int, q_bs: int,
         k_bs: int, v_bs: int, scale: float, prescale_q: bool, lens: Optional[torch.Tensor] = None,
-        out_blk: Optional[torch.Tensor] = None) -> torch.Tensor:
+        out_blk: Optional[torch.Tensor] = None, valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
     """softmax(q k^T * scale) v; q/k/v may be views into one fused [B, 3*heads*D, T] tensor (pass batch strides).
     ``out_blk``: write the result as the fp16 blk16 operand of the conv that follows (tensor-core kernel only) and
-    return that buffer instead of a fp32 tensor."""
+    return that buffer instead of a fp32 tensor.  ``valid_len`` (int32 [B], self-attention, not with ``lens``): item b
+    is its first valid_len[b] frames as if run alone with Tq = Tk = valid_len[b]; its rows past that are 0."""
     for t, n in ((q, "q"), (k, "k"), (v, "v")):
         if not t.is_cuda or t.dtype != torch.float32:
             raise RuntimeError(f"mha: {n} must be a CUDA float32 tensor")
     if lens is not None:
         _req(lens, "lens", torch.int32)
     lib = _lib.load()
+    if valid_len is not None:
+        _req_len(valid_len, B, q.device)
+        if lens is not None or Tq != Tk:
+            raise ValueError("mha: valid_len is per-item self-attention (Tq == Tk, no lens)")
+        if out_blk is not None:
+            _req(out_blk, "out_blk", torch.float16, 4)
+            if tuple(out_blk.shape) != blk16_shape(B, heads * D, Tq):
+                raise ValueError("mha: blk16 buffer shape mismatch")
+            out = out_blk
+        else:
+            out = torch.empty(B, heads * D, Tq, dtype=torch.float32, device=q.device)
+        _lib.check(lib.hsv_mha_ragged(_p(q), _p(k), _p(v), _p(out), int(out_blk is not None), None, _p(valid_len), B, heads,
+                                      D, Tq, Tk, int(q_bs), int(k_bs), int(v_bs), float(scale), int(prescale_q), _stream()),
+                   "hsv_mha_ragged")
+        return out
     if out_blk is not None:
         _req(out_blk, "out_blk", torch.float16, 4)
         if tuple(out_blk.shape) != blk16_shape(B, heads * D, Tq):
@@ -715,7 +762,9 @@ def mha(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, B: int, heads: int, D
 
 
 def conv1d_c1_strided(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], stride: int, pad: int,
-                      mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+                      mask: Optional[torch.Tensor] = None, valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Conv1d(1, Cout, k, stride, pad) * mask.  ``valid_len`` (int32 [B], output frames): item b reads
+    x[b, 0, :stride * valid_len[b]] only, as its own run with that many samples, and its output past valid_len[b] is 0."""
     _req(x, "x", ndim=3); _req(w, "w", ndim=3)
     B, one, Lin = x.shape
     cout, one_w, k = w.shape
@@ -724,17 +773,29 @@ def conv1d_c1_strided(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Ten
     Lout = (Lin + 2 * pad - k) // stride + 1
     out = torch.empty(B, cout, Lout, dtype=torch.float32, device=x.device)
     lib = _lib.load()
-    _lib.check(lib.hsv_conv1d_c1_strided(_p(x), _p(w), _p(bias), _p(mask), _p(out), B, cout, Lin, Lout, k, stride, pad,
-                                         _stream()), "hsv_conv1d_c1_strided")
+    if valid_len is not None:
+        _req_len(valid_len, B, x.device)
+        _lib.check(lib.hsv_conv1d_c1_strided_ragged(_p(x), _p(w), _p(bias), _p(mask), _p(valid_len), _p(out), B, cout, Lin,
+                                                    Lout, k, stride, pad, _stream()), "hsv_conv1d_c1_strided_ragged")
+    else:
+        _lib.check(lib.hsv_conv1d_c1_strided(_p(x), _p(w), _p(bias), _p(mask), _p(out), B, cout, Lin, Lout, k, stride, pad,
+                                             _stream()), "hsv_conv1d_c1_strided")
     return out
 
 
-def masked_mean(x: torch.Tensor, mask: Optional[torch.Tensor]) -> torch.Tensor:
+def masked_mean(x: torch.Tensor, mask: Optional[torch.Tensor], valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """x.sum(2) / mask.sum(2) over all L frames; ``valid_len`` (int32 [B]): item b's mean over its first valid_len[b]
+    frames, summed in the order of its own run (the mask is then not read)."""
     _req(x, "x", ndim=3)
     B, C, L = x.shape
     out = torch.empty(B, C, dtype=torch.float32, device=x.device)
     lib = _lib.load()
-    _lib.check(lib.hsv_masked_mean(_p(x), _p(mask), _p(out), B, C, L, _stream()), "hsv_masked_mean")
+    if valid_len is not None:
+        _req_len(valid_len, B, x.device)
+        _lib.check(lib.hsv_masked_mean_ragged(_p(x), _p(mask), _p(valid_len), _p(out), B, C, L, _stream()),
+                   "hsv_masked_mean_ragged")
+    else:
+        _lib.check(lib.hsv_masked_mean(_p(x), _p(mask), _p(out), B, C, L, _stream()), "hsv_masked_mean")
     return out
 
 

@@ -176,6 +176,21 @@ def ragged_batches(indices: Sequence[int], lengths: Sequence[int], max_batch: in
     return out
 
 
+def ragged_prompt_batches(indices: Sequence[int], lengths: Sequence[int], prompt_lengths: Sequence[int], max_batch: int,
+                          frame_multiple: int = 50, prompt_multiple: int = 50) -> List[Tuple[List[int], int, int]]:
+    """Micro-batches for the per-item voice-conversion calls (``HierSpeechSynthesizer.*(..., per_item=True)``):
+    ``ragged_batches`` of the source lengths, each with its prompts padded to their longest rounded up to a multiple
+    of ``prompt_multiple``: [(ids, T_padded, Tm_padded)].  Both roundings bound the number of distinct padded shapes
+    (one captured CUDA graph each)."""
+    if prompt_multiple < 1:
+        raise ValueError("prompt_multiple must be >= 1")
+    out = []
+    for ids, T in ragged_batches(indices, lengths, max_batch, frame_multiple):
+        longest = max(int(prompt_lengths[i]) for i in ids)
+        out.append((ids, T, -(-longest // prompt_multiple) * prompt_multiple))
+    return out
+
+
 def gather_packed(flat: torch.Tensor, dst: int = 0):
     """The collective under ``gather_waveforms``: every rank contributes one 1-D buffer of the SAME size and dtype
     (pad to the largest shard), rank ``dst`` gets a [world, n] tensor, the others None.  No metadata exchange, no
