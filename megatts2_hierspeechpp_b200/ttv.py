@@ -20,8 +20,8 @@ from torch.nn import Conv1d, ConvTranspose1d
 
 from . import ops
 from .front import WN, _conv, _mask2d, _vec
-from .modules import (_Folded, _MAIN_SLOT, _as_input, _bump_on_load, _row_tiles, _weight_norm, get_padding,
-                      sum_of_blocks)
+from .modules import (_Folded, _MAIN_SLOT, _as_input, _bump_on_load, _frame_mask, _hops, _length_table,
+                      _lengths_tensor, _row_tiles, _vl, _weight_norm, get_padding, sum_of_blocks)
 
 LRELU_SLOPE = 0.1
 _SLOT2 = 12       # second operand workspace of a resblock stream (slots 0..2 -> 12..14)
@@ -47,10 +47,16 @@ class W2VDecoder(nn.Module):
         self._f_proj = _Folded(self.proj)
         _bump_on_load(self)
 
-    def forward(self, x, x_mask, g=None):
-        x = _as_input(x)
-        mask = _mask2d(x_mask)
+    def forward(self, x, x_mask, g=None, *, lengths=None):
+        """``lengths`` (frames per item: int CUDA tensor [B] or host sequence): a padded batch whose item b equals, bit for
+        bit, its own unpadded run with ``x_mask`` = ones, with 0 past its length; ``x_mask`` is then derived from them (the
+        one passed is not read) and x past an item is never used."""
         B, _, T = x.shape
+        vl = _lengths_tensor(lengths, B, T, x.device)
+        x = _as_input(x)
+        if vl is not None:
+            x_mask = _frame_mask(vl, T).unsqueeze(1)
+        mask = _mask2d(x_mask)
         h = _conv(x, self._f_pre, mask=mask)                     # pre(x * x_mask)
         ops.frame_op(ops.OP_MASK, h, None, None, mask, h, None, B, self.hidden_channels, T)
         h = self.enc(h, x_mask, g=g)
@@ -78,8 +84,10 @@ class ResBlock1(nn.Module):
         _bump_on_load(self)
 
     def run(self, x: torch.Tensor, slot: int = 0, acc: Optional[torch.Tensor] = None, acc_mode: int = ops.ACC_NONE,
-            before_final=None) -> Optional[torch.Tensor]:
-        """Same contract as ``AMPBlock1.run``: x is not modified; with ``acc`` the result is only accumulated."""
+            before_final=None, valid_len: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
+        """Same contract as ``AMPBlock1.run``: x is not modified; with ``acc`` the result is only accumulated.
+        ``valid_len`` (int32 [B]): item b is x[b, :, :valid_len[b]]; the output below that equals the item's own run, past
+        it it is not meaningful (every operand built from it is zero there, as in the item's own run)."""
         B, C, L = x.shape
         if C != self.channels or C % 16:
             raise ValueError(f"ResBlock1 expects {self.channels} channels (multiple of 16), got {C}")
@@ -89,14 +97,16 @@ class ResBlock1(nn.Module):
         cur = x
         nl = len(self.dilation)
         rt = _row_tiles(B, L)
+        mask = None if valid_len is None else _frame_mask(valid_len, L)
         for i, d in enumerate(self.dilation):
             last = i == nl - 1
             w1, nt1 = self._f1[i].packed_weight(rt)
             w2, nt2 = self._f2[i].packed_weight(rt)
-            ops.pack_blk16(cur, buf, True)
+            ops.pack_blk16(cur, buf, True, **_vl(valid_len))
             ops.check_saturation(buf, C, L)
-            # c1's epilogue applies the second leaky_relu and writes c2's fp16 operand (no fp32 round trip, no pack)
-            ops.conv1d_umma_blk(buf, w1, self._f1[i].bias(), L, C, C, k, d, nt1, buf2, ops.BLK_LRELU)
+            # c1's epilogue applies the second leaky_relu and writes c2's fp16 operand (no fp32 round trip, no pack);
+            # with lengths, the mask gives that operand the zero tail of the item's own run
+            ops.conv1d_umma_blk(buf, w1, self._f1[i].bias(), L, C, C, k, d, nt1, buf2, ops.BLK_LRELU, mask=mask)
             ops.check_saturation(buf2, C, L)
             buf, buf2 = buf2, buf
             if last and before_final is not None:
@@ -170,11 +180,19 @@ class PitchPredictor(nn.Module):
             self._post_key = key
         return self._post_w
 
-    def forward(self, x, g):
-        x, g = _as_input(x), _as_input(g)
+    def forward(self, x, g, *, lengths=None):
+        """``lengths`` (frames of x per item: int CUDA tensor [B] or host sequence): a padded batch whose item b's pitch
+        [:4 * lengths[b]] equals, bit for bit, its own unpadded run, with 0 past it; x past an item is never used.
+        ``lengths=None`` is the reference's call, which runs the padding through like any other frame."""
         B, _, T = x.shape
+        V = _length_table(lengths, B, T, x.device, _hops(self.upsample_rates))
+        vl = (lambda i: None) if V is None else (lambda i: V[i])
+        x, g = _as_input(x), _as_input(g)
         c0 = self.conv_pre.out_channels
-        h = _conv(x, self._f_pre, k=7)                                        # split-K over the 1024 input channels
+        if V is None:
+            h = _conv(x, self._f_pre, k=7)                                    # split-K over the 1024 input channels
+        else:   # the batch-1 split-K launches at every B; padding never enters the operand
+            h = _conv(x, self._f_pre, k=7, mask=_frame_mask(V[0], T), strided=True)
         cg = _vec(g.reshape(B, -1), self._f_cond)
         ops.frame_op(ops.OP_ADD_BCAST, h, None, cg, None, h, None, B, c0, T, cstride=c0)
         sc = 1.0
@@ -183,15 +201,17 @@ class PitchPredictor(nn.Module):
             cin = (h[0] if isinstance(h, list) else h).shape[1]
             f = self._f_ups[i]
             buf = ops.blk16_buffer(B, cin, L, x.device, _MAIN_SLOT)
-            ops.pack_blk16(h, buf, True, scale=sc)                            # leaky_relu(x / num_kernels, 0.1)
+            ops.pack_blk16(h, buf, True, scale=sc, **_vl(vl(i)))             # leaky_relu(x / num_kernels, 0.1)
             ops.check_saturation(buf, cin, L)
             wp, nt = f.packedT_weight(self.upsample_rates[i], _row_tiles(B, L))
             h = ops.conv_transpose1d_umma(buf, wp, f.bias(), L, cin, f.conv.out_channels,
                                           self.ups[i].kernel_size[0], self.upsample_rates[i], nt)
             L *= self.upsample_rates[i]
             blocks: Sequence[ResBlock1] = self.resblocks[i * self.num_kernels:(i + 1) * self.num_kernels]
-            h, sc = sum_of_blocks(h, blocks, parallel=self.parallel_blocks, separate=i < self.num_upsamples - 1)
-        return ops.conv1d_direct(h, self._post_weight(sc), None, pad=3, flags=ops.CONV_LRELU001_IN)
+            h, sc = sum_of_blocks(h, blocks, parallel=self.parallel_blocks, separate=i < self.num_upsamples - 1,
+                                  valid_len=vl(i + 1))
+        return ops.conv1d_direct(h, self._post_weight(sc), None, pad=3, flags=ops.CONV_LRELU001_IN,
+                                 **_vl(vl(self.num_upsamples)))
 
     def remove_weight_norm(self):
         for l in self.ups:
@@ -204,7 +224,13 @@ class PitchPredictor(nn.Module):
 class TTVTail(nn.Module):
     """``w2v_decoder`` + ``pp`` under the reference's attribute names, so a text-to-vec checkpoint's
     ``w2v_decoder.*`` / ``pp.*`` entries load with ``load_state_dict(..., strict=False)`` and the synthetic
-    ``ttv_tail_sd`` loads strictly.  ``forward(z, y_mask, g) -> (w2v, pitch)`` (:1109-1110)."""
+    ``ttv_tail_sd`` loads strictly.  ``forward(z, y_mask, g) -> (w2v, pitch)`` (:1109-1110).
+
+    ``forward(z, y_mask, g, lengths=...)`` (frames of z per item: int CUDA tensor [B] or host sequence): a padded batch
+    whose item b's w2v [:lengths[b]] and pitch [:4 * lengths[b]] equal, bit for bit, ``forward`` on that item alone with
+    ``y_mask`` = ones, with 0 past them; ``y_mask`` may be passed but is not read, and z past an item is never used.
+    Its outputs go on as they are to ``HierSpeechSynthesizer.voice_conversion_noise_control(w2v, lengths, ..., pitch,
+    per_item=True)``."""
 
     def __init__(self, inter_channels: int = 256, gin_channels: int = 256):
         super().__init__()
@@ -212,6 +238,7 @@ class TTVTail(nn.Module):
                                       gin_channels=gin_channels)
         self.pp = PitchPredictor()
 
-    def forward(self, z, y_mask, g):
-        w2v = self.w2v_decoder(z, y_mask, g=g)
-        return w2v, self.pp(w2v, g)
+    def forward(self, z, y_mask, g, *, lengths=None):
+        vl = _lengths_tensor(lengths, z.shape[0], z.shape[-1], z.device)
+        w2v = self.w2v_decoder(z, y_mask, g=g, lengths=vl)
+        return w2v, self.pp(w2v, g, lengths=vl)
