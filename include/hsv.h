@@ -268,6 +268,10 @@ int hsv_blk16_stats(const void *in, void *stats, int B, int C, int64_t L, void *
  */
 int hsv_peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1, float s2,
                         int per_row, void *stream);
+/* the same with one peak and one s2 per row: s2 [rows] fp32, device (the prompt peak of each utterance,
+ * inference_plm.py:183-188 with scale_norm="prompt").  Row b equals hsv_peak_norm_pcm16 of row b alone with s2[b]. */
+int hsv_peak_norm_pcm16_rows(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1,
+                             const float *s2, void *stream);
 
 /* ---- frame-rate operators of the step BEFORE the vocoder (SURVEY.md §8f2; csrc/frame_ops.cu).  fp32 [B,C,T] tensors,
  * mask = [B,T] (1 = valid frame, may be NULL), blk16 outputs feed hsv_conv1d_umma.
@@ -336,6 +340,19 @@ int hsv_masked_mean(const float *x, const float *mask, float *out, int B, int C,
  * valid_len[b]; mask is not read. */
 int hsv_masked_mean_ragged(const float *x, const float *mask, const int32_t *valid_len, float *out, int B, int C,
                            int64_t L, void *stream);
+
+/* ---- seeded noise of per-item batches (csrc/noise.cu).  The value at (item b, channel c, frame t) depends on
+ * (seeds[b], c, t) only: Philox4x32-10 keyed by the 64-bit seed, counter (t >> 2, c, 0, 0), Box-Muller normal t & 3.
+ * This is the project's own bit pattern, not torch's randn stream.  seeds [B] int64, valid_len [B] int32 (NULL = T),
+ * both device; 1 <= T <= 2^34.
+ * hsv_seeded_normal: out [B, C, T] fp32 = the normals, 0 at t >= valid_len[b].
+ * hsv_sample_ragged: out [B, C, T] = m + n * exp(logs) * s_b with stats [B, 2C, T] = (m | logs), in the operation order
+ *   and with the expf of hsv_frame_op's sample op (so its output equals that op fed with the same noise and mask 1);
+ *   0 at t >= valid_len[b], where nothing is read or generated.  n: generated in registers from seeds (eps NULL) or
+ *   read from eps [B, C, T] (seeds NULL); s_b = noise_scale[b] ([B] fp32, device) or s when noise_scale is NULL. */
+int hsv_seeded_normal(const int64_t *seeds, float *out, int B, int C, int64_t T, const int32_t *valid_len, void *stream);
+int hsv_sample_ragged(const float *stats, const float *eps, const int64_t *seeds, const float *noise_scale, float s,
+                      const int32_t *valid_len, float *out, int B, int C, int64_t T, void *stream);
 
 /* ---- f0-driven harmonic sine source (BASELINE.json north_star item 3; NSF / HiFTNet-style SineGen -- the
  * reference repository has no counterpart on this path, SURVEY.md §0.3).  The phase accumulator is 64-bit fixed point

@@ -80,10 +80,14 @@ SIGNATURES = {
                                              c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
     "hsv_masked_mean": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
     "hsv_masked_mean_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p]),
+    "hsv_seeded_normal": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p, c_void_p]),
+    "hsv_sample_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_int, c_int,
+                                  c_int64, c_void_p]),
     "hsv_sinegen_workspace": (c_int64, [c_int, c_int64, c_int]),
     "hsv_sinegen": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int, c_float, c_int, c_float,
                             c_void_p]),
     "hsv_peak_norm_pcm16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_float, c_float, c_int, c_void_p]),
+    "hsv_peak_norm_pcm16_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_float, c_void_p, c_void_p]),
 }
 
 # bring-up aids exported by the library but not part of the drop-in contract

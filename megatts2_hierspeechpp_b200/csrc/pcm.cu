@@ -26,10 +26,14 @@ __global__ void absmax_kernel(const float *__restrict__ x, unsigned int *__restr
   if ((threadIdx.x & 31) == 0 && m) atomicMax(peak_bits + row, m);
 }
 
+// ROW_S2: s2 = s2_row[row] (one prompt peak per utterance), else the scalar s2
+template <bool ROW_S2>
 __global__ void pcm16_kernel(const float *__restrict__ x, const unsigned int *__restrict__ peak_bits,
-                             int16_t *__restrict__ out, int64_t L, int peak_stride, float s1, float s2) {
+                             int16_t *__restrict__ out, int64_t L, int peak_stride, float s1, float s2,
+                             const float *__restrict__ s2_row) {
   const int row = blockIdx.y;
   const float peak = __uint_as_float(peak_bits[row * peak_stride]);
+  if (ROW_S2) s2 = __ldg(s2_row + row);
   const float *xr = x + (int64_t)row * L;
   int16_t *orow = out + (int64_t)row * L;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < L; i += (int64_t)gridDim.x * blockDim.x) {
@@ -54,8 +58,8 @@ __global__ void rowmax_kernel(unsigned int *peak_bits, int rows) {
 
 }  // namespace
 
-extern "C" int hsv_peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1,
-                                   float s2, int per_row, void *stream) {
+static int peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1, float s2,
+                           const float *s2_row, int per_row, void *stream) {
   if (rows == 0 || L == 0) return HSV_OK;  // empty batch / sequence
   HSV_REQUIRE(x && out && peak_ws, "peak_norm_pcm16: null pointer");
   HSV_REQUIRE(rows > 0 && rows <= 65535 && L > 0, "peak_norm_pcm16: bad shape rows=%d L=%lld", rows, (long long)L);
@@ -71,6 +75,20 @@ extern "C" int hsv_peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws,
   gx = gx < 1 ? 1 : (gx > 148 * 8 ? 148 * 8 : gx);
   absmax_kernel<<<dim3(gx, rows), 256, 0, st>>>(x, bits, L);
   if (!per_row && rows > 1) rowmax_kernel<<<1, 32, 0, st>>>(bits, rows);
-  pcm16_kernel<<<dim3(gx, rows), 256, 0, st>>>(x, bits, out, L, per_row ? 1 : 0, s1, s2);
+  if (s2_row)
+    pcm16_kernel<true><<<dim3(gx, rows), 256, 0, st>>>(x, bits, out, L, 1, s1, s2, s2_row);
+  else
+    pcm16_kernel<false><<<dim3(gx, rows), 256, 0, st>>>(x, bits, out, L, per_row ? 1 : 0, s1, s2, nullptr);
   return hsv::check_launch("peak_norm_pcm16");
+}
+
+extern "C" int hsv_peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1,
+                                   float s2, int per_row, void *stream) {
+  return peak_norm_pcm16(x, out, peak_ws, rows, L, s1, s2, nullptr, per_row, stream);
+}
+
+extern "C" int hsv_peak_norm_pcm16_rows(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1,
+                                        const float *s2, void *stream) {
+  HSV_REQUIRE(s2 || rows == 0 || L == 0, "peak_norm_pcm16_rows: null s2");
+  return peak_norm_pcm16(x, out, peak_ws, rows, L, s1, 0.f, s2, 1, stream);
 }

@@ -15,6 +15,7 @@ Inference only (``reverse=True`` for the flows, eval-mode dropout).  CUDA tensor
 from __future__ import annotations
 
 import math
+import numbers
 from typing import Optional
 
 import torch
@@ -330,14 +331,18 @@ class PosteriorSFEncoder(nn.Module):
         self._f_proj = _Folded(self.proj)
         _bump_on_load(self)
 
-    def forward(self, x_src, x_ftr, x_mask, g=None, *, eps=None, noise_scale: float = 1.0, lengths=None):
+    def forward(self, x_src, x_ftr, x_mask, g=None, *, eps=None, noise_scale=1.0, lengths=None, seed=None):
         """``eps``: the noise of z = (m + eps * exp(logs) * noise_scale) * mask, fp32 [B, out_channels, T] (default: one
         ``torch.randn_like(m)`` draw, the reference's :201).  ``lengths`` (frames per item: int CUDA tensor [B] or host
         sequence): a padded batch whose item b equals its own unpadded run with ``x_mask`` = ones (f0 past
-        4 * lengths[b] is never read, nor is any other input past the item); ``x_mask`` is then derived from them."""
-        x_src, x_ftr = _as_input(x_src), _as_input(x_ftr)
+        4 * lengths[b] is never read, nor is any other input past the item); ``x_mask`` is then derived from them.
+        With ``lengths`` only: ``seed`` (int64 CUDA tensor [B] or host sequence; not with ``eps``) generates item b's noise
+        from seed[b] inside the sampling launch, equal to ``eps = ops.seeded_normal(seed[b:b+1], out_channels, len[b])``;
+        ``noise_scale`` may be a floating CUDA tensor [B] (item b as with ``float(noise_scale[b])``)."""
         B, _, T = x_src.shape
         vl = _lengths_tensor(lengths, B, T, x_src.device)
+        seeds = _per_item_noise_args(vl is not None, B, x_src.device, eps, seed, noise_scale=noise_scale)
+        x_src, x_ftr = _as_input(x_src), _as_input(x_ftr)
         if vl is not None:
             x_mask = _frame_mask(vl, T).unsqueeze(1)
         mask = _mask2d(x_mask)
@@ -371,6 +376,15 @@ class PosteriorSFEncoder(nn.Module):
         stats = _conv(x, self._f_proj)
         ops.frame_op(ops.OP_MASK, stats, None, None, mask, stats, None, B, 2 * self.out_channels, T)
         m, logs = torch.split(stats, self.out_channels, dim=1)
+        per_item_ns = vl is not None and _per_item_control(noise_scale, B, stats.device)
+        if seeds is not None or per_item_ns:
+            if eps is not None:
+                _check_eps(eps, B, self.out_channels, T, stats.device)
+            elif seeds is None:
+                eps = torch.randn_like(m)
+            ns = noise_scale.to(torch.float32).contiguous() if per_item_ns else float(noise_scale)
+            z = ops.sample_ragged(stats, ns, vl, eps=None if eps is None else eps.contiguous(), seeds=seeds)
+            return z, m, logs
         if eps is None:
             eps = torch.randn_like(m)                  # the reference's draw (:201), same generator, same shape
         else:
@@ -379,6 +393,55 @@ class PosteriorSFEncoder(nn.Module):
         ops.frame_op(ops.OP_SAMPLE, stats, eps.contiguous(), None, mask, z, None, B, self.out_channels, T,
                      s=float(noise_scale))
         return z, m, logs
+
+
+def _seeds_tensor(seed, B: int, device) -> torch.Tensor:
+    """Per-item seeds as a contiguous int64 [B] tensor on ``device``: an int64 tensor there is only checked (never read
+    back, so the call stays capturable); a host sequence of ints in the int64 range is copied."""
+    device = torch.device(device)
+    if isinstance(seed, torch.Tensor):
+        if seed.device != device:
+            raise ValueError(f"seed is on {seed.device}, the input is on {device}")
+        if tuple(seed.shape) != (B,) or seed.dtype != torch.int64:
+            raise ValueError(f"seed must be an int64 tensor of shape ({B},), got {seed.dtype} {tuple(seed.shape)}")
+        return seed.contiguous()
+    try:
+        if isinstance(seed, (str, bytes)):
+            raise TypeError
+        vals = list(seed)
+    except TypeError:
+        raise ValueError("seed must be a tensor or a sequence with one seed per item") from None
+    if len(vals) != B:
+        raise ValueError(f"seed has {len(vals)} entries for a batch of {B}")
+    if any(not isinstance(v, numbers.Integral) for v in vals):
+        raise ValueError("seeds must be integers")
+    vals = [int(v) for v in vals]
+    if any(not -(1 << 63) <= v < (1 << 63) for v in vals):
+        raise ValueError("seeds must lie in the int64 range")
+    return torch.tensor(vals, dtype=torch.int64, device=device)
+
+
+def _per_item_control(v, B: int, device) -> bool:
+    """noise_scale / denoise_ratio of a per-item call: a floating tensor of shape (B,) on the input's device holds one
+    value per item; a Python number or any other one-element tensor is one value for the whole call, as before."""
+    return (isinstance(v, torch.Tensor) and v.is_floating_point() and tuple(v.shape) == (B,)
+            and v.device == torch.device(device))
+
+
+def _per_item_noise_args(per_item: bool, B: int, device, eps, seed, **controls) -> Optional[torch.Tensor]:
+    """Checks ``seed`` and the controls of a call (a tensor of more than one element is per item: per-item calls only,
+    and there a floating [B] tensor on the input's device); returns the int64 seeds or None."""
+    multi = [k for k, v in controls.items() if isinstance(v, torch.Tensor) and v.numel() > 1]
+    if not per_item and (seed is not None or multi):
+        what = ", ".join((["seed"] if seed is not None else []) + [f"a tensor {k} of several values" for k in multi])
+        raise ValueError(f"{what}: per-item batches only (per_item=True / lengths=)")
+    if seed is not None and eps is not None:
+        raise ValueError("seed= and eps= are exclusive: the seed generates the noise eps would give")
+    for k, v in controls.items():
+        if isinstance(v, torch.Tensor) and v.numel() > 1 and not _per_item_control(v, B, device):
+            raise ValueError(f"{k} must be a float, a one-element tensor or a floating tensor of shape ({B},) on "
+                             f"{device}, got {v.dtype} {tuple(v.shape)} on {v.device}")
+    return None if seed is None else _seeds_tensor(seed, B, device)
 
 
 def _check_eps(eps, B: int, C: int, T: int, device):
@@ -738,14 +801,15 @@ class HierSpeechSynthesizer(nn.Module):
         self.emb_g = StyleEncoder(in_dim=80, hidden_dim=256, out_dim=gin_channels)
 
     @torch.no_grad()
-    def infer(self, x_mel, w2v, length, f0, *, per_item=False, eps=None):
-        """``per_item``: see ``voice_conversion_noise_control``; x_mel [B, 80, T] shares ``length`` with w2v, and ``eps``
-        is the draw inside ``enc_p_l`` (:201).  Returns (waveform, pitch prediction) as the reference does."""
+    def infer(self, x_mel, w2v, length, f0, *, per_item=False, eps=None, seed=None):
+        """``per_item``: see ``voice_conversion_noise_control``; x_mel [B, 80, T] shares ``length`` with w2v, and ``eps`` /
+        ``seed`` give the draw inside ``enc_p_l`` (:201).  Returns (waveform, pitch prediction) as the reference does."""
         if per_item:
-            vl, _ = self._per_item_args(w2v, length, f0, x_mel, None, w2v.shape[0], eps)
+            vl, _, seeds = self._per_item_args(w2v, length, f0, x_mel, None, w2v.shape[0], eps, seed)
             g = self.emb_g(_as_input(x_mel), lengths=vl).unsqueeze(-1)
-            return self._convert(w2v, vl, f0, g, eps, 1.0, need_pred=True)
+            return self._convert(w2v, vl, f0, g, eps, 1.0, need_pred=True, seeds=seeds)
         _no_eps(eps)
+        _per_item_noise_args(False, 0, None, None, seed)
         x_mask = torch.unsqueeze(sequence_mask(length, x_mel.size(2)), 1).to(x_mel.dtype)
         g = self.emb_g(x_mel, x_mask).unsqueeze(-1)
         z, _, _ = self.enc_p_l(w2v, f0, x_mask, g=g)
@@ -755,7 +819,7 @@ class HierSpeechSynthesizer(nn.Module):
 
     @torch.no_grad()
     def voice_conversion_noise_control(self, src, src_length, trg_mel, trg_length, f0, noise_scale=0.333, uncond=False,
-                                       denoise_ratio=0, *, per_item=False, eps=None):
+                                       denoise_ratio=0, *, per_item=False, eps=None, seed=None):
         """``per_item=True``: B utterances of different lengths padded into one batch, each computed exactly as this
         method (``per_item=False``) computes it alone -- batch 1, unpadded, its own prompts, the same noise -- bit for bit.
 
@@ -765,19 +829,34 @@ class HierSpeechSynthesizer(nn.Module):
           reference's [2, 80, Tm] layout); ``trg_length`` [2B].  Item b uses (1 - r) g[b] + r g[B + b].  (Equality with
           the item's own call holds when its two prompts have the same length: the own call pads them to each other.)
         * ``eps``: fp32 CUDA [B, 192, T], the noise multiplying exp(logs_p) (the reference's second draw, :687); item b
-          uses eps[b, :, :len[b]].  With ``eps=None`` one ``randn`` of the padded shape is drawn: capturable, but then an
-          item's noise depends on the batch it is in.
+          uses eps[b, :, :len[b]].  With ``eps=None`` and ``seed=None`` one ``randn`` of the padded shape is drawn:
+          capturable, but then an item's noise depends on the batch it is in.
+        * ``seed`` (instead of ``eps``): int64 CUDA tensor [B] or host sequence of 64-bit seeds.  Item b's noise is
+          generated from seed[b] on the device, inside the sampling launch, and equals
+          ``eps = ops.seeded_normal(seed[b:b+1], 192, len[b])`` of its own call: same request, same seed, same audio, in
+          any batch.  This is the project's own generator (Philox4x32-10), not torch's ``randn`` stream.
+        * ``noise_scale`` and ``denoise_ratio`` may be floating CUDA tensors [B], one value per item: item b equals its
+          own call with ``float(noise_scale[b])`` and ``float(denoise_ratio[b])`` (noise_scale rounded to fp32 once,
+          1 - r evaluated in float64 and then rounded, as the Python-float call does).  As device tensors they are
+          inputs of a captured graph, so one graph serves every mix of seeds and controls.
         * Nothing past an item's length is read (any finite padding gives the same result); the waveform is
           [B, 1, 320 T] with item b's samples past 320 len[b] exactly 0."""
         if uncond:
             raise NotImplementedError("classifier-free guidance branch (cfg=True models) is not on this path")
         if per_item:
             B = src.shape[0]
-            vl, tl = self._per_item_args(src, src_length, f0, trg_mel, trg_length, 2 * B, eps)
+            vl, tl, seeds = self._per_item_args(src, src_length, f0, trg_mel, trg_length, 2 * B, eps, seed,
+                                                noise_scale=noise_scale, denoise_ratio=denoise_ratio)
             g = self.emb_g(_as_input(trg_mel), lengths=tl).unsqueeze(-1)
-            g = ((1 - denoise_ratio) * g[:B] + denoise_ratio * g[B:]).contiguous()
-            return self._convert(src, vl, f0, g, eps, noise_scale)[0]
+            if _per_item_control(denoise_ratio, B, src.device):
+                # the scalar call's arithmetic per item: (1 - r) in float64, both weights rounded to fp32, fp32 products
+                r = denoise_ratio.detach().to(torch.float64).view(B, 1, 1)
+                g = ((1 - r).float() * g[:B] + r.float() * g[B:]).contiguous()
+            else:
+                g = ((1 - denoise_ratio) * g[:B] + denoise_ratio * g[B:]).contiguous()
+            return self._convert(src, vl, f0, g, eps, noise_scale, seeds=seeds)[0]
         _no_eps(eps)
+        _per_item_noise_args(False, 0, None, None, seed, noise_scale=noise_scale, denoise_ratio=denoise_ratio)
         trg_mask = torch.unsqueeze(sequence_mask(trg_length, trg_mel.size(2)), 1).to(trg_mel.dtype)
         g = self.emb_g(trg_mel, trg_mask).unsqueeze(-1)
         g_org, g_denoise = g[:1, :, :], g[1:, :, :]
@@ -794,15 +873,17 @@ class HierSpeechSynthesizer(nn.Module):
 
     @torch.no_grad()
     def voice_conversion(self, src, src_length, trg_mel, trg_length, f0, noise_scale=0.333, uncond=False, *,
-                         per_item=False, eps=None):
+                         per_item=False, eps=None, seed=None):
         """``per_item``: see ``voice_conversion_noise_control``, with one prompt per item: ``trg_mel`` [B, 80, Tm]."""
         if uncond:
             raise NotImplementedError("classifier-free guidance branch (cfg=True models) is not on this path")
         if per_item:
-            vl, tl = self._per_item_args(src, src_length, f0, trg_mel, trg_length, src.shape[0], eps)
+            vl, tl, seeds = self._per_item_args(src, src_length, f0, trg_mel, trg_length, src.shape[0], eps, seed,
+                                                noise_scale=noise_scale)
             g = self.emb_g(_as_input(trg_mel), lengths=tl).unsqueeze(-1)
-            return self._convert(src, vl, f0, g, eps, noise_scale)[0]
+            return self._convert(src, vl, f0, g, eps, noise_scale, seeds=seeds)[0]
         _no_eps(eps)
+        _per_item_noise_args(False, 0, None, None, seed, noise_scale=noise_scale)
         trg_mask = torch.unsqueeze(sequence_mask(trg_length, trg_mel.size(2)), 1).to(trg_mel.dtype)
         g = self.emb_g(trg_mel, trg_mask).unsqueeze(-1)
         y_mask = torch.unsqueeze(sequence_mask(src_length, src.size(2)), 1).to(trg_mel.dtype)
@@ -816,9 +897,10 @@ class HierSpeechSynthesizer(nn.Module):
         return vocode(self.sn, self.dec, z, g)[0]
 
     # ---- per-item batches
-    def _per_item_args(self, src, src_length, f0, mel, mel_length, rows: int, eps):
+    def _per_item_args(self, src, src_length, f0, mel, mel_length, rows: int, eps, seed, **controls):
         """Checks every argument of a per-item call before anything runs; returns the int32 lengths of the source and
-        of the prompts (``mel_length=None``: the prompts share the source's lengths and T, as ``infer``'s x_mel)."""
+        of the prompts (``mel_length=None``: the prompts share the source's lengths and T, as ``infer``'s x_mel) and the
+        int64 seeds (or None)."""
         if src.dim() != 3:
             raise ValueError(f"the source must be [B, C, T], got {tuple(src.shape)}")
         B, _, T = src.shape
@@ -832,16 +914,17 @@ class HierSpeechSynthesizer(nn.Module):
             raise ValueError(f"f0 must be [{B}, 1, {4 * T}], got {tuple(f0.shape)}")
         if eps is not None:
             _check_eps(eps, B, self.enc_p_l.out_channels, T, src.device)
-        return vl, tl
+        seeds = _per_item_noise_args(True, B, src.device, eps, seed, **controls)
+        return vl, tl, seeds
 
-    def _convert(self, src, src_length, f0, g, eps, noise_scale: float, need_pred: bool = False):
+    def _convert(self, src, src_length, f0, g, eps, noise_scale, need_pred: bool = False, seeds=None):
         """enc_p_l -> flow_l -> flow -> vocoder of a per-item batch (g [B, gin, 1] per item); returns vocode's pair."""
         src, f0 = _as_input(src), _as_input(f0)
         B, _, T = src.shape
         vl = _lengths_tensor(src_length, B, T, src.device)
-        if eps is None:
+        if eps is None and seeds is None:
             eps = torch.randn(B, self.enc_p_l.out_channels, T, dtype=torch.float32, device=src.device)
-        z, _, _ = self.enc_p_l(src, f0, None, g=g, eps=eps, noise_scale=noise_scale, lengths=vl)
+        z, _, _ = self.enc_p_l(src, f0, None, g=g, eps=eps, noise_scale=noise_scale, lengths=vl, seed=seeds)
         z = self.flow_l(z, None, g=g, reverse=True, lengths=vl)
         z = self.flow(z, None, g=g, reverse=True, lengths=vl)
         return vocode(self.sn, self.dec, z, g, need_pred, lengths=vl)

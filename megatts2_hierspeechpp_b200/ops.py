@@ -609,6 +609,23 @@ def peak_norm_pcm16(x: torch.Tensor, s1: float = 32767.0, s2: float = 0.999, per
     return out, (peaks if per_row else peaks[:1])
 
 
+def peak_norm_pcm16_rows(x: torch.Tensor, s2: torch.Tensor, s1: float = 32767.0):
+    """``peak_norm_pcm16(per_row=True)`` with one ``s2`` per row: row b equals ``peak_norm_pcm16(x[b], s1, s2[b])``.
+    s2: fp32 CUDA [rows].  Returns (pcm int16, peaks fp32 [rows])."""
+    _req(x, "x"); _req(s2, "s2", ndim=1)
+    if x.dim() < 1:
+        raise ValueError("x must have at least one dim")
+    L = x.shape[-1]
+    rows = x.numel() // L if L else 0
+    if s2.numel() != rows or s2.device != x.device:
+        raise ValueError(f"s2: expected {rows} values on {x.device}, got {s2.numel()} on {s2.device}")
+    out = torch.empty(x.shape, dtype=torch.int16, device=x.device)
+    peaks = torch.zeros(max(rows, 1), dtype=torch.float32, device=x.device)
+    _lib.check(_lib.load().hsv_peak_norm_pcm16_rows(_p(x), _p(out), _p(peaks), rows, L, float(s1), _p(s2), _stream()),
+               "hsv_peak_norm_pcm16_rows")
+    return out, peaks
+
+
 # ----------------------------------------------------------------------------------------------
 # frame-rate operators of the step before the vocoder (csrc/frame_ops.cu)
 # ----------------------------------------------------------------------------------------------
@@ -796,6 +813,60 @@ def masked_mean(x: torch.Tensor, mask: Optional[torch.Tensor], valid_len: Option
                    "hsv_masked_mean_ragged")
     else:
         _lib.check(lib.hsv_masked_mean(_p(x), _p(mask), _p(out), B, C, L, _stream()), "hsv_masked_mean")
+    return out
+
+
+def _req_seeds(seeds: torch.Tensor, B: Optional[int] = None):
+    _req(seeds, "seeds", torch.int64, 1)
+    if B is not None and seeds.numel() != B:
+        raise ValueError(f"seeds: expected {B} elements, got {seeds.numel()}")
+
+
+def seeded_normal(seeds: torch.Tensor, C: int, T: int, valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """fp32 [B, C, T] standard normals; the value at (b, c, t) depends on (seeds[b], c, t) only (csrc/noise.cu: Philox4x32-10
+    + Box-Muller, the project's own stream, not torch's ``randn``).  seeds: int64 CUDA [B].  ``valid_len`` (int32 [B]):
+    0 at t >= valid_len[b]."""
+    _req_seeds(seeds)
+    B = seeds.numel()
+    _req_len(valid_len, B, seeds.device)
+    out = torch.empty(B, C, T, dtype=torch.float32, device=seeds.device)
+    _lib.check(_lib.load().hsv_seeded_normal(_p(seeds), _p(out), B, int(C), int(T), _p(valid_len), _stream()),
+               "hsv_seeded_normal")
+    return out
+
+
+def sample_ragged(stats: torch.Tensor, s, valid_len: Optional[torch.Tensor] = None, eps: Optional[torch.Tensor] = None,
+                  seeds: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """z = (m + n * exp(logs) * s[b]) for stats = [B, 2C, T] (m | logs), the same bits as ``frame_op(OP_SAMPLE)`` fed with
+    the same noise n; 0 at t >= valid_len[b] (int32 [B]), where nothing is read.  n: ``eps`` [B, C, T] or, from
+    ``seeds`` (int64 [B]), ``seeded_normal(seeds, C, T)`` generated in registers (no noise tensor).  ``s``: a float or a
+    fp32 CUDA tensor [B]."""
+    _req(stats, "stats", ndim=3)
+    B, C2, T = stats.shape
+    C = C2 // 2
+    if C2 % 2:
+        raise ValueError(f"stats must have 2C channels, got {C2}")
+    if (eps is None) == (seeds is None):
+        raise ValueError("sample_ragged: pass exactly one of eps and seeds")
+    if eps is not None:
+        _req(eps, "eps", ndim=3)
+        if tuple(eps.shape) != (B, C, T):
+            raise ValueError(f"eps must have shape {(B, C, T)}, got {tuple(eps.shape)}")
+    else:
+        _req_seeds(seeds, B)
+    _req_len(valid_len, B, stats.device)
+    svec = None
+    if isinstance(s, torch.Tensor):
+        _req(s, "s", ndim=1)
+        if s.numel() != B:
+            raise ValueError(f"s: expected {B} elements, got {s.numel()}")
+        svec, s = s, 0.0
+    for t, n in ((eps, "eps"), (seeds, "seeds"), (svec, "s")):
+        if t is not None and t.device != stats.device:
+            raise ValueError(f"{n}: on {t.device}, stats is on {stats.device}")
+    out = torch.empty(B, C, T, dtype=torch.float32, device=stats.device)
+    _lib.check(_lib.load().hsv_sample_ragged(_p(stats), _p(eps), _p(seeds), _p(svec), float(s), _p(valid_len), _p(out), B,
+                                             C, T, _stream()), "hsv_sample_ragged")
     return out
 
 

@@ -12,14 +12,28 @@ from typing import Callable, Dict, List, Sequence, Tuple
 import torch
 
 
-def to_pcm16(audio: torch.Tensor, scale_norm: str = "max", prompt_audio_max: float = 1.0, order: str = "plm",
+def to_pcm16(audio: torch.Tensor, scale_norm: str = "max", prompt_audio_max=1.0, order: str = "plm",
              per_utterance: bool = False) -> torch.Tensor:
     """int16 PCM of a generated waveform, on the device (the step after the path, SURVEY.md §8f3).
 
     ``order="plm"``: ``audio / |audio|.max() * 32767.0 * s`` with s = 0.999, or ``prompt_audio_max`` when
     ``scale_norm == "prompt"`` (inference_plm.py:183-188); ``order="speechsr"``: ``... * 0.999 * 32767.0``
-    (inference_speechsr.py:39-41).  Bit-exact with the reference's fp32 arithmetic + ``astype('int16')``."""
+    (inference_speechsr.py:39-41).  Bit-exact with the reference's fp32 arithmetic + ``astype('int16')``.
+    With ``per_utterance=True`` and ``scale_norm="prompt"``, ``prompt_audio_max`` may be a floating CUDA tensor of one
+    value per row (each utterance's own prompt peak): row b then equals ``to_pcm16(row b, "prompt",
+    float(prompt_audio_max[b]))``."""
     from . import ops
+    if isinstance(prompt_audio_max, torch.Tensor):
+        if order != "plm" or scale_norm != "prompt" or not per_utterance:
+            raise ValueError("a per-row prompt_audio_max needs order='plm', scale_norm='prompt', per_utterance=True")
+        if not prompt_audio_max.is_floating_point() or prompt_audio_max.dim() != 1:
+            raise ValueError("prompt_audio_max must be a 1-D floating tensor, one value per row")
+        rows = audio.numel() // audio.shape[-1] if audio.dim() and audio.shape[-1] else 0
+        if prompt_audio_max.numel() != rows:
+            raise ValueError(f"prompt_audio_max has {prompt_audio_max.numel()} values for {rows} rows")
+        # fp32 rounding, as ctypes.c_float rounds the scalar
+        s2 = prompt_audio_max.detach().to(torch.float32).contiguous()
+        return ops.peak_norm_pcm16_rows(audio.detach().contiguous(), s2)[0]
     if order == "plm":
         s1, s2 = 32767.0, (float(prompt_audio_max) if scale_norm == "prompt" else 0.999)
     elif order == "speechsr":
