@@ -61,11 +61,17 @@ int64_t hsv_blk16_rows(int64_t L);
 /* Test hook, read-only: which kernel variant the most recent host-side launch decision of a family chose.
  * Process-global (like the bring-up switches); it never changes what is launched.  Copies min(n, count) ints to
  * out and returns count (negative on a bad argument).
- *   family 0, tcgen05 conv (count 14): kind (0 one-tile, 1 persistent, 2 fused activation, 3 operand-writing
+ *   family 0, tcgen05 conv (count 15): kind (0 one-tile, 1 persistent, 2 fused activation, 3 operand-writing
  *             epilogue), msub, warps per CTA, vec_epi (float4 epilogue), nphase, n_tile, stages, G (weight blocks
- *             per ring stage), resident, nabuf (persistent only, else 0), grid x, y, z, launches so far
+ *             per ring stage), resident, nabuf (persistent only, else 0), grid x, y, z, blk_mode (kind 3: the
+ *             hsv_conv1d_umma_blk16 mode 0-3, 4 = hsv_conv1d_umma_wn_tail; else 0), launches so far
  *   family 1, Activation1d (count 4): run length R (0 when the tensor-core kernel ran), act1d_mma ran, out_mode,
- *             launches so far */
+ *             launches so far
+ *   family 2, attention (count 13): kernel (0 tensor-core, 1 fp32 CUDA-core), D, out_mode, lens given, valid_len
+ *             given, prescale, kv16 (K / V tiles copied in 16-byte chunks: Tk % 4 == 0, 16-byte aligned k and v,
+ *             batch strides % 4 == 0), q16 (tensor-core kernel: Q tiles copied in 16-byte chunks: Tq % 4 == 0,
+ *             16-byte aligned q, q batch stride % 4 == 0; 0 for the fp32 kernel), key tiles, grid x, y, z, launches
+ *             so far */
 int hsv_last_launch_config(int family, int *out, int n);
 
 /* ---- Activation1d(SnakeBeta): alias_free_torch/act.py:23-27 =

@@ -42,13 +42,23 @@ extern "C" int hsv_device_supported(void) {
 extern "C" int64_t hsv_blk16_rows(int64_t L) { return hsv::blk16_rows(L); }
 
 namespace hsv {
-int g_last_launch[2][16] = {};
+int g_last_launch[3][16] = {};
+
+void note_mha_launch(int kernel, int D, int out_mode, int has_lens, int has_valid_len, int prescale, int kv16, int q16,
+                     int key_tiles, dim3 grid) {
+  const int v[LAST_MHA_N - 1] = {kernel, D, out_mode, has_lens, has_valid_len, prescale ? 1 : 0, kv16, q16, key_tiles,
+                                 (int)grid.x, (int)grid.y, (int)grid.z};
+  int *last = g_last_launch[2];
+  for (int i = 0; i < LAST_MHA_N - 1; ++i) last[i] = v[i];
+  ++last[LAST_MHA_N - 1];
+}
 }
 
 extern "C" int hsv_last_launch_config(int family, int *out, int n) {
-  HSV_REQUIRE(family == 0 || family == 1, "last_launch_config: family must be 0 (conv) or 1 (activation), got %d", family);
+  HSV_REQUIRE(family >= 0 && family <= 2,
+              "last_launch_config: family must be 0 (conv), 1 (activation) or 2 (attention), got %d", family);
   HSV_REQUIRE(n >= 0 && (out || n == 0), "last_launch_config: null output");
-  const int have = family == 0 ? hsv::LAST_CONV_N : hsv::LAST_ACT_N;
+  const int have = family == 0 ? hsv::LAST_CONV_N : (family == 1 ? hsv::LAST_ACT_N : hsv::LAST_MHA_N);
   for (int i = 0; i < n && i < have; ++i) out[i] = hsv::g_last_launch[family][i];
   return have;
 }

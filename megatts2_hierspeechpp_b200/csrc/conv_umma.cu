@@ -1060,12 +1060,13 @@ int g_persist = 1;  // persistent variant for eligible launches (hsv_set_umma_de
 constexpr int PERSIST_EPW = 4;
 
 // hsv_last_launch_config, family 0: kind (0 one-tile, 1 persistent, 2 fused activation, 3 operand-writing epilogue),
-// msub, warps per CTA, vec_epi, nphase, n_tile, stages, G, resident, nabuf, grid x / y / z, running launch count
+// msub, warps per CTA, vec_epi, nphase, n_tile, stages, G, resident, nabuf, grid x / y / z, blk_mode (kind 3 only, else
+// 0), running launch count
 void note_launch(int kind, const Params &p, int warps, dim3 grid) {
   const bool persist = kind == 1;  // resident / nabuf are only set (and read) by the persistent variant
   const int v[hsv::LAST_CONV_N - 1] = {kind, p.msub, warps, p.vec_epi, p.tt.nphase, p.n_tile, p.stages, p.G,
                                        persist ? p.resident : 0, persist ? p.nabuf : 0, (int)grid.x, (int)grid.y,
-                                       (int)grid.z};
+                                       (int)grid.z, kind == 3 ? p.blk_mode : 0};
   int *last = hsv::g_last_launch[0];
   for (int i = 0; i < hsv::LAST_CONV_N - 1; ++i) last[i] = v[i];
   ++last[hsv::LAST_CONV_N - 1];

@@ -446,6 +446,7 @@ int mha_launch(const float *q, const float *k, const float *v, float *out, const
   auto al = [](const void *p_) { return (reinterpret_cast<uintptr_t>(p_) & 15) == 0; };
   const int fast = (Tk % 4 == 0) && al(k) && al(v) && (kbs % 4 == 0) && (vbs % 4 == 0);
   dim3 grid((unsigned)((Tq + QT - 1) / QT), (unsigned)heads, (unsigned)B);
+  hsv::note_mha_launch(1, D, 0, lens != nullptr, 0, prescale, fast, 0, (Tk + MHA_K - 1) / MHA_K, grid);
   mha_kernel<D, RW><<<grid, MHA_THREADS, smem, st>>>(q, k, v, out, lens, Tq, Tk, qbs, kbs, vbs, heads, scale, prescale, fast);
   return hsv::check_launch("mha");
 }

@@ -424,6 +424,9 @@ int launch(const float *q, const float *k, const float *v, void *out, const int 
   auto al = [](const void *p_) { return (reinterpret_cast<uintptr_t>(p_) & 15) == 0; };
   const int fast = (Tk % 4 == 0) && al(k) && al(v) && (kbs % 4 == 0) && (vbs % 4 == 0);
   dim3 grid((unsigned)((Tq + QT - 1) / QT), (unsigned)(heads * NSPLIT), (unsigned)B);   // cluster dims (1, NSPLIT, 1)
+  hsv::note_mha_launch(0, D, BLK, lens != nullptr, VLEN, prescale, fast,
+                       (Tq % 4 == 0) && al(q) && (qbs % 4 == 0),   // the Q tile's 16-byte copies (full tiles only)
+                       (Tk + KT - 1) / KT, grid);
   mha_mma_kernel<D, BLK, VLEN><<<grid, 32 * NWARP, smem, st>>>(q, k, v, out, lens, vlen, Tq, Tk, qbs, kbs, vbs, heads,
                                                              scale, prescale, fast);
   return hsv::check_launch("mha_mma");

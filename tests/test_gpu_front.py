@@ -50,6 +50,26 @@ def test_pack_act_modes(hsv):
     assert _rel(ops.unpack_blk16(buf, C, T), xm * torch.tanh(F.softplus(xm)) * mask.unsqueeze(1)) <= 1e-3
     ops.pack_blk16_act(x, buf, C, ops.PACK_MASK)
     assert _rel(ops.unpack_blk16(buf, C, T), x[:, :C]) <= 1e-3
+    # arguments across softplus's threshold of 20 and saturated gate arguments, against fp64: within one fp16 spacing
+    # of the value (2^-24 below the normal range) plus a few fp32 roundings of it
+    xe = _edge_args(B, 2 * C, T, g).to(DEV)
+    bz = torch.zeros(B, 2 * C, device=DEV)
+    x64 = xe.double()
+    for mode, ref in ((ops.PACK_GATE, torch.tanh(x64[:, :C]) * torch.sigmoid(x64[:, C:])),
+                      (ops.PACK_MISH, x64[:, :C] * torch.tanh(F.softplus(x64[:, :C])))):
+        ops.pack_blk16_act(xe, buf, C, mode, bcast=bz if mode == ops.PACK_GATE else None)
+        got = ops.unpack_blk16(buf, C, T).double()
+        ulp = torch.exp2(torch.floor(torch.log2(ref.abs().clamp_min(2.0 ** -14))) - 10)
+        assert bool(((got - ref).abs() <= ulp + 1e-6 * ref.abs()).all()), (mode, float((got - ref).abs().max()))
+
+
+def _edge_args(B, C, T, g):
+    """Arguments in [-100, 100] with the exact values around softplus's threshold of 20 and deep saturation."""
+    x = torch.rand(B, C, T, generator=g) * 200 - 100
+    edges = torch.tensor([-100., -88., -40., -20.5, -20., -19.5, -1., 0., 1., 19.5, 19.999, 20., 20.001, 20.5, 40., 88.])
+    x[..., :len(edges)] = edges
+    x[:, ::2, len(edges):2 * len(edges)] = edges.flip(0)
+    return x
 
 
 @pytest.mark.parametrize("C", [192, 256])
@@ -122,6 +142,14 @@ def test_frame_ops(hsv):
     assert torch.allclose(out, (x + rs[:, :C] * torch.sigmoid(rs[:, C:])) * mk, atol=1e-6)
     ops.frame_op(ops.OP_MISH, x, None, None, mask, out, None, B, C, T)
     assert torch.allclose(out, x * torch.tanh(F.softplus(x)) * mk, atol=1e-6)
+    xe = _edge_args(B, C, T, g).to(DEV)                 # across softplus's threshold of 20, against fp64
+    ops.frame_op(ops.OP_MISH, xe, None, None, None, out, None, B, C, T)
+    ref = xe.double() * torch.tanh(F.softplus(xe.double()))
+    assert bool(((out.double() - ref).abs() <= 2e-6 * ref.abs() + 1e-37).all())       # + the fp32 subnormal range
+    ys = torch.cat([_edge_args(B, C, T, g), _edge_args(B, C, T, g).flip(1)], 1).to(DEV)   # saturated sigmoid
+    ops.frame_op(ops.OP_GLU_RES, x, ys, None, None, out, None, B, C, T)
+    ref = x.double() + ys[:, :C].double() * torch.sigmoid(ys[:, C:].double())
+    assert bool(((out.double() - ref).abs() <= 1e-6 * (x.double().abs() + ys[:, :C].double().abs())).all())
     ops.frame_op(ops.OP_FLIP, x, None, None, None, out, None, B, C, T)
     assert torch.equal(out, torch.flip(x, [1]))
     ops.frame_op(ops.OP_ADD, x, y, None, None, out, None, B, C, T)

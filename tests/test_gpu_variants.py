@@ -15,6 +15,8 @@ simplest variants, so every case here forces (a, c) or naturally selects (b) a v
 
 (d) is a census: the variant of every conv / activation launch of the benchmark workloads must be in ``VERIFIED``, the
 set of variants the cases above check.  A policy change that ships a new variant fails it until a case covers it.
+The operand-writing epilogue's variants (``operand-out:{mode}:n{n_tile}``) are checked against fp64 by
+test_gpu_front_variants.py (c), which declares them in ``OPERAND_KEYS``.
 """
 import argparse
 import os
@@ -27,6 +29,7 @@ import torch.nn.functional as F
 
 from oracle import closed_form as CF
 from oracle import functional as OF
+from test_gpu_front_variants import OPERAND_KEYS, operand_key
 
 DEV = "cuda:0"
 SLOT = 11          # blk16 workspace slot of this file (modules use 0..7 and 15, other tests 7..10)
@@ -53,7 +56,7 @@ def conv_key(c):
     if kind == 2:
         return "fused-act"
     if kind == 3:
-        return "operand-out"
+        return operand_key(c["blk_mode"], c["n_tile"])
     if c["nphase"] > 1:
         return f"convT:m{c['msub']}:w{c['warps']}:n{c['n_tile']}"
     return f"conv:m{c['msub']}:w{c['warps']}:{'vec' if c['vec_epi'] else 'scalar'}:n{c['n_tile']}"
@@ -158,12 +161,12 @@ CONV_NATURAL = [
 ]
 
 # ----------------------------------------------------------------------------------------------
-# (d) the variants (a)-(c) verify.  "operand-out" (hsv_conv1d_umma_blk16 / _wn_tail) and "fused-act"
-# (hsv_act_conv1d_umma) are checked by test_gpu_kernels.py::test_conv1d_umma_operand_writing_epilogue and
-# ::test_act_conv_fused_equals_unfused; they are listed here on the strength of those tests.
+# (d) the variants (a)-(c) verify, and the operand-writing epilogue's (test_gpu_front_variants.py (c)).  "fused-act"
+# (hsv_act_conv1d_umma) is checked by test_gpu_kernels.py::test_act_conv_fused_equals_unfused; it is listed here on the
+# strength of that test.
 # ----------------------------------------------------------------------------------------------
-VERIFIED = {
-    "operand-out", "fused-act",
+VERIFIED = set(OPERAND_KEYS) | {
+    "fused-act",
     "persist:ring:a2", "persist:ring:a1", "persist:resident:a2",
     "conv:m1:w4:vec:n16", "conv:m1:w4:scalar:n16", "conv:m2:w4:vec:n16", "conv:m2:w4:scalar:n16",
     "conv:m4:w4:vec:n16", "conv:m4:w4:scalar:n16",
@@ -186,7 +189,7 @@ VERIFIED = {
 
 def _declared_keys():
     """The variant keys the cases of (a)-(c) assert (each case checks its key through the hook when it runs)."""
-    keys = {"operand-out", "fused-act"}
+    keys = {"fused-act"} | set(OPERAND_KEYS)
     keys |= {_conv_key_expected(c[0], c[1], c[4], c[6], c[7], c[8]) for c in CONV_MATRIX}
     keys |= {_conv_key_expected(c[0], c[1], c[4], c[6], c[7], None, True) for c in CONVT_MATRIX}
     keys |= {c[-1] for c in PERSIST_MATRIX}
@@ -201,13 +204,15 @@ def test_verified_set_is_covered_by_the_cases():
     assert not missing, sorted(missing)
 
 
-def test_last_launch_config_hook():
-    """The hook reports the documented field counts and rejects an unknown family (host-only, no GPU)."""
+def test_last_launch_config_hook_three_families():
+    """The hook reports the documented fields of its three families (conv, activation, attention) and rejects an
+    unknown family (host-only, no GPU)."""
     from megatts2_hierspeechpp_b200 import _lib, build, ops
     build.build()
-    assert set(ops.last_launch_config(ops.LAUNCH_CONV)) >= {"kind", "msub", "warps", "vec_epi", "launches"}
+    assert set(ops.last_launch_config(ops.LAUNCH_CONV)) >= {"kind", "msub", "warps", "vec_epi", "blk_mode", "launches"}
     assert set(ops.last_launch_config(ops.LAUNCH_ACT)) == {"R", "mma", "out_mode", "launches"}
-    assert _lib.load().hsv_last_launch_config(2, None, 0) < 0
+    assert set(ops.last_launch_config(ops.LAUNCH_MHA)) >= {"kernel", "D", "out_mode", "kv16", "q16", "launches"}
+    assert _lib.load().hsv_last_launch_config(3, None, 0) < 0
 
 
 # ----------------------------------------------------------------------------------------------
