@@ -71,7 +71,11 @@ int64_t hsv_blk16_rows(int64_t L);
  *             given, prescale, kv16 (K / V tiles copied in 16-byte chunks: Tk % 4 == 0, 16-byte aligned k and v,
  *             batch strides % 4 == 0), q16 (tensor-core kernel: Q tiles copied in 16-byte chunks: Tq % 4 == 0,
  *             16-byte aligned q, q batch stride % 4 == 0; 0 for the fp32 kernel), key tiles, grid x, y, z, launches
- *             so far */
+ *             so far
+ *   family 3, CUDA-core conv (hsv_conv1d_direct[_ragged], hsv_conv_transpose1d_direct; count 7): kernel (0 vecdot,
+ *             1 rowdot, 2 thin_vec, 3 thin_smem, 4 thin, 5 tiled, 6 ConvTranspose direct), flags (HSV_CONV_*; for
+ *             the ConvTranspose HSV_CONV_ADD_OUT when `add` is given, else 0), valid_len given, grid x, y, z,
+ *             launches so far.  A call that launches nothing (B = 0, Lout <= 0 or Lin = 0) leaves it unchanged. */
 int hsv_last_launch_config(int family, int *out, int n);
 
 /* ---- Activation1d(SnakeBeta): alias_free_torch/act.py:23-27 =

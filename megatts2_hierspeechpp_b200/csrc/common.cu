@@ -42,7 +42,7 @@ extern "C" int hsv_device_supported(void) {
 extern "C" int64_t hsv_blk16_rows(int64_t L) { return hsv::blk16_rows(L); }
 
 namespace hsv {
-int g_last_launch[3][16] = {};
+int g_last_launch[4][16] = {};
 
 void note_mha_launch(int kernel, int D, int out_mode, int has_lens, int has_valid_len, int prescale, int kv16, int q16,
                      int key_tiles, dim3 grid) {
@@ -52,13 +52,22 @@ void note_mha_launch(int kernel, int D, int out_mode, int has_lens, int has_vali
   for (int i = 0; i < LAST_MHA_N - 1; ++i) last[i] = v[i];
   ++last[LAST_MHA_N - 1];
 }
+
+void note_direct_launch(int kernel, int flags, int has_valid_len, dim3 grid) {
+  const int v[LAST_DIRECT_N - 1] = {kernel, flags, has_valid_len, (int)grid.x, (int)grid.y, (int)grid.z};
+  int *last = g_last_launch[3];
+  for (int i = 0; i < LAST_DIRECT_N - 1; ++i) last[i] = v[i];
+  ++last[LAST_DIRECT_N - 1];
+}
 }
 
 extern "C" int hsv_last_launch_config(int family, int *out, int n) {
-  HSV_REQUIRE(family >= 0 && family <= 2,
-              "last_launch_config: family must be 0 (conv), 1 (activation) or 2 (attention), got %d", family);
+  HSV_REQUIRE(family >= 0 && family <= 3,
+              "last_launch_config: family must be 0 (conv), 1 (activation), 2 (attention) or 3 (CUDA-core conv), got %d",
+              family);
   HSV_REQUIRE(n >= 0 && (out || n == 0), "last_launch_config: null output");
-  const int have = family == 0 ? hsv::LAST_CONV_N : (family == 1 ? hsv::LAST_ACT_N : hsv::LAST_MHA_N);
+  const int have_n[4] = {hsv::LAST_CONV_N, hsv::LAST_ACT_N, hsv::LAST_MHA_N, hsv::LAST_DIRECT_N};
+  const int have = have_n[family];
   for (int i = 0; i < n && i < have; ++i) out[i] = hsv::g_last_launch[family][i];
   return have;
 }

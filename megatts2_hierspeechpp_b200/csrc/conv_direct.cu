@@ -826,10 +826,12 @@ extern "C" int hsv_conv1d_direct_ragged(const float *x, const float *w, const fl
   if (k == 1 && Lin == 1 && pad == 0 && (Cin & 3) == 0 && ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(w)) & 15) == 0) {
     const int64_t nwarps = (int64_t)B * Cout;
     HSV_REQUIRE(nwarps * 32 / 256 + 1 < (1ll << 31), "conv1d_direct: grid too large");
+    hsv::note_direct_launch(0, flags, 0, dim3((unsigned)((nwarps * 32 + 255) / 256)));
     conv1d_vecdot_kernel<<<(unsigned)((nwarps * 32 + 255) / 256), 256, 0, st>>>(x, w, bias, out, B, Cin, Cout, flags);
   } else if (Lout <= 8 && !valid_len) {   // (with valid_len, short items take the warp reduction inside the thin kernels)
     const int64_t nwarps = (int64_t)B * Cout * Lout;
     HSV_REQUIRE(nwarps * 32 / 256 + 1 < (1ll << 31), "conv1d_direct: grid too large");
+    hsv::note_direct_launch(1, flags, 0, dim3((unsigned)((nwarps * 32 + 255) / 256)));
     conv1d_rowdot_kernel<<<(unsigned)((nwarps * 32 + 255) / 256), 256, 0, st>>>(x, w, bias, out, B, Cin, Cout, Lin,
                                                                                Lout, k, d, pad, flags);
   } else if (Cout <= 4 && d == 1 && k == 7) {
@@ -837,15 +839,18 @@ extern "C" int hsv_conv1d_direct_ragged(const float *x, const float *w, const fl
     dim3 grid((unsigned)((Lout + 511) / 512), (unsigned)B);
     const bool vec = pad == 3 && (Lin & 3) == 0 && Lout == Lin &&
                      ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
+    hsv::note_direct_launch(vec ? 2 : 3, flags, valid_len != nullptr, grid);
     if (vec) conv1d_thin_vec_kernel<<<grid, 128, 0, st>>>(x, w, bias, out, valid_len, Cin, Cout, Lin, Lout, flags);
     else conv1d_thin_smem_kernel<7><<<grid, 256, 0, st>>>(x, w, bias, out, valid_len, Cin, Cout, Lin, Lout, pad, flags);
   } else if (Cout <= 4) {
+    hsv::note_direct_launch(4, flags, 0, dim3((unsigned)grid_for((int64_t)B * Lout, 256)));
     conv1d_thin_kernel<<<grid_for((int64_t)B * Lout, 256), 256, 0, st>>>(x, w, bias, out, B, Cin, Cout, Lin,
                                                                         Lout, k, d, pad, flags);
   } else {
     constexpr int TCO = 32, TT = 64;
     HSV_REQUIRE(B <= 65535 && (Cout + TCO - 1) / TCO <= 65535, "conv1d_direct: grid too large");
     dim3 grid((unsigned)((Lout + TT - 1) / TT), (unsigned)((Cout + TCO - 1) / TCO), (unsigned)B);
+    hsv::note_direct_launch(5, flags, 0, grid);
     conv1d_tiled_kernel<TCO, TT><<<grid, (TCO / 4) * (TT / 4), 0, st>>>(x, w, bias, out, Cin, Cout, Lin, Lout, k,
                                                                        d, pad, flags);
   }
@@ -866,6 +871,7 @@ extern "C" int hsv_conv_transpose1d_direct(const float *x, const float *w, const
   const int nco = (Cout + TCO - 1) / TCO;
   HSV_REQUIRE(B <= 65535 && (int64_t)nco * u <= 65535, "conv_transpose1d: grid too large");
   dim3 grid((unsigned)((Lin + TT - 1) / TT), (unsigned)(nco * u), (unsigned)B);
+  hsv::note_direct_launch(6, add ? HSV_CONV_ADD_OUT : 0, 0, grid);   // flags: the add operand as ADD_OUT
   conv_transpose1d_kernel<TCO, TT><<<grid, (TCO / 4) * (TT / 4), 0, hsv::as_stream(stream)>>>(
       x, w, bias, add, out, Cin, Cout, Lin, k, u, nco);
   return hsv::check_launch("conv_transpose1d_direct");

@@ -75,13 +75,16 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 
 // What the most recent host-side launch decision of a kernel family chose (hsv_last_launch_config, common.cu):
 // [0] = the tcgen05 conv (conv_umma.cu), [1] = the fused activation (act1d.cu), [2] = attention (mha_mma.cu and the
-// fp32 kernel of frame_ops.cu).  Process-global bookkeeping, written just before the launch; it never changes what is
-// launched.
-constexpr int LAST_CONV_N = 15, LAST_ACT_N = 4, LAST_MHA_N = 13;
-extern int g_last_launch[3][16];
+// fp32 kernel of frame_ops.cu), [3] = the CUDA-core convs of conv_direct.cu.  Process-global bookkeeping, written just
+// before the launch; it never changes what is launched.
+constexpr int LAST_CONV_N = 15, LAST_ACT_N = 4, LAST_MHA_N = 13, LAST_DIRECT_N = 7;
+extern int g_last_launch[4][16];
 // family 2: kernel (0 tensor-core, 1 fp32 CUDA-core), D, out_mode, lens, valid_len, prescale, kv16 (16-byte K / V tile
 // copies), q16 (16-byte Q tile copies), key tiles, grid x / y / z; then the running launch count
 void note_mha_launch(int kernel, int D, int out_mode, int has_lens, int has_valid_len, int prescale, int kv16, int q16,
                      int key_tiles, dim3 grid);
+// family 3: kernel (0 vecdot, 1 rowdot, 2 thin_vec, 3 thin_smem, 4 thin, 5 tiled, 6 ConvTranspose direct), flags (the
+// ConvTranspose: HSV_CONV_ADD_OUT when it adds), valid_len given, grid x / y / z; then the running launch count
+void note_direct_launch(int kernel, int flags, int has_valid_len, dim3 grid);
 
 }  // namespace hsv

@@ -904,20 +904,24 @@ def set_umma_debug(flags: int):
     _lib.load().hsv_set_umma_debug(int(flags))
 
 
-LAUNCH_CONV, LAUNCH_ACT, LAUNCH_MHA = 0, 1, 2
+LAUNCH_CONV, LAUNCH_ACT, LAUNCH_MHA, LAUNCH_DIRECT = 0, 1, 2, 3
 _LAUNCH_FIELDS = {
     LAUNCH_CONV: ("kind", "msub", "warps", "vec_epi", "nphase", "n_tile", "stages", "G", "resident", "nabuf",
                   "grid_x", "grid_y", "grid_z", "blk_mode", "launches"),
     LAUNCH_ACT: ("R", "mma", "out_mode", "launches"),
     LAUNCH_MHA: ("kernel", "D", "out_mode", "has_lens", "has_valid_len", "prescale", "kv16", "q16", "key_tiles",
                  "grid_x", "grid_y", "grid_z", "launches"),
+    LAUNCH_DIRECT: ("kernel", "flags", "has_valid_len", "grid_x", "grid_y", "grid_z", "launches"),
 }
 CONV_ONE_TILE, CONV_PERSISTENT, CONV_FUSED_ACT, CONV_OPERAND_OUT = range(4)
+# LAUNCH_DIRECT kernels (csrc/conv_direct.cu)
+DIRECT_VECDOT, DIRECT_ROWDOT, DIRECT_THIN_VEC, DIRECT_THIN_SMEM, DIRECT_THIN, DIRECT_TILED, DIRECT_CONVT = range(7)
 
 
 def last_launch_config(family: int) -> Dict[str, int]:
     """Test hook: the variant the most recent host-side launch decision of a kernel family chose (``LAUNCH_CONV``: the
-    tcgen05 conv, ``LAUNCH_ACT``: the fused activation, ``LAUNCH_MHA``: attention), as a dict of the fields
+    tcgen05 conv, ``LAUNCH_ACT``: the fused activation, ``LAUNCH_MHA``: attention, ``LAUNCH_DIRECT``: the CUDA-core
+    conv / ConvTranspose of conv_direct.cu), as a dict of the fields
     ``hsv_last_launch_config`` fills.
     Read-only; needs no GPU."""
     names = _LAUNCH_FIELDS[family]

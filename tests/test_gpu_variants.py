@@ -204,15 +204,19 @@ def test_verified_set_is_covered_by_the_cases():
     assert not missing, sorted(missing)
 
 
-def test_last_launch_config_hook_three_families():
-    """The hook reports the documented fields of its three families (conv, activation, attention) and rejects an
-    unknown family (host-only, no GPU)."""
+def test_last_launch_config_hook_four_families():
+    """The hook reports the documented fields of its four families (conv, activation, attention, CUDA-core conv) and
+    rejects an unknown family (host-only, no GPU)."""
     from megatts2_hierspeechpp_b200 import _lib, build, ops
     build.build()
     assert set(ops.last_launch_config(ops.LAUNCH_CONV)) >= {"kind", "msub", "warps", "vec_epi", "blk_mode", "launches"}
     assert set(ops.last_launch_config(ops.LAUNCH_ACT)) == {"R", "mma", "out_mode", "launches"}
     assert set(ops.last_launch_config(ops.LAUNCH_MHA)) >= {"kernel", "D", "out_mode", "kv16", "q16", "launches"}
-    assert _lib.load().hsv_last_launch_config(3, None, 0) < 0
+    assert tuple(ops.last_launch_config(ops.LAUNCH_DIRECT)) == ("kernel", "flags", "has_valid_len", "grid_x", "grid_y",
+                                                                "grid_z", "launches")
+    assert _lib.load().hsv_last_launch_config(3, None, 0) == 7
+    assert _lib.load().hsv_last_launch_config(4, None, 0) < 0
+    assert _lib.load().hsv_last_launch_config(-1, None, 0) < 0
 
 
 # ----------------------------------------------------------------------------------------------
