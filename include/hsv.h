@@ -235,6 +235,38 @@ int hsv_sr_pre_interp_ragged(const float *x, const float *w, const float *bias, 
                              const int32_t *valid_len_out, float *out, int B, int C, int64_t Lin, int64_t Lout,
                              void *stream);
 
+/* Streaming windows (hsv.SpeechSRStream): item b is a window x[b, 0, :valid_len_in[b]] of a longer stream, whose input
+ * sample 0 is the stream's sample origin[b, 0] and whose output sample 0 is the stream's output origin[b, 1]; origin
+ * [B, 3] int64, device.  Output t of the window is computed for the stream's output index origin[b, 1] + t with the
+ * stream's constant scale (float)down / (float)up (up / down = 3 / 1 or 3 / 2, the ratio Lout / Lin), the Lin - 1
+ * clamp at the stream's total length origin[b, 2] when that is >= 0 (no clamp when it is -1), and conv_pre taps
+ * outside the window read 0; outputs at t >= valid_len_out[b] are 0.  An output whose taps all lie inside the window
+ * (or at the stream's own edges) equals, bit for bit, hsv_sr_pre_interp on the whole stream, provided the stream's
+ * length L has up * L < 2^24 and is a multiple of down. */
+int hsv_sr_pre_interp_stream(const float *x, const float *w, const float *bias, const int32_t *valid_len_in,
+                             const int32_t *valid_len_out, const int64_t *origin, float *out, int B, int C,
+                             int64_t Lin, int64_t Lout, int up, int down, void *stream);
+
+/* Per-step bookkeeping of S concurrent SpeechSR streams (all device memory, nothing read back).
+ * State: hist [S, H] fp32 (the last min(received, H) input samples of each slot, right-aligned) and state [S, 3] int64
+ * (samples received, output samples emitted, stream open), zero-initialised.  Inputs: x_new [S, N] fp32, n_new [S]
+ * int32 (valid samples of x_new per slot), start / end [S] int32 flags (a new stream begins in this slot / this is its
+ * last chunk).  A slot request is ignored (the slot stays as it was and emits nothing) when n_new < 0, n_new > N,
+ * n_new % down != 0, or when it carries samples or an end while no stream is open and start is not set.
+ * Window: writes win [S, H + N] (history then new samples), the windows' valid lengths in / out (0 for slots with
+ * nothing to emit), origin [S, 3] for hsv_sr_pre_interp_stream and a plan [S, 6] int64 for the emit launch; state
+ * and hist are only read.  The stream's first (received * up / down - lookahead) outputs are final before its end,
+ * all of them at its end. */
+int hsv_sr_stream_window(const float *x_new, const int32_t *n_new, const int32_t *start, const int32_t *end,
+                         const float *hist, const int64_t *state, float *win, int32_t *valid_len_in,
+                         int32_t *valid_len_out, int64_t *origin, int64_t *plan, int S, int N, int H, int up, int down,
+                         int lookahead, void *stream);
+/* Emit: y [S, Lout] (the windows' SpeechSR outputs, Lout = (H + N) * up / down) -> out [S, cap] (each slot's newly final
+ * outputs, then zeros) and n_out [S] int32; advances hist and state (a slot closed by end is reset). */
+int hsv_sr_stream_emit(const float *y, const float *win, const int64_t *origin, const int64_t *plan, float *hist,
+                       int64_t *state, float *out, int32_t *n_out, int S, int H, int W, int64_t Lout, int cap,
+                       void *stream);
+
 /* Index probe for the bit-exact part of the parity contract: writes, for each
  * dst in [0,Lout): i0, i1 (int32) and lambda (fp32) of the linear interpolation. */
 int hsv_interp_linear_table(int64_t Lin, int64_t Lout, int32_t *i0, int32_t *i1, float *lam, void *stream);

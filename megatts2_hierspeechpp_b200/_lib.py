@@ -49,6 +49,12 @@ SIGNATURES = {
     "hsv_sr_pre_interp": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int64, c_void_p]),
     "hsv_sr_pre_interp_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                          c_int64, c_int64, c_void_p]),
+    "hsv_sr_pre_interp_stream": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                         c_int, c_int64, c_int64, c_int, c_int, c_void_p]),
+    "hsv_sr_stream_window": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "hsv_sr_stream_emit": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_int, c_int, c_int, c_int64, c_int, c_void_p]),
     "hsv_interp_linear_table": (c_int, [c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsv_nearest_gather": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p]),
     "hsv_add3_bcast": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int64, c_void_p]),

@@ -643,6 +643,62 @@ __global__ void sr_pre_interp_kernel(const float *__restrict__ x, const float *_
   }
 }
 
+// Streaming windows: item b is the window x[b, :vl_in[b]] of a longer stream, starting at the stream's input sample
+// org[b].in and output sample org[b].out.  Output t of the window is the stream's output org.out + t: i0 / i1 / lambda
+// come from that global index and the stream's constant scale (down / up, which is what (float)L / (float)Lout rounds
+// to for every L the stream accepts), the Lin - 1 clamp uses the stream's total length org[b].total only when it is
+// known (>= 0, the stream's last window), and conv_pre taps outside the window read 0.  Where every tap of an output
+// lies inside the window (or at the stream's own edges), it equals the full-length kernel on the whole stream.
+struct StreamOrigin {
+  int64_t in, out, total;
+};
+static_assert(sizeof(StreamOrigin) == 3 * sizeof(int64_t), "origin rows are int64 [B, 3]");
+
+__global__ void sr_pre_interp_stream_kernel(const float *__restrict__ x, const float *__restrict__ w,
+                                            const float *__restrict__ bias, float *__restrict__ out,
+                                            const int32_t *__restrict__ vl_in, const int32_t *__restrict__ vl_out,
+                                            const StreamOrigin *__restrict__ org, int B, int C, int64_t Lin,
+                                            int64_t Lout, float scale) {
+  const int64_t n = (int64_t)B * Lout;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int b = (int)(i / Lout);
+    const int64_t t = i - (int64_t)b * Lout;
+    const int vi = __ldg(vl_in + b), vo = __ldg(vl_out + b);
+    const int64_t Li = vi < 0 ? 0 : (vi > Lin ? Lin : vi);
+    const int64_t Lo = vo < 0 ? 0 : (vo > Lout ? Lout : vo);
+    if (t >= Lo || Li == 0) {
+      for (int c = 0; c < C; ++c) out[((int64_t)b * C + c) * Lout + t] = 0.f;
+      continue;
+    }
+    const StreamOrigin o = org[b];
+    int i0, i1;
+    float lam;
+    lin_src(o.out + t, scale, o.total >= 0 ? o.total : INT64_MAX, i0, i1, lam);
+    const float *xr = x + (int64_t)b * Lin;
+    float xa[7], xb[7];
+#pragma unroll
+    for (int j = 0; j < 7; ++j) {
+      const int64_t ta = (int64_t)i0 - 3 + j - o.in, tb = (int64_t)i1 - 3 + j - o.in;   // window-relative taps
+      xa[j] = (ta >= 0 && ta < Li) ? __ldg(xr + ta) : 0.f;
+      xb[j] = (tb >= 0 && tb < Li) ? __ldg(xr + tb) : 0.f;
+    }
+    const float w0 = 1.0f - lam, w1 = lam;
+    for (int c = 0; c < C; ++c) {
+      float va = 0.f, vb = 0.f;
+#pragma unroll
+      for (int j = 0; j < 7; ++j) {
+        const float wj = __ldg(w + c * 7 + j);
+        va = fmaf(wj, xa[j], va);
+        vb = fmaf(wj, xb[j], vb);
+      }
+      const float bv = bias ? __ldg(bias + c) : 0.f;
+      va += bv;
+      vb += bv;
+      out[((int64_t)b * C + c) * Lout + t] = w0 * va + w1 * vb;
+    }
+  }
+}
+
 __global__ void interp_table_kernel(int64_t Lin, int64_t Lout, float scale, int32_t *__restrict__ i0,
                                     int32_t *__restrict__ i1, float *__restrict__ lam) {
   for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < Lout; t += (int64_t)gridDim.x * blockDim.x) {
@@ -893,6 +949,20 @@ extern "C" int hsv_sr_pre_interp_ragged(const float *x, const float *w, const fl
   sr_pre_interp_kernel<<<grid_for((int64_t)B * Lout, 256), 256, 0, hsv::as_stream(stream)>>>(
       x, w, bias, out, valid_len_in, valid_len_out, B, C, Lin, Lout, scale);
   return hsv::check_launch("sr_pre_interp");
+}
+
+extern "C" int hsv_sr_pre_interp_stream(const float *x, const float *w, const float *bias, const int32_t *valid_len_in,
+                                        const int32_t *valid_len_out, const int64_t *origin, float *out, int B, int C,
+                                        int64_t Lin, int64_t Lout, int up, int down, void *stream) {
+  if (B == 0) return HSV_OK;
+  HSV_REQUIRE(x && w && out && valid_len_in && valid_len_out && origin, "sr_pre_interp_stream: null pointer");
+  HSV_REQUIRE(C > 0 && Lin > 0 && Lout > 0, "sr_pre_interp_stream: bad shape");
+  HSV_REQUIRE((up == 3 && down == 1) || (up == 3 && down == 2), "sr_pre_interp_stream: ratio must be 3/1 or 3/2");
+  const float scale = (float)down / (float)up;   // == (float)L / (float)(L * up / down) for L * up < 2^24, (L % down) == 0
+  sr_pre_interp_stream_kernel<<<grid_for((int64_t)B * Lout, 256), 256, 0, hsv::as_stream(stream)>>>(
+      x, w, bias, out, valid_len_in, valid_len_out, reinterpret_cast<const StreamOrigin *>(origin), B, C, Lin, Lout,
+      scale);
+  return hsv::check_launch("sr_pre_interp_stream");
 }
 
 extern "C" int hsv_interp_linear_table(int64_t Lin, int64_t Lout, int32_t *i0, int32_t *i1, float *lam,

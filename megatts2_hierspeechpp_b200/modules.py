@@ -852,6 +852,18 @@ class SpeechSRGenerator(_VocoderBase):
         x = ops.act1d(x, *self.activation_post.params(), scale=sc, **_vl(vout))
         return ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, flags=ops.CONV_TANH, **_vl(vout))
 
+    def _stream_forward(self, win: torch.Tensor, vin: torch.Tensor, vout: torch.Tensor, origin: torch.Tensor):
+        """``forward`` of the streaming windows of ``SpeechSRStream``: win fp32 [S, W], item b the window
+        win[b, :vin[b]] at the stream origins origin[b] (``ops.sr_pre_interp_stream``).  Returns [S, 1, W * scale];
+        outputs of item b below vout[b] away from the window's edges equal those of the whole stream's ``forward``."""
+        up, down = ops.SR_RATIOS[self.scale]
+        x = ops.sr_pre_interp_stream(win.unsqueeze(1), self._f_pre.weight(), self._f_pre.bias(),
+                                     win.shape[-1] * up // down, (vin, vout), origin, (up, down))
+        x, sc = self._stage(x, 0, valid_len=vout)
+        self.activation_post.check_filters()
+        x = ops.act1d(x, *self.activation_post.params(), scale=sc, valid_len=vout)
+        return ops.conv1d_direct(x, self._f_post.weight(), None, pad=3, flags=ops.CONV_TANH, valid_len=vout)
+
     def remove_weight_norm(self):
         for l in self.resblocks:
             l.remove_weight_norm()

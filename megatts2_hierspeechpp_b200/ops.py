@@ -552,6 +552,89 @@ def sr_pre_interp(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor]
     return out
 
 
+SR_RATIOS = {3: (3, 1), 1.5: (3, 2)}   # SpeechSR scale -> (up, down)
+
+
+def _req_ratio(ratio):
+    if tuple(ratio) not in SR_RATIOS.values():
+        raise ValueError(f"ratio must be one of {sorted(SR_RATIOS.values())} (up, down), got {ratio}")
+    return tuple(ratio)
+
+
+def sr_pre_interp_stream(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], Lout: int,
+                         valid_len: Tuple[torch.Tensor, torch.Tensor], origin: torch.Tensor, ratio):
+    """``sr_pre_interp`` of streaming windows: item b is the window x[b, 0, :valid_len[0][b]] of a stream, at the stream's
+    input / output sample origin[b, 0] / origin[b, 1] (int64 [B, 3]; origin[b, 2] = the stream's total length on its last
+    window, else -1).  ``ratio`` = (up, down) = (3, 1) or (3, 2).  Outputs are those of the whole stream at the same
+    global indices wherever every conv_pre tap lies inside the window (include/hsv.h)."""
+    _req(x, "x", ndim=3); _req(w, "w", ndim=3)
+    if bias is not None:
+        _req(bias, "bias")
+    B, one, Lin = x.shape
+    C = w.shape[0]
+    if one != 1 or tuple(w.shape[1:]) != (1, 7):
+        raise ValueError("sr_pre_interp_stream expects x [B,1,L] and w [C,1,7]")
+    up, down = _req_ratio(ratio)
+    vin, vout = valid_len
+    _req_len(vin, B, x.device, "valid_len[0]"); _req_len(vout, B, x.device, "valid_len[1]")
+    _req(origin, "origin", torch.int64, 2)
+    if tuple(origin.shape) != (B, 3) or origin.device != x.device:
+        raise ValueError(f"origin must be int64 [{B}, 3] on {x.device}, got {tuple(origin.shape)} on {origin.device}")
+    out = torch.empty(B, C, Lout, dtype=torch.float32, device=x.device)
+    lib = _lib.load()
+    _lib.check(lib.hsv_sr_pre_interp_stream(_p(x), _p(w), _p(bias), _p(vin), _p(vout), _p(origin), _p(out), B, C, Lin,
+                                            Lout, up, down, _stream()), "hsv_sr_pre_interp_stream")
+    return out
+
+
+def sr_stream_window(x_new: torch.Tensor, n_new: torch.Tensor, start: torch.Tensor, end: torch.Tensor,
+                     hist: torch.Tensor, state: torch.Tensor, ratio, lookahead: int):
+    """One step's windows of S SpeechSR streams (include/hsv.h, ``hsv_sr_stream_window``).  Returns (win [S, H + N],
+    valid_len_in [S], valid_len_out [S], origin [S, 3], plan [S, 6]); ``hist`` / ``state`` are only read."""
+    _req(x_new, "x_new", ndim=2)
+    S, N = x_new.shape
+    for t, name in ((n_new, "n_new"), (start, "start"), (end, "end")):
+        _req_len(t, S, x_new.device, name)
+    _req(hist, "hist", ndim=2); _req(state, "state", torch.int64, 2)
+    H = hist.shape[1]
+    if hist.shape[0] != S or tuple(state.shape) != (S, 3):
+        raise ValueError(f"hist must be [{S}, H] and state [{S}, 3], got {tuple(hist.shape)} and {tuple(state.shape)}")
+    if hist.device != x_new.device or state.device != x_new.device:
+        raise ValueError("hist and state must be on the device of x_new")
+    up, down = _req_ratio(ratio)
+    dev = x_new.device
+    win = torch.empty(S, H + N, dtype=torch.float32, device=dev)
+    vin = torch.empty(S, dtype=torch.int32, device=dev)
+    vout = torch.empty(S, dtype=torch.int32, device=dev)
+    origin = torch.empty(S, 3, dtype=torch.int64, device=dev)
+    plan = torch.empty(S, 6, dtype=torch.int64, device=dev)
+    lib = _lib.load()
+    _lib.check(lib.hsv_sr_stream_window(_p(x_new), _p(n_new), _p(start), _p(end), _p(hist), _p(state), _p(win), _p(vin),
+                                        _p(vout), _p(origin), _p(plan), S, N, H, up, down, int(lookahead), _stream()),
+               "hsv_sr_stream_window")
+    return win, vin, vout, origin, plan
+
+
+def sr_stream_emit(y: torch.Tensor, win: torch.Tensor, origin: torch.Tensor, plan: torch.Tensor, hist: torch.Tensor,
+                   state: torch.Tensor, cap: int):
+    """Copy each stream's newly final outputs of ``y`` [S, Lout] into out [S, cap], and advance ``hist`` / ``state`` in
+    place (include/hsv.h, ``hsv_sr_stream_emit``).  Returns (out, n_out int32 [S])."""
+    _req(y, "y", ndim=2); _req(win, "win", ndim=2); _req(origin, "origin", torch.int64, 2)
+    _req(plan, "plan", torch.int64, 2); _req(hist, "hist", ndim=2); _req(state, "state", torch.int64, 2)
+    S, Lout = y.shape
+    H, W = hist.shape[1], win.shape[1]
+    for t in (win, origin, plan, hist, state):
+        if t.shape[0] != S or t.device != y.device:
+            raise ValueError(f"every stream tensor must have {S} rows on {y.device}")
+    dev = y.device
+    out = torch.empty(S, cap, dtype=torch.float32, device=dev)
+    n_out = torch.empty(S, dtype=torch.int32, device=dev)
+    lib = _lib.load()
+    _lib.check(lib.hsv_sr_stream_emit(_p(y), _p(win), _p(origin), _p(plan), _p(hist), _p(state), _p(out), _p(n_out), S,
+                                      H, W, Lout, int(cap), _stream()), "hsv_sr_stream_emit")
+    return out, n_out
+
+
 def interp_linear_table(Lin: int, Lout: int, device):
     i0 = torch.empty(Lout, dtype=torch.int32, device=device)
     i1 = torch.empty(Lout, dtype=torch.int32, device=device)

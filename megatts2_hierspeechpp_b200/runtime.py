@@ -132,6 +132,11 @@ class CudaGraphRunner:
         graph.replay()
         return static_out
 
+    def ready(self, *args) -> bool:
+        """Whether a call with arguments of these shapes would replay a current graph (no eager run, no capture)."""
+        entry = self._graphs.get(self._key(args))
+        return entry is not None and entry[3] == self._version()
+
     def static_inputs(self, *args):
         """The static input buffers for this shape signature (capture first if needed)."""
         self(*args)
