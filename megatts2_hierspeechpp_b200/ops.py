@@ -885,7 +885,11 @@ def conv1d_c1_strided(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Ten
 
 def masked_mean(x: torch.Tensor, mask: Optional[torch.Tensor], valid_len: Optional[torch.Tensor] = None) -> torch.Tensor:
     """x.sum(2) / mask.sum(2) over all L frames; ``valid_len`` (int32 [B]): item b's mean over its first valid_len[b]
-    frames, summed in the order of its own run (the mask is then not read)."""
+    frames, summed in the order of its own run (the mask is then not read).
+
+    Empty items are not rejected: an item with valid_len 0 gives NaN (0 / 0, the mean of its own, empty run, as
+    ``torch.mean`` of an empty tensor); without ``valid_len`` an all-zero mask row gives x.sum(2) / 0 as the reference
+    does (+-inf, or NaN where the sum is 0)."""
     _req(x, "x", ndim=3)
     B, C, L = x.shape
     out = torch.empty(B, C, dtype=torch.float32, device=x.device)
