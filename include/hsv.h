@@ -65,8 +65,8 @@ int64_t hsv_blk16_rows(int64_t L);
  *             epilogue), msub, warps per CTA, vec_epi (float4 epilogue), nphase, n_tile, stages, G (weight blocks
  *             per ring stage), resident, nabuf (persistent only, else 0), grid x, y, z, blk_mode (kind 3: the
  *             hsv_conv1d_umma_blk16 mode 0-3, 4 = hsv_conv1d_umma_wn_tail; else 0), launches so far
- *   family 1, Activation1d (count 4): run length R (0 when the tensor-core kernel ran), act1d_mma ran, out_mode,
- *             launches so far
+ *   family 1, Activation1d (count 5): run length R (0 when the tensor-core kernel ran), act1d_mma ran, out_mode,
+ *             valid_len given (hsv_act1d_snakebeta_ragged with lengths), launches so far
  *   family 2, attention (count 13): kernel (0 tensor-core, 1 fp32 CUDA-core), D, out_mode, lens given, valid_len
  *             given, prescale, kv16 (K / V tiles copied in 16-byte chunks: Tk % 4 == 0, 16-byte aligned k and v,
  *             batch strides % 4 == 0), q16 (tensor-core kernel: Q tiles copied in 16-byte chunks: Tq % 4 == 0,

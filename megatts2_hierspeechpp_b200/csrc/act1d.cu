@@ -227,13 +227,15 @@ int g_act_run = 0;      // bring-up aid: force the run length (17 or 25); 0 = au
 #endif
 int g_act_mma = 0;      // fp16-operand output: 0 = auto, 1 = CUDA-core kernel (act1d.cu), 2 = tensor-core kernel (act1d_mma.cu)
 
-// hsv_last_launch_config, family 1: run length R (0 for the tensor-core kernel), act1d_mma ran, out_mode, launch count
-void note_launch(int R, int mma, int out_mode) {
+// hsv_last_launch_config, family 1: run length R (0 for the tensor-core kernel), act1d_mma ran, out_mode, valid_len
+// given, launch count
+void note_launch(int R, int mma, int out_mode, int has_valid_len) {
   int *last = hsv::g_last_launch[1];
   last[0] = R;
   last[1] = mma;
   last[2] = out_mode;
-  ++last[3];
+  last[3] = has_valid_len;
+  ++last[4];
 }
 
 template <int R, int OUT_MODE>
@@ -263,7 +265,7 @@ int launch(const float *x, void *out, const float *alpha, const float *beta, con
   const int nt_i = (int)ntiles;
   const int64_t Lp = hsv::blk16_rows(L);
   const int cw = OUT_MODE == 1 ? hsv::blk_cw(C) : 0;
-  note_launch(R, 0, OUT_MODE);
+  note_launch(R, 0, OUT_MODE, valid_len != nullptr);
   cudaError_t e = cudaLaunchKernelEx(&cfg, act1d_kernel<R, OUT_MODE>, x, out, alpha, beta, valid_len, C, L, nrows, nt_i, Lp,
                                      sc, cw);
   if (e != cudaSuccess) {
@@ -337,7 +339,7 @@ extern "C" int hsv_act1d_snakebeta_ragged(const float *x, void *out, const float
   if (g_act_mma == 2 || (g_act_mma == 0 && HSV_ACT_MMA_AUTO && L >= 256 && !valid_len)) {
     const int rc = hsv::act1d_mma_launch(x, out, alpha, beta, B, C, L, in_scale, st);
     if (rc != 1) {
-      note_launch(0, 1, 1);
+      note_launch(0, 1, 1, 0);
       return rc;
     }
     HSV_REQUIRE(g_act_mma != 2, "act1d: shape not eligible for the forced tensor-core variant");

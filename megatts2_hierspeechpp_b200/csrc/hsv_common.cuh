@@ -77,7 +77,7 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // [0] = the tcgen05 conv (conv_umma.cu), [1] = the fused activation (act1d.cu), [2] = attention (mha_mma.cu and the
 // fp32 kernel of frame_ops.cu), [3] = the CUDA-core convs of conv_direct.cu.  Process-global bookkeeping, written just
 // before the launch; it never changes what is launched.
-constexpr int LAST_CONV_N = 15, LAST_ACT_N = 4, LAST_MHA_N = 13, LAST_DIRECT_N = 7;
+constexpr int LAST_CONV_N = 15, LAST_ACT_N = 5, LAST_MHA_N = 13, LAST_DIRECT_N = 7;
 extern int g_last_launch[4][16];
 // family 2: kernel (0 tensor-core, 1 fp32 CUDA-core), D, out_mode, lens, valid_len, prescale, kv16 (16-byte K / V tile
 // copies), q16 (16-byte Q tile copies), key tiles, grid x / y / z; then the running launch count

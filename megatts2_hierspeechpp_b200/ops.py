@@ -678,7 +678,9 @@ def peak_norm_pcm16(x: torch.Tensor, s1: float = 32767.0, s2: float = 0.999, per
     """int16 PCM of ``x / max|x| * s1 * s2`` (fp32, reference operation order, truncation like numpy's astype).
 
     x: fp32 [..., L]; leading dims are rows.  ``per_row=False`` uses one peak for the whole tensor
-    (inference_plm.py:183-188 / inference_speechsr.py:39-41), ``True`` one per row.  Returns (pcm int16, peaks fp32)."""
+    (inference_plm.py:183-188 / inference_speechsr.py:39-41), ``True`` one per row.  An all-zero row (or tensor, for
+    the global peak) has peak 0: 0 / 0 is NaN, and the device's float-to-int conversion makes it 0, so its PCM is all
+    zeros (numpy's NaN -> int16 cast is platform-defined).  Returns (pcm int16, peaks fp32)."""
     _req(x, "x")
     if x.dim() < 1:
         raise ValueError("x must have at least one dim")
@@ -995,7 +997,7 @@ LAUNCH_CONV, LAUNCH_ACT, LAUNCH_MHA, LAUNCH_DIRECT = 0, 1, 2, 3
 _LAUNCH_FIELDS = {
     LAUNCH_CONV: ("kind", "msub", "warps", "vec_epi", "nphase", "n_tile", "stages", "G", "resident", "nabuf",
                   "grid_x", "grid_y", "grid_z", "blk_mode", "launches"),
-    LAUNCH_ACT: ("R", "mma", "out_mode", "launches"),
+    LAUNCH_ACT: ("R", "mma", "out_mode", "has_valid_len", "launches"),
     LAUNCH_MHA: ("kernel", "D", "out_mode", "has_lens", "has_valid_len", "prescale", "kv16", "q16", "key_tiles",
                  "grid_x", "grid_y", "grid_z", "launches"),
     LAUNCH_DIRECT: ("kernel", "flags", "has_valid_len", "grid_x", "grid_y", "grid_z", "launches"),

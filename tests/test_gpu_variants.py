@@ -11,10 +11,13 @@ simplest variants, so every case here forces (a, c) or naturally selects (b) a v
   the epilogue formula (conv + bias) + residual do not depend on the variant;
 * activation: against the fp32 oracle (1e-5 x max(1, peak)) and the fp64 closed form, over the whole tensor including
   both replicate-clamped edges, and bit for bit across run lengths (one thread computes an output over the same taps
-  whatever R is).
+  whatever R is); the ragged body (valid_len given, a separately inlined copy of the kernel body) at every run length
+  with item lengths on both sides of a 16 R-step tile edge, against the fp64 closed form of each item alone.
 
 (d) is a census: the variant of every conv / activation launch of the benchmark workloads must be in ``VERIFIED``, the
-set of variants the cases above check.  A policy change that ships a new variant fails it until a case covers it.
+set of variants the cases above check (activation keys ``act:R{R}:{f32|blk16}:{full|ragged}``).  A policy change that
+ships a new variant fails it until a case covers it.  The SpeechSR24, streaming SpeechSR and ragged-batch entry points
+are censused by test_gpu_sr_variants.py.
 The operand-writing epilogue's variants (``operand-out:{mode}:n{n_tile}``) are checked against fp64 by
 test_gpu_front_variants.py (c), which declares them in ``OPERAND_KEYS``.
 """
@@ -65,7 +68,7 @@ def conv_key(c):
 def act_key(c):
     if c["mma"]:
         return "act:mma"
-    return f"act:R{c['R']}:{'blk16' if c['out_mode'] else 'f32'}"
+    return f"act:R{c['R']}:{'blk16' if c['out_mode'] else 'f32'}:{'ragged' if c['has_valid_len'] else 'full'}"
 
 
 # ----------------------------------------------------------------------------------------------
@@ -182,9 +185,8 @@ VERIFIED = set(OPERAND_KEYS) | {
     "convT:m1:w4:n64", "convT:m2:w4:n64", "convT:m4:w4:n32",
     "convT:m1:w8:n128", "convT:m1:w4:n128", "convT:m2:w8:n128", "convT:m2:w4:n128", "convT:m4:w4:n128",
     "convT:m1:w4:n32", "convT:m2:w4:n32", "convT:m1:w4:n16", "convT:m2:w4:n16", "convT:m4:w4:n16",
-    "act:R9:f32", "act:R9:blk16", "act:R17:f32", "act:R17:blk16", "act:R21:f32", "act:R21:blk16",
-    "act:R25:f32", "act:R25:blk16",
 }
+VERIFIED |= {f"act:R{R}:{m}:{form}" for R in RUNS for m in ("f32", "blk16") for form in ("full", "ragged")}
 
 
 def _declared_keys():
@@ -194,7 +196,8 @@ def _declared_keys():
     keys |= {_conv_key_expected(c[0], c[1], c[4], c[6], c[7], None, True) for c in CONVT_MATRIX}
     keys |= {c[-1] for c in PERSIST_MATRIX}
     keys |= {c[-1] for c in CONV_NATURAL}
-    keys |= {f"act:R{R}:{m}" for R in RUNS for m in ("f32", "blk16")}
+    keys |= {f"act:R{R}:{m}:full" for R in RUNS for m in ("f32", "blk16")}
+    keys |= {f"act:R{R}:{m}:ragged" for R in RUNS for m in ("f32", "blk16")}
     return keys
 
 
@@ -204,13 +207,14 @@ def test_verified_set_is_covered_by_the_cases():
     assert not missing, sorted(missing)
 
 
-def test_last_launch_config_hook_four_families():
-    """The hook reports the documented fields of its four families (conv, activation, attention, CUDA-core conv) and
-    rejects an unknown family (host-only, no GPU)."""
+def test_last_launch_config_hook_four_families_ragged_act():
+    """The hook reports the documented fields of its four families (conv, activation with its valid_len flag,
+    attention, CUDA-core conv) and rejects an unknown family (host-only, no GPU)."""
     from megatts2_hierspeechpp_b200 import _lib, build, ops
     build.build()
     assert set(ops.last_launch_config(ops.LAUNCH_CONV)) >= {"kind", "msub", "warps", "vec_epi", "blk_mode", "launches"}
-    assert set(ops.last_launch_config(ops.LAUNCH_ACT)) == {"R", "mma", "out_mode", "launches"}
+    assert tuple(ops.last_launch_config(ops.LAUNCH_ACT)) == ("R", "mma", "out_mode", "has_valid_len", "launches")
+    assert _lib.load().hsv_last_launch_config(1, None, 0) == 5
     assert set(ops.last_launch_config(ops.LAUNCH_MHA)) >= {"kernel", "D", "out_mode", "kv16", "q16", "launches"}
     assert tuple(ops.last_launch_config(ops.LAUNCH_DIRECT)) == ("kernel", "flags", "has_valid_len", "grid_x", "grid_y",
                                                                 "grid_z", "launches")
@@ -428,18 +432,18 @@ def _fp16_neighbour_ok(y, ref):
     return bool(((y - ref).abs() <= ulp + 1e-5 * max(1.0, a.max().item())).all())
 
 
-def _act_run(ops, x, al, be, R, blk):
+def _act_run(ops, x, al, be, R, blk, valid_len=None):
     """The activation forced to run length R; returns (fp32 [B,C,L] result, key that ran)."""
     B, C, L = x.shape
     try:
         with _Flags(ops, act=R << 8):
             if blk:
                 buf = ops.blk16_buffer(B, C, L, DEV, slot=SLOT)
-                ops.act1d_blk16(x, al, be, buf)
+                ops.act1d_blk16(x, al, be, buf, valid_len=valid_len)
                 key = act_key(ops.last_launch_config(ops.LAUNCH_ACT))
                 y = ops.unpack_blk16(buf, C, L)
             else:
-                y = ops.act1d(x, al, be)
+                y = ops.act1d(x, al, be, valid_len=valid_len)
                 key = act_key(ops.last_launch_config(ops.LAUNCH_ACT))
     finally:
         ops.set_act_variant(0)
@@ -459,7 +463,7 @@ def test_act_run_length_vs_oracle(hsv, R, blk):
         al, be = _act_params(C, R + i)
         ref = _act_oracle(x, al, be)
         y, key = _act_run(ops, x.to(DEV), al.to(DEV), be.to(DEV), R, blk)
-        assert key == f"act:R{R}:{'blk16' if blk else 'f32'}", key
+        assert key == f"act:R{R}:{'blk16' if blk else 'f32'}:full", key
         y = y.cpu()
         if blk:
             assert _fp16_neighbour_ok(y, ref), ((B, C, L), (y - ref).abs().max().item())
@@ -486,6 +490,46 @@ def test_act_run_lengths_bit_identical(hsv):
                 assert torch.equal(y, ys[0]), (B, C, L, R, blk, (y - ys[0]).abs().max().item())
 
 
+def _ragged_lens(R):
+    """(L, valid lengths): 0, 1, both sides of the first 16 R-step tile edge, and the full row."""
+    T = 16 * R
+    L = 3 * T + 5
+    return L, [0, 1, T - 1, T, T + 1, L]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("blk", [False, True], ids=["f32", "blk16"])
+@pytest.mark.parametrize("R", RUNS)
+def test_act_ragged_run_length_vs_fp64(hsv, R, blk):
+    """The ragged body (valid_len given) at every run length: each item against the fp64 closed form on its own
+    valid_len[b] steps (the replicate clamp at its length, not at L), NaN past the length never read, exact zeros
+    written there, and bit for bit the dense kernel on the item alone."""
+    ops = hsv.ops
+    L, lens = _ragged_lens(R)
+    B, C = len(lens), 32
+    gen = torch.Generator().manual_seed(77 * R + blk)
+    x = torch.randn(B, C, L, generator=gen) * 1.5
+    for b, n in enumerate(lens):
+        x[b, :, n:] = float("nan")
+    al, be = _act_params(C, R)
+    vl = torch.tensor(lens, dtype=torch.int32, device=DEV)
+    y, key = _act_run(ops, x.to(DEV), al.to(DEV), be.to(DEV), R, blk, valid_len=vl)
+    assert key == f"act:R{R}:{'blk16' if blk else 'f32'}:ragged", key
+    for b, n in enumerate(lens):
+        assert bool((y[b, :, n:] == 0).all()), (b, n)
+        if n == 0:
+            continue
+        alone, _ = _act_run(ops, x[b:b + 1, :, :n].contiguous().to(DEV), al.to(DEV), be.to(DEV), R, blk)
+        assert torch.equal(y[b:b + 1, :, :n], alone), (b, n)
+        got = y[b, :, :n].cpu().double().numpy()
+        cf = CF.activation1d(x[b:b + 1, :, :n].numpy(), al.numpy(), be.numpy())[0]
+        tol = 1e-4 * max(1.0, np.abs(cf).max())
+        if blk:
+            a = np.abs(cf)
+            tol = tol + np.exp2(np.floor(np.log2(np.maximum(a, 2.0 ** -14))) - 10)
+        assert (np.abs(got - cf) <= tol).all(), (b, n, np.abs(got - cf).max())
+
+
 def _windows(L, n, seed):
     """First and last 1024 steps plus n seeded windows straddling 512-step boundaries: [(start, stop)]."""
     rng = np.random.default_rng(seed)
@@ -504,10 +548,10 @@ def test_act_natural_policy(hsv, B, C, L, R):
     x = torch.randn(B, C, L, generator=gen) * 1.5
     al, be = _act_params(C, L)
     y = ops.act1d(x.to(DEV), al.to(DEV), be.to(DEV))
-    assert act_key(ops.last_launch_config(ops.LAUNCH_ACT)) == f"act:R{R}:f32"
+    assert act_key(ops.last_launch_config(ops.LAUNCH_ACT)) == f"act:R{R}:f32:full"
     buf = ops.blk16_buffer(B, C, L, DEV, slot=SLOT)
     ops.act1d_blk16(x.to(DEV), al.to(DEV), be.to(DEV), buf)
-    assert act_key(ops.last_launch_config(ops.LAUNCH_ACT)) == f"act:R{R}:blk16"
+    assert act_key(ops.last_launch_config(ops.LAUNCH_ACT)) == f"act:R{R}:blk16:full"
     yb = ops.unpack_blk16(buf, C, L).cpu()
     y = y.cpu()
     H = 16   # halo: an output depends on 6 inputs either side
