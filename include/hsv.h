@@ -315,6 +315,29 @@ int hsv_peak_norm_pcm16(const float *x, int16_t *out, float *peak_ws, int rows, 
 int hsv_peak_norm_pcm16_rows(const float *x, int16_t *out, float *peak_ws, int rows, int64_t L, float s1,
                              const float *s2, void *stream);
 
+/* ---- the step before SpeechSR (inference_speechsr.py:28-34): torchaudio.functional.resample(x, orig, new_freq,
+ * resampling_method="kaiser_window") (lowpass_filter_width 6, rolloff 0.99, beta 14.769656459379492) of a ragged batch
+ * with one rate per item (csrc/resample.cu).
+ *   x          [B, T] fp32 (x_int16 = 0) or int16 PCM (x_int16 = 1, read as (float)s * (1.0f / 32768), exact)
+ *   rate       [B] int32, device: each item's sample rate
+ *   valid_len  [B] int32, device: each item's input samples, clamped to [0, T]; x[b, t >= valid_len[b]] is never
+ *              read and counts as zero, as torchaudio's padding does
+ *   host_desc  [n_desc][6] int32, HOST (1 <= n_desc <= 16, distinct rates): {rate, o, n, width, K, offset} with
+ *              o : n = rate : new_freq reduced, K = 2 width + o, the item's filter stored transposed as
+ *              table[offset + k * n + p] = torchaudio's kernel[p, 0, k] (fp32).  The entry of rate == new_freq is the
+ *              copy {new_freq, 1, 1, 0, 0, 0}: its items are copied (converted, for int16), bit for bit.
+ *   table      [table_len] fp32, device (may be NULL when table_len == 0)
+ *   out        [B, T_out] fp32, n_out [B] int32, device
+ * Item b's first n_out[b] = min(N_b, T_out) outputs, N_b = min(ceil((float)((double)(n L_b) / o)), (L_b / o + 1) n)
+ * (torchaudio's output count: its ceil(torch.as_tensor(n * L / o)) rounds the quotient to fp32), are y[f n + p] = sum_{k < K} t[p][k] x[f o + k -
+ * width], summed in an order that depends on K alone, so they equal, bit for bit, the item's own call with B = 1 and
+ * no padding; the rest of its row is 0.  An item whose rate has no descriptor gets n_out = 0 and zeros;
+ * nothing else is checked on the device.  Argument errors (descriptors, shapes, a rate ratio whose 256 outputs need
+ * more than 12288 staged input samples) are reported before any CUDA call. */
+int hsv_resample_ragged(const void *x, int x_int16, const int32_t *rate, const int32_t *valid_len, const float *table,
+                        int64_t table_len, const int32_t *host_desc, int n_desc, int new_freq, float *out,
+                        int32_t *n_out, int B, int64_t T, int64_t T_out, void *stream);
+
 /* ---- frame-rate operators of the step BEFORE the vocoder (SURVEY.md §8f2; csrc/frame_ops.cu).  fp32 [B,C,T] tensors,
  * mask = [B,T] (1 = valid frame, may be NULL), blk16 outputs feed hsv_conv1d_umma.
  *

@@ -11,6 +11,7 @@ from .modules import (AMPBlock0, AMPBlock1, Activation1d, DBlock, DownSample1d, 
 from .config import HIER_CFG, SR_CFG
 from .runtime import CudaGraphRunner, patch_reference, shard_utterances, to_pcm16
 from .sr_stream import SpeechSRStream
+from .resample import Resample, SpeechSRAudio
 from . import front, ops, ttv
 from .front import HierSpeechSynthesizer
 from .ttv import PitchPredictor, TTVTail, W2VDecoder
@@ -21,4 +22,5 @@ __all__ = [
     "UpSample1d", "Vocoder", "VocoderSR", "get_padding", "kaiser_sinc_filter1d", "HIER_CFG", "SR_CFG", "CudaGraphRunner",
     "patch_reference", "shard_utterances", "ops", "front", "HierSpeechSynthesizer", "invalidate_caches", "to_pcm16",
     "ttv", "W2VDecoder", "PitchPredictor", "TTVTail", "SpeechSRStream",
+    "Resample", "SpeechSRAudio",
 ]

@@ -94,6 +94,8 @@ SIGNATURES = {
                             c_void_p]),
     "hsv_peak_norm_pcm16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_float, c_float, c_int, c_void_p]),
     "hsv_peak_norm_pcm16_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_float, c_void_p, c_void_p]),
+    "hsv_resample_ragged": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int,
+                                    c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p]),
 }
 
 # bring-up aids exported by the library but not part of the drop-in contract

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 OUT = os.path.join(_HERE, "libhsv.so")
-SOURCES = ["common.cu", "act1d.cu", "act1d_mma.cu", "conv_direct.cu", "conv_umma.cu", "pcm.cu", "sinegen.cu", "frame_ops.cu", "mha_mma.cu", "noise.cu", "sr_stream.cu"]
+SOURCES = ["common.cu", "act1d.cu", "act1d_mma.cu", "conv_direct.cu", "conv_umma.cu", "pcm.cu", "sinegen.cu", "frame_ops.cu", "mha_mma.cu", "noise.cu", "sr_stream.cu", "resample.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-shared",

@@ -711,6 +711,29 @@ def peak_norm_pcm16_rows(x: torch.Tensor, s2: torch.Tensor, s1: float = 32767.0)
     return out, peaks
 
 
+def resample(x: torch.Tensor, rate: torch.Tensor, valid_len: torch.Tensor, table: torch.Tensor, desc, new_freq: int,
+             out_len: int):
+    """Kaiser-windowed sinc resampling of a ragged batch to ``new_freq`` (include/hsv.h, ``hsv_resample_ragged``).
+    x: fp32 or int16 [B, T]; rate / valid_len: int32 [B] on x's device; table: fp32 [n] (the filters, [K][n] each);
+    desc: host rows (rate, o, n, width, K, offset).  Returns (y fp32 [B, out_len], n_out int32 [B])."""
+    if not isinstance(x, torch.Tensor) or x.dtype not in (torch.float32, torch.int16):
+        raise ValueError("x: expected a float32 or int16 tensor")
+    _req(x, "x", x.dtype, 2)
+    B, T = x.shape
+    _req_len(rate, B, x.device, "rate"); _req_len(valid_len, B, x.device, "valid_len")
+    _req(table, "table", ndim=1)
+    if table.device != x.device:
+        raise ValueError(f"table is on {table.device}, x on {x.device}")
+    flat = [int(v) for row in desc for v in row]
+    host_desc = (ctypes.c_int32 * len(flat))(*flat)
+    y = torch.empty(B, out_len, dtype=torch.float32, device=x.device)
+    n_out = torch.empty(B, dtype=torch.int32, device=x.device)
+    _lib.check(_lib.load().hsv_resample_ragged(_p(x), int(x.dtype == torch.int16), _p(rate), _p(valid_len), _p(table),
+                                               table.numel(), host_desc, len(desc), int(new_freq), _p(y), _p(n_out), B,
+                                               T, int(out_len), _stream()), "hsv_resample_ragged")
+    return y, n_out
+
+
 # ----------------------------------------------------------------------------------------------
 # frame-rate operators of the step before the vocoder (csrc/frame_ops.cu)
 # ----------------------------------------------------------------------------------------------

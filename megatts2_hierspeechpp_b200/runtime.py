@@ -57,7 +57,10 @@ class CudaGraphRunner:
     ``config_token`` for host-side switches read at capture time (``parallel_blocks``, the fusion threshold):
     entries from an older epoch are dropped and recaptured, never replayed.  The cache is an LRU of at most
     ``max_graphs`` shapes; a shape is only captured on its ``capture_after``-th call (default: the first), earlier
-    calls run eagerly -- set it to 2 under variable-length traffic so one-off lengths never pay a capture."""
+    calls run eagerly -- set it to 2 under variable-length traffic so one-off lengths never pay a capture.
+
+    Keyword arguments are passed to ``fn`` unchanged and are part of the signature (one graph per value): they take
+    hashable host values, such as an output length or a flag."""
 
     def __init__(self, fn: Callable, warmup: int = 2, max_graphs: int = 16, capture_after: int = 1):
         from collections import OrderedDict
@@ -79,15 +82,20 @@ class CudaGraphRunner:
         return (M._CACHE_EPOCH[0], ops.WORKSPACE_EPOCH[0], M.FUSE_MAX_CHANNELS[0], M.FUSE_MAX_ELEMS[0],
                 M.SEPARATE_MAX_ELEMS[0], ops.MHA_VARIANT[0], par)
 
-    def _key(self, args):
-        return tuple((tuple(a.shape), a.dtype, a.device.index) for a in args)
+    def _key(self, args, kwargs=None):
+        key = tuple((tuple(a.shape), a.dtype, a.device.index) for a in args)
+        if not kwargs:
+            return key
+        if any(isinstance(v, torch.Tensor) for v in kwargs.values()):
+            raise TypeError("CudaGraphRunner: pass tensors positionally (keyword arguments are host values)")
+        return key + (tuple(sorted(kwargs.items())),)
 
-    def __call__(self, *args: torch.Tensor):
+    def __call__(self, *args: torch.Tensor, **kwargs):
         from . import ops
         for a in args:
             if not a.is_cuda:
                 raise RuntimeError("CudaGraphRunner: CUDA tensors only")
-        key = self._key(args)
+        key = self._key(args, kwargs)
         entry = self._graphs.get(key)
         if entry is not None and entry[3] != self._version():
             del self._graphs[key]          # stale pointers (weights refolded / workspaces moved): never replay
@@ -98,7 +106,7 @@ class CudaGraphRunner:
                 self._seen.clear()
             if self._seen[key] < self.capture_after:
                 with torch.no_grad():
-                    return self.fn(*args)
+                    return self.fn(*args, **kwargs)
             static_in = [torch.empty_like(a) for a in args]
             for s, a in zip(static_in, args):
                 s.copy_(a)
@@ -108,13 +116,13 @@ class CudaGraphRunner:
                 side.wait_stream(torch.cuda.current_stream())
                 with torch.cuda.stream(side), torch.no_grad():
                     for _ in range(self.warmup):  # folds weights, allocates workspaces, loads modules
-                        self.fn(*static_in)
+                        self.fn(*static_in, **kwargs)
                 torch.cuda.current_stream().wait_stream(side)
                 torch.cuda.synchronize()
                 version = self._version()      # after warm-up: folding / packing may have happened in it
                 graph = torch.cuda.CUDAGraph()
                 with torch.no_grad(), torch.cuda.graph(graph):
-                    static_out = self.fn(*static_in)
+                    static_out = self.fn(*static_in, **kwargs)
             finally:
                 ops._pin_depth[0] -= 1
             if version != self._version():
@@ -132,15 +140,15 @@ class CudaGraphRunner:
         graph.replay()
         return static_out
 
-    def ready(self, *args) -> bool:
+    def ready(self, *args, **kwargs) -> bool:
         """Whether a call with arguments of these shapes would replay a current graph (no eager run, no capture)."""
-        entry = self._graphs.get(self._key(args))
+        entry = self._graphs.get(self._key(args, kwargs))
         return entry is not None and entry[3] == self._version()
 
-    def static_inputs(self, *args):
+    def static_inputs(self, *args, **kwargs):
         """The static input buffers for this shape signature (capture first if needed)."""
-        self(*args)
-        return self._graphs[self._key(args)][1]
+        self(*args, **kwargs)
+        return self._graphs[self._key(args, kwargs)][1]
 
     def clear(self):
         self._graphs.clear()
